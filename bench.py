@@ -1,8 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- the headline benchmark of the rrt hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the framebuffer the last timed step produced (the [H, W, 3] sums of every pixel, row 0 =
+bottom scanline, as rank 0 holds it) to DIR/image.npy, so that two builds run with the same arguments can be compared
+output for output: the scene, the seed and therefore every sample are fixed by the arguments.  Over 64 MB, a fixed
+sample of pixels is written with their indices (DIR/pixel_index.npy); --workload final_anim writes such a sample of
+every frame of the animation, [frames, k, 3].
 
 Workload (BASELINE.json configs[1]): scenes/final.txt (488 spheres), 1200x800, 500 spp, depth 50.
 A step = one full render of that image: 480 M camera paths, ~1.21 G ray segments.
@@ -305,6 +311,35 @@ def cpu_baseline_sample(rays_per_path):
             "sample": "oracle port (OpenMP) final.txt %dx%d, %d spp, %.2f s" % (W, H, spp, sec)}
 
 
+DUMP_BYTES = 64 * 10**6  # every file of one dump together, .npy headers included
+DUMP_SAMPLE_PIXELS = 1 << 20
+
+
+def dump_pixel_sample(n_pixels, k):
+    """k of n_pixels flat pixel indices, sorted; seeded, so the same for every run of the same image size."""
+    import numpy as np
+
+    return np.sort(np.random.default_rng(SEED).choice(n_pixels, k, replace=False))
+
+
+def dump_outputs(dirname, image, pixel_index=None):
+    """DIR/image.npy = the [H, W, 3] framebuffer.  A framebuffer larger than DUMP_BYTES is replaced by a fixed sample of
+    DUMP_SAMPLE_PIXELS pixels: DIR/image.npy holds their [k, 3] sums and DIR/pixel_index.npy their flat indices y * W + x.
+    A caller that sampled the pixels itself passes their indices as pixel_index."""
+    import numpy as np
+
+    os.makedirs(dirname, exist_ok=True)
+    image = np.asarray(image)
+    assert image.dtype in (np.float32, np.float64)
+    if pixel_index is None and image.nbytes > DUMP_BYTES:
+        px = image.reshape(-1, 3)
+        pixel_index = dump_pixel_sample(len(px), DUMP_SAMPLE_PIXELS)
+        image = px[pixel_index]
+    if pixel_index is not None:
+        np.save(os.path.join(dirname, "pixel_index.npy"), np.asarray(pixel_index).astype(np.float64))
+    np.save(os.path.join(dirname, "image.npy"), image)
+
+
 def run_anim(args, wl, rank, world, local_rank):
     """--workload final_anim: the reference's 261-frame camera dolly (1280x720, 50 spp) as ONE uploaded scene +
     one camera update and one kernel launch per frame; frames dealt round-robin over the ranks (no collective).
@@ -336,7 +371,7 @@ def run_anim(args, wl, rank, world, local_rank):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def step(p=params):
+    def step(p=params, keep=None):
         rays = 0
         for f in mine:
             ctx.set_camera(cams[f])
@@ -345,6 +380,8 @@ def run_anim(args, wl, rank, world, local_rank):
             st = ctx.render_device(p, acc.data_ptr())
             rays += st["rays"]
             ctx.resolve_device(acc.data_ptr(), out.data_ptr(), n)
+            if keep is not None:
+                keep[f] = out.view(-1, 3)[keep_index]
         return rays
 
     rays = torch.tensor([step(pcount)], dtype=torch.int64, device=dev)
@@ -364,6 +401,22 @@ def run_anim(args, wl, rank, world, local_rank):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     sec = t.item() / args.steps
+    if args.dump_outputs:
+        # a step renders every frame, each into the same buffer: the last step is rendered once more, untimed (same
+        # cameras, same seed, hence the same sums), keeping a fixed pixel sample of every frame, gathered on rank 0
+        k = min(Wl * Hl, (DUMP_BYTES - 4096) // (12 * len(cams) + 8))  # float3 per frame + a float64 index per pixel
+        idx = dump_pixel_sample(Wl * Hl, k)
+        keep_index = torch.from_numpy(idx).to(dev)
+        frames = torch.zeros((len(cams), k, 3), dtype=torch.float32, device=dev)
+        step(keep=frames)
+        if world > 1:
+            dist.all_reduce(frames)  # every frame is rendered by one rank; the others contribute zeros
+        if rank == 0:
+            frames = frames.cpu().numpy()
+            if k == Wl * Hl:
+                dump_outputs(args.dump_outputs, frames.reshape(len(cams), Hl, Wl, 3))
+            else:
+                dump_outputs(args.dump_outputs, frames, idx)
     # e2e: host framebuffer per frame through rrtb_render (D2H inside), scene uploaded once per step
     barrier()
     t0 = time.perf_counter()
@@ -406,7 +459,12 @@ def main():
     ap.add_argument("--height", type=int, default=0)
     ap.add_argument("--shard", default="tiles", choices=["tiles", "samples"])
     ap.add_argument("--precision", default="f32", choices=["f32", "f64"], help="f64 = the double integrator (the reference's rrtd build); not the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the framebuffer of the last timed step to DIR/image.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
 
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # `python bench.py --gpus N` without a launcher: re-run under torch.distributed.run, one rank per GPU
@@ -520,6 +578,20 @@ def main():
     dev_s, wall, kern_s = tt.tolist()
     sec_per_step = dev_s / args.steps
     value = total_rays / sec_per_step / 1e6
+    if args.dump_outputs:
+        image = np.empty((Hl, Wl, 3), np.float64 if f64 else np.float32) if rank == 0 else None
+        if world > 1 and shard_mode == 1:
+            # the ranks ADD their samples into rank 0's sum buffer, which only a download resolves and clears: it holds
+            # every step so far.  Clear it, then render the last step once more, untimed (same seed, same sums).
+            if rank == 0:
+                ctx.frame_download(image, shard_mode)
+            barrier()
+            step()
+            barrier()
+        if rank == 0:
+            # world > 1, tiles: every rank's tiles of the last step are in rank 0's frame (barrier above)
+            image = out.cpu().numpy().reshape(Hl, Wl, 3) if world == 1 else ctx.frame_download(image, shard_mode)
+            dump_outputs(args.dump_outputs, image)
 
     # ---- e2e: through the C ABI with HOST buffers, every step: scene upload + LBVH build + render + D2H of the frame
     from rrt_b200 import PinnedBuffer

@@ -21,7 +21,7 @@ from rrt_b200.types import (
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 REF_DIR = os.path.join(ORACLE_DIR, "_ref")
-REFERENCE_SRC = "/root/reference"
+GOLDEN_SCENES = os.path.join(ROOT, "tests", "golden", "scenes")
 
 
 def _p(a, t):
@@ -262,8 +262,10 @@ def have_ref():
 
 
 def ref_scene_path(name):
-    """Scene text file staged by oracle/Makefile (oracle/_ref/scenes), else the read-only reference."""
-    for base in (os.path.join(REF_DIR, "scenes"), os.path.join(REFERENCE_SRC, "scenes")):
+    """The reference's scene file as staged by oracle/Makefile (oracle/_ref/scenes), else its stored stand-in
+    (tests/golden/scenes): a text written from the reference parser's arrays (tests/golden/scene_*.npz) that parses
+    back to exactly those arrays and counts."""
+    for base in (os.path.join(REF_DIR, "scenes"), GOLDEN_SCENES):
         p = os.path.join(base, name)
         if os.path.exists(p):
             return p

@@ -43,3 +43,24 @@ def test_our_arm_line_reduced_spp():
     assert cb["kind"] in ("reference", "port") and cb["value"] > 0 and cb["cores"] >= 1 and "sample" in cb
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     assert "workload" in d["config"] and "model" not in d["config"]
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_framebuffer_of_the_timed_path(tmp_path, ctx):
+    """--dump-outputs writes the last timed step's framebuffer: the same sums the host-buffer render returns."""
+    import numpy as np
+
+    from conftest import load_golden
+
+    d = run_bench("--spp", "4", "--steps", "2", "--warmup", "0", "--no-baselines", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 2
+    got = np.load(tmp_path / "image.npy")
+    assert got.shape == (800, 1200, 3) and got.dtype == np.float32
+    ctx.set_scene(load_golden("final")[0], use_bvh=True)
+    want, _ = ctx.render(1200, 800, 4, 50, seed=1984)
+    assert got.tobytes() == want.tobytes()

@@ -14,7 +14,9 @@ EXE = os.path.join(ROOT, "rrt_b200", "bin", "rrt")
 
 @pytest.mark.parametrize("name", ["test1", "test2", "test3", "final"])
 def test_parser_bit_exact_vs_reference_parse(name, built_lib):
-    """The four shipped scenes parse to exactly the arrays the reference's own parser produced (fixture)."""
+    """The four shipped scenes parse to exactly the arrays the reference's own parser produced (fixture).  Where the
+    reference's files are not staged (oracle/_ref/scenes), the stand-ins of tests/golden/scenes are parsed: texts
+    written from that fixture by tools/make_scene_texts.py, so this checks the parser on them, not on the originals."""
     from rrt_b200 import Scene
 
     p = ref_scene_path(name + ".txt")
@@ -237,9 +239,9 @@ def test_parser_survives_mutated_scenes_under_sanitizers():
     may not crash, read out of bounds or leak."""
     import shutil
 
-    scenes = "/root/reference/scenes" if os.path.isdir("/root/reference/scenes") else os.path.join(ROOT, "oracle", "_ref", "scenes")
-    if not os.path.isdir(scenes) or shutil.which("g++") is None:
-        pytest.skip("needs the reference's scene files and g++")
+    scenes = os.path.dirname(ref_scene_path("final.txt"))
+    if shutil.which("g++") is None:
+        pytest.skip("needs g++")
     r = subprocess.run(["bash", os.path.join(ROOT, "tools", "fuzz_parser.sh"), "300", scenes], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "sanitizer findings 0" in r.stdout

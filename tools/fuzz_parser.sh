@@ -3,8 +3,8 @@
 # AddressSanitizer + UndefinedBehaviorSanitizer behind a tiny driver and feed it mutated copies of the reference's scenes
 # (truncated, shuffled, tokens replaced by keywords / nan / inf / huge numbers, random bytes inserted).  The parser may
 # reject a file, it may not crash, overflow or leak.   usage: tools/fuzz_parser.sh [n_files] [scenes_dir]
-N=${1:-600}; SC=${2:-/root/reference/scenes}
-[ -d "$SC" ] || SC="$(dirname "$0")/../oracle/_ref/scenes"
+N=${1:-600}; SC=${2:-$(dirname "$0")/../oracle/_ref/scenes}
+[ -d "$SC" ] || SC="$(dirname "$0")/../tests/golden/scenes"
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"; W=$(mktemp -d /tmp/rrtb_fuzz.XXXXXX); mkdir -p $W/in
 cat > $W/drv.cpp <<EOF
 #include <stdint.h>
