@@ -111,21 +111,17 @@ int launch_render(rrtb_ctx *ctx, const rrtb_render_params *p, uint64_t *d_accum,
 int finish_render(rrtb_ctx *ctx, rrtb_stats *stats);
 int launch_resolve_tiles(rrtb_ctx *ctx, const uint64_t *d_accum, void *d_out, const rrtb_render_params *p, bool f64);
 int launch_accumulate_atomic(rrtb_ctx *ctx, uint64_t *d_dst, const uint64_t *d_src, size_t n);
-int launch_resolve(rrtb_ctx *ctx, const uint64_t *d_accum, float *d_out, size_t n);
-int launch_resolve_f64(rrtb_ctx *ctx, const uint64_t *d_accum, double *d_out, size_t n);
 int launch_accumulate(rrtb_ctx *ctx, uint64_t *d_dst, const uint64_t *d_src, size_t n);
-int launch_trace(rrtb_ctx *ctx, const float *d_rays7, int n, float t_min, int mode, int32_t *d_id, float *d_t,
-                 float *d_rec7);
-int launch_camera_rays(rrtb_ctx *ctx, const rrtb_render_params *p, const int32_t *d_pix, int n, int sample,
-                       float *d_rays7);
 int launch_philox(rrtb_ctx *ctx, const uint32_t *d_ctr, int n, uint32_t k0, uint32_t k1, uint32_t *d_out);
 int launch_probe(rrtb_ctx *ctx, int mix, double *lane_instr_per_s);
-int launch_scatter(rrtb_ctx *ctx, const float *d_in16, const uint32_t *d_rnd4, int n, float *d_out8);
-// the double integrator's hooks (rrtb_render_f64.cuh)
-int launch_trace_f64(rrtb_ctx *ctx, const double *d_rays7, int n, double t_min, int mode, int32_t *d_id, double *d_t,
-                     double *d_rec7);
-int launch_camera_rays_f64(rrtb_ctx *ctx, const rrtb_render_params *p, const int32_t *d_pix, int n, int sample,
-                           double *d_rays7);
-int launch_scatter_f64(rrtb_ctx *ctx, const double *d_in16, const uint32_t *d_rnd4, int n, double *d_out8);
+// T / real = float: the float integrator and framebuffer, double: the double ones (instantiated for both)
+template <typename T>
+int launch_resolve(rrtb_ctx *ctx, const uint64_t *d_accum, T *d_out, size_t n);
+template <typename real>
+int launch_trace(rrtb_ctx *ctx, const real *d_rays7, int n, real t_min, int mode, int32_t *d_id, real *d_t, real *d_rec7);
+template <typename real>
+int launch_camera_rays(rrtb_ctx *ctx, const rrtb_render_params *p, const int32_t *d_pix, int n, int sample, real *d_rays7);
+template <typename real>
+int launch_scatter(rrtb_ctx *ctx, const real *d_in16, const uint32_t *d_rnd4, int n, real *d_out8);
 
 } // namespace rrtb
