@@ -158,7 +158,9 @@ enum { RRTB_PRECISION_F32 = 0, RRTB_PRECISION_F64 = 1 };
 
 typedef struct rrtb_render_params {
     int32_t width, height;     /* -w -h   (main.cpp:56-57) */
-    int32_t spp;               /* -s      (main.cpp:58)    */
+    int32_t spp;               /* -s      (main.cpp:58); 1 <= spp <= 2^23.  Each sample's radiance is clamped to
+                                 C = min(2^20, 2^(23 - ceil(log2 spp))) before the 2^40 fixed-point sum, so no pixel
+                                 sum passes 2^63 whatever the albedos; C >= 1 never clips radiance <= 1 */
     int32_t max_depth;         /* -d      (main.cpp:66)    */
     uint64_t seed;             /* Philox key; the reference's seed constant is 1984 (rrt.cu:88) */
     int32_t rank, world;       /* this context renders shard `rank` of `world` (1 GPU: 0,1) */
@@ -187,8 +189,9 @@ typedef struct rrtb_stats {
  * writes 3*W*H floats (RGB sums) to the HOST buffer out_rgb. Pixels outside the shard are 0. */
 int rrtb_render(rrtb_ctx *ctx, const rrtb_render_params *p, float *out_rgb, rrtb_stats *stats);
 /* The same render handed back as DOUBLE sums -- what the reference's `rrtd` build returns (FP_T = double,
- * rtweekend.h:20-28; Makefile:36-37).  The 64-bit fixed-point accumulators convert to double exactly, so this is
- * the framebuffer of the `rrtd` drop-in; rays, RNG and intersection arithmetic are those of rrtb_render. */
+ * rtweekend.h:20-28; Makefile:36-37).  A 64-bit fixed-point accumulator converts to double exactly while it is below
+ * 2^53 (a pixel sum below 8192 at 2^40 per unit of radiance), and is rounded once above that; this is the framebuffer
+ * of the `rrtd` drop-in; rays, RNG and intersection arithmetic are those of rrtb_render. */
 int rrtb_render_f64(rrtb_ctx *ctx, const rrtb_render_params *p, double *out_rgb, rrtb_stats *stats);
 
 /* Device-resident entry points (used by the multi-GPU host and bench.py):

@@ -848,10 +848,10 @@ void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int
     /* exceeded depth: black (rrt.cu:78) */
 }
 
-static inline uint64_t to_fixed(float x) /* value * 2^40, round to nearest even, clamped to [0, 2^20] */
+static inline uint64_t to_fixed(float x, float clamp) /* value * 2^40, round to nearest even, clamped to [0, clamp] */
 {
     if (!(x > 0.0f)) return 0;
-    if (x > 1048576.0f) x = 1048576.0f;
+    if (x > clamp) x = clamp;
     return (uint64_t)llrint((double)x * 1099511627776.0);
 }
 
@@ -861,6 +861,7 @@ void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, i
     orc_counters total;
     memset(&total, 0, sizeof(total));
     int tiles_x = (W + 7) / 8;
+    const float clamp = orc_fixed_clamp(spp); /* the total spp: every shard clamps alike */
     if (world < 1) world = 1;
 #pragma omp parallel
     {
@@ -881,7 +882,7 @@ void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, i
                         if (world > 1 && shard_mode == RRTB_SHARD_SAMPLES && (sm % world) != rank) continue;
                         float rgb[3];
                         orc_path(s, bvh, W, H, pixel, sm, max_depth, seed, rgb, &local);
-                        for (int k = 0; k < 3; ++k) acc[k] += to_fixed(rgb[k]);
+                        for (int k = 0; k < 3; ++k) acc[k] += to_fixed(rgb[k], clamp);
                     }
                 }
                 for (int k = 0; k < 3; ++k) {

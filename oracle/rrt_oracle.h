@@ -75,8 +75,19 @@ void orc_trace_bvh(const orc_scene *s, const orc_bvh *b, const float *rays7, int
 /* material.h scatter with an explicit Philox block. in16/out8 as rrtb_scatter. */
 void orc_scatter(const orc_scene *s, const float *in16, const uint32_t *rnd4, int n, float *out8);
 
+/* per-sample radiance clamp of a render of spp samples in all: min(2^20, 2^(23 - ceil(log2 spp))), so that a pixel's
+ * sum of spp fixed-point samples stays <= 2^63 (the product's fixed_clamp, rrt_b200/csrc/rrtb_device.cuh) */
+static inline float orc_fixed_clamp(int spp)
+{
+    int lg = 0;
+    while (lg < 31 && (1u << lg) < (unsigned)spp) ++lg;
+    int e = 23 - lg;
+    return (float)(1u << (e > 20 ? 20 : (e < 0 ? 0 : e)));
+}
+
 /* the estimator (rrt.cu:42-79,109-121 semantics, product RNG). out_rgb = 3*W*H float sums, bottom-up.
- * bvh may be NULL (flat scan). Pixels with (tile_index % world) != rank are left 0 when world > 1. */
+ * bvh may be NULL (flat scan). Pixels with (tile_index % world) != rank are left 0 when world > 1.
+ * Each sample's radiance is clamped to orc_fixed_clamp(spp) (spp = the whole render's, also for a shard). */
 void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, int max_depth, uint64_t seed,
                 int rank, int world, int shard_mode, float *out_rgb, uint64_t *out_fixed, orc_counters *cnt);
 /* ray_color for an explicit primary ray ((pixel, sample) only key the bounce RNG) */

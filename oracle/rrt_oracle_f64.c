@@ -443,10 +443,10 @@ static void path_d(const orc_scene *s, const orc_bvh *bvh, int W, int H, int pix
     }
 }
 
-static inline uint64_t to_fixed_d(double x)
+static inline uint64_t to_fixed_d(double x, double clamp)
 {
     if (!(x > 0.0)) return 0;
-    if (x > 1048576.0) x = 1048576.0;
+    if (x > clamp) x = clamp;
     return (uint64_t)llrint(x * 1099511627776.0);
 }
 
@@ -456,6 +456,7 @@ void orc_d_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp,
 {
     orc_counters total;
     memset(&total, 0, sizeof(total));
+    const double clamp = orc_fixed_clamp(spp);
 #pragma omp parallel
     {
         orc_counters local;
@@ -468,7 +469,7 @@ void orc_d_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp,
                 for (int sm = 0; sm < spp; ++sm) {
                     double rgb[3];
                     path_d(s, bvh, W, H, pixel, sm, max_depth, seed, rgb, &local);
-                    for (int k = 0; k < 3; ++k) acc[k] += to_fixed_d(rgb[k]);
+                    for (int k = 0; k < 3; ++k) acc[k] += to_fixed_d(rgb[k], clamp);
                 }
                 for (int k = 0; k < 3; ++k) {
                     if (out_fixed) out_fixed[3 * (size_t)pixel + k] = acc[k];

@@ -425,6 +425,7 @@ static int check_render(rrtb_ctx *ctx, const rrtb_render_params *p)
     }
     if (p->width < 2 || p->height < 2) return invalid(ctx, "image must be at least 2x2 (u = (i+xi)/(W-1), rrt.cu:112)");
     if (p->spp < 1 || p->max_depth < 0) return invalid(ctx, "spp must be >= 1 and max_depth >= 0");
+    if (p->spp > rrtb::MAX_SPP) return invalid(ctx, "spp must be <= 2^23 (64-bit fixed-point pixel sums, rrtb_device.cuh fixed_clamp)");
     if ((long long)p->width * p->height >= (1ll << 28)) return invalid(ctx, "image too large (limit 2^28 pixels)");
     if (p->rank < 0 || p->rank >= (p->world > 1 ? p->world : 1)) return invalid(ctx, "rank out of range (0 <= rank < max(world, 1))");
     if (p->shard_mode != RRTB_SHARD_TILES && p->shard_mode != RRTB_SHARD_SAMPLES) return invalid(ctx, "bad shard_mode");

@@ -779,12 +779,25 @@ __device__ __forceinline__ void sky(const Ray &r, float &cr, float &cg, float &c
     cb = fmaf(t, 1.0f, w);
 }
 
+// The per-sample radiance clamp of a render of spp samples in all (every shard uses the same value):
+// C = min(2^20, 2^(23 - ceil(log2 spp))), a power of two, so that spp * C * 2^40 <= 2^63 and no pixel sum can wrap,
+// whatever the albedos.  spp <= 2^23 (rrtb_render_params.spp): C >= 1, so radiance <= 1 (sky through albedos
+// <= 1) is never clipped and such images do not depend on the rule.
+static constexpr int MAX_SPP = 1 << 23;
+__host__ __device__ inline float fixed_clamp(int spp)
+{
+    int lg = 0; // ceil(log2 spp)
+    while (lg < 31 && (1u << lg) < (unsigned)spp) ++lg;
+    const int e = 23 - lg;
+    return (float)(1u << (e > 20 ? 20 : (e < 0 ? 0 : e)));
+}
+
 // radiance -> 2^40 fixed point (integer accumulation is associative => bit-reproducible images under
-// any scheduling, sharding or reduction order)
-__device__ __forceinline__ unsigned long long to_fixed(float x)
+// any scheduling, sharding or reduction order), clamped to [0, fixed_clamp(spp)]
+__device__ __forceinline__ unsigned long long to_fixed(float x, float clamp)
 {
     if (!(x > 0.0f)) return 0ull;
-    x = fminf(x, 1048576.0f);
+    x = fminf(x, clamp);
     return __double2ull_rn((double)x * 1099511627776.0);
 }
 

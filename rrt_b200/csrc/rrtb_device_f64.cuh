@@ -354,10 +354,11 @@ __device__ __forceinline__ void sky_d(const RayD &r, double tr, double tg, doubl
     cb = __dmul_rn(tb, __fma_rn(t, 1.0, w));
 }
 
-__device__ __forceinline__ unsigned long long to_fixed_d(double x)
+// radiance -> 2^40 fixed point, clamped to [0, clamp] (to_fixed in rrtb_device.cuh)
+__device__ __forceinline__ unsigned long long to_fixed_d(double x, double clamp)
 {
     if (!(x > 0.0)) return 0ull;
-    x = fmin(x, 1048576.0);
+    x = fmin(x, clamp);
     return __double2ull_rn(__dmul_rn(x, 1099511627776.0));
 }
 

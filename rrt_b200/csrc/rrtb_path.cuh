@@ -52,15 +52,15 @@ struct PathF32 { // the float integrator (rrtb_device.cuh)
         return scatter(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
     }
     static __device__ __forceinline__ float mul(float x, float y) { return x * y; }
-    // sky x throughput -> fixed point (rrt.cu:68-75)
-    static __device__ __forceinline__ void sky_fixed(const Ray &r, float tr, float tg, float tb, unsigned long long &fr,
+    // sky x throughput -> fixed point (rrt.cu:68-75), clamped to fixed_clamp(spp)
+    static __device__ __forceinline__ void sky_fixed(const Ray &r, float tr, float tg, float tb, float clamp, unsigned long long &fr,
                                                      unsigned long long &fg, unsigned long long &fb)
     {
         float cr, cg, cb;
         sky(r, cr, cg, cb);
-        fr = to_fixed(tr * cr);
-        fg = to_fixed(tg * cg);
-        fb = to_fixed(tb * cb);
+        fr = to_fixed(tr * cr, clamp);
+        fg = to_fixed(tg * cg, clamp);
+        fb = to_fixed(tb * cb, clamp);
     }
     static __device__ __forceinline__ Ray camera(const DeviceCamera &cam, int W, int H, int i, int j, int sample, uint2 key)
     {
@@ -108,14 +108,14 @@ struct PathF64 { // the double integrator (rrtb_device_f64.cuh); bit-exact again
         return scatter_d(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
     }
     static __device__ __forceinline__ double mul(double x, double y) { return __dmul_rn(x, y); }
-    static __device__ __forceinline__ void sky_fixed(const RayD &r, double tr, double tg, double tb, unsigned long long &fr,
+    static __device__ __forceinline__ void sky_fixed(const RayD &r, double tr, double tg, double tb, float clamp, unsigned long long &fr,
                                                      unsigned long long &fg, unsigned long long &fb)
     {
         double lr, lg, lb;
         sky_d(r, tr, tg, tb, lr, lg, lb);
-        fr = to_fixed_d(lr);
-        fg = to_fixed_d(lg);
-        fb = to_fixed_d(lb);
+        fr = to_fixed_d(lr, clamp);
+        fg = to_fixed_d(lg, clamp);
+        fb = to_fixed_d(lb, clamp);
     }
     static __device__ __forceinline__ RayD camera(const DeviceCamera &cam, int W, int H, int i, int j, int sample, uint2 key)
     {

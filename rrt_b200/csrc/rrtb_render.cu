@@ -41,6 +41,7 @@ struct RenderArgs {
     DeviceScene scene;
     DeviceCamera cam;
     int W, H, spp, max_depth;
+    float clamp; // per-sample radiance clamp of the whole render, fixed_clamp(spp)
     uint2 key;
     int rank, world, shard_mode;
     int tiles_x, tiles_y;
@@ -127,7 +128,7 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
             bool path_end = false;
             if (h.ref < 0) { // sky x throughput (rrt.cu:68-75)
                 unsigned long long fr, fg, fb;
-                P::sky_fixed(ray, thr_r, thr_g, thr_b, fr, fg, fb);
+                P::sky_fixed(ray, thr_r, thr_g, thr_b, a.clamp, fr, fg, fb);
                 acc_r += fr;
                 acc_g += fg;
                 acc_b += fb;
@@ -464,6 +465,7 @@ int launch_render(rrtb_ctx *ctx, const rrtb_render_params *p, uint64_t *d_accum,
     a.W = p->width;
     a.H = p->height;
     a.spp = p->spp;
+    a.clamp = fixed_clamp(p->spp); // the total spp, not the shard's: every shard clamps alike
     a.max_depth = p->max_depth;
     a.key = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
     a.world = g.world;

@@ -166,7 +166,7 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
                 typename P::RayT r;
                 r.dx = wp.dx[sl]; r.dy = wp.dy[sl]; r.dz = wp.dz[sl];
                 unsigned long long fr, fg, fb;
-                P::sky_fixed(r, wp.tr[sl], wp.tg[sl], wp.tb[sl], fr, fg, fb);
+                P::sky_fixed(r, wp.tr[sl], wp.tg[sl], wp.tb[sl], a.clamp, fr, fg, fb);
                 unsigned long long *dst = a.accum + 3ull * (unsigned long long)wp.pixel[sl];
                 atomicAdd(dst + 0, fr);
                 atomicAdd(dst + 1, fg);
