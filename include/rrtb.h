@@ -42,7 +42,11 @@ typedef enum rrtb_status {
 /* ---- scene vocabulary (reference scene.h:43-54,183-208; camera.h:40-48) ------------------------
  * All float, exactly the values the reference's float build (`rrt`) would hold. */
 
-enum { RRTB_LAMBERTIAN = 0, RRTB_METAL = 1, RRTB_DIELECTRIC = 2 }; /* scene.h:183 */
+/* RRTB_DIFFUSE_LIGHT (book 2's diffuse_light; the reference has no lights): an emitter.  It emits its albedo as the
+ * radiance Le on both faces and never scatters: a segment that hits it ends the path and adds throughput x Le to the
+ * pixel, clamped by the same per-sample clamp C as the sky (rrtb_render_params.spp), so emitted radiance above C is
+ * clipped (at spp = 2^23, C = 1).  Le is not validated, as albedos are not; a negative component adds 0. */
+enum { RRTB_LAMBERTIAN = 0, RRTB_METAL = 1, RRTB_DIELECTRIC = 2, RRTB_DIFFUSE_LIGHT = 3 }; /* scene.h:183 */
 
 typedef struct rrtb_camera { /* the derived fields of camera.h:8-29 */
     float origin[3];
@@ -55,8 +59,8 @@ typedef struct rrtb_camera { /* the derived fields of camera.h:8-29 */
 } rrtb_camera;
 
 typedef struct rrtb_material {
-    int32_t type;    /* RRTB_LAMBERTIAN | RRTB_METAL | RRTB_DIELECTRIC */
-    float albedo[3]; /* lambertian, metal */
+    int32_t type;    /* RRTB_LAMBERTIAN | RRTB_METAL | RRTB_DIELECTRIC | RRTB_DIFFUSE_LIGHT */
+    float albedo[3]; /* lambertian, metal; diffuse_light: emitted radiance Le */
     float param;     /* metal: fuzz (clamped to <= 1 at use, material.h:48); dielectric: index of refraction */
 } rrtb_material;
 
@@ -132,6 +136,10 @@ int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *m
 /* Stage moving triangles (SURVEY 8f4) for the NEXT rrtb_scene_set / rrtb_scene_upload on this context, which
  * consumes them (a later rrtb_scene_set without a new staging call has none).  n == 0 clears the stage. */
 int rrtb_scene_stage_moving_triangles(rrtb_ctx *ctx, const rrtb_mtriangle *mtriangles, int n_mtriangles);
+/* Stage a constant background for the NEXT rrtb_scene_set / rrtb_scene_upload on this context, with the same staging
+ * rule: a segment that leaves the scene adds throughput x rgb3 instead of the reference's sky (rrt.cu:68-75).
+ * rgb3 == NULL clears the stage; a rrtb_scene_set without a staged background renders with the sky, bit for bit. */
+int rrtb_scene_stage_background(rrtb_ctx *ctx, const float *rgb3);
 /* Replace only the camera (animation frames that differ in the camera only; SURVEY f2).  The primitives stay on the
  * device.  If the scene has moving primitives and the shutter interval changed (their boxes span it, rrt.cu:169), or
  * the camera moved farther from the origin than the one the traversal boxes were padded for, the LBVH is rebuilt on
@@ -292,13 +300,18 @@ int rrtb_scatter_f64(rrtb_ctx *ctx, const double *in16, const uint32_t *rnd4, in
 
 typedef struct rrtb_scene rrtb_scene;
 
-/* Two grammar EXTENSIONS (SURVEY 8f4; lines the reference ignores silently, like any unknown prefix):
+/* Grammar EXTENSIONS (SURVEY 8f4 and lights; lines the reference ignores silently, like any unknown prefix, or, for
+ * an unknown material type, rejects with exit code 3):
  *   mobj <obj index> <material> <dx> <dy> <dz> <time0> <time1> [t x y z | s x y z | r deg x y z]...
  * = `obj` (scene.h:387-427) whose instance, placed by the transforms at time0, translates by (dx, dy, dz) until
  * time1 -- the instance counterpart of `msphere c0 c1 time0 time1 r material`;
  *   kobj <obj index> <material> <time0> <time1> [transforms of the pose at time0]... / [transforms of the pose at time1]...
  * = an instance KEYFRAMED between two poses (any mix of translation, rotation and scale; the word `/` separates the
- * two transform lists): every vertex moves linearly from its place in the first pose to its place in the second.
+ * two transform lists): every vertex moves linearly from its place in the first pose to its place in the second;
+ *   material <name> diffuse_light <r> <g> <b>
+ * = an emitter (RRTB_DIFFUSE_LIGHT) of radiance (r, g, b);
+ *   background <r> <g> <b>
+ * = the constant background of rrtb_scene_stage_background; the LAST background line wins, as for `camera`.
  * On failure *out = NULL and *ref_exit_code (optional) receives the exit code the reference would
  * have used (1, 2, 3 or 4); err/err_len (optional) receive the reference's message. */
 int rrtb_scene_parse_file(const char *path, int image_width, int image_height, rrtb_scene **out,
@@ -314,7 +327,9 @@ const rrtb_triangle *rrtb_scene_triangles(const rrtb_scene *s);
 /* moving triangles of `mobj` instances (grammar extension, see rrtb_scene_parse_file) */
 int rrtb_scene_mtriangle_count(const rrtb_scene *s);
 const rrtb_mtriangle *rrtb_scene_mtriangles(const rrtb_scene *s);
-/* rrtb_scene_set with a parsed scene. */
+/* 1 and rgb3 = the file's `background` (grammar extension), or 0 (rgb3 untouched) if it has none: the sky */
+int rrtb_scene_background(const rrtb_scene *s, float *rgb3);
+/* rrtb_scene_set with a parsed scene (its moving triangles and background staged first). */
 int rrtb_scene_upload(rrtb_ctx *ctx, const rrtb_scene *s, int use_bvh);
 /* camera.h:8-29 in the reference's float arithmetic. */
 int rrtb_camera_derive(const float lookfrom[3], const float lookat[3], const float vup[3], float vfov,

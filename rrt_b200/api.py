@@ -65,6 +65,7 @@ class Scene:
             cnt = (C.c_int32 * 6)()
             lib.rrtb_scene_counts(h, cnt)
             nm, ns, nms, nt, nobj, ninst = list(cnt)
+            bg = np.zeros(3, np.float32)
 
             def grab(ptr, n, dt):
                 if n == 0 or not ptr:
@@ -79,6 +80,7 @@ class Scene:
                 grab(lib.rrtb_scene_mspheres(h), nms, msphere_dtype),
                 grab(lib.rrtb_scene_triangles(h), nt, triangle_dtype),
                 grab(lib.rrtb_scene_mtriangles(h), lib.rrtb_scene_mtriangle_count(h), mtriangle_dtype),
+                background=bg if lib.rrtb_scene_background(h, _vp(bg)) else None,
             )
         finally:
             lib.rrtb_scene_free(h)
@@ -201,6 +203,7 @@ class Context:
         a = scene.arrays if isinstance(scene, Scene) else scene
         # SURVEY 8f4: moving triangles are staged, then consumed by rrtb_scene_set
         self._check(self.lib.rrtb_scene_stage_moving_triangles(self.h, _vp(a.mtriangles), len(a.mtriangles)))
+        self._check(self.lib.rrtb_scene_stage_background(self.h, _vp(a.background)))  # None: the sky
         self._check(
             self.lib.rrtb_scene_set(
                 self.h, _vp(a.camera), _vp(a.materials), len(a.materials), _vp(a.spheres), len(a.spheres),

@@ -196,14 +196,25 @@ int rrtb_scene_stage_moving_triangles(rrtb_ctx *ctx, const rrtb_mtriangle *mtria
     return RRTB_OK;
 }
 
+int rrtb_scene_stage_background(rrtb_ctx *ctx, const float *rgb3)
+{
+    if (!ctx) return RRTB_ERR_INVALID;
+    ctx->staged_background = rgb3 != nullptr;
+    for (int k = 0; k < 3; ++k) ctx->staged_bg[k] = rgb3 ? rgb3[k] : 0.f;
+    return RRTB_OK;
+}
+
 int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *materials, int n_materials,
                    const rrtb_sphere *spheres, int n_spheres, const rrtb_msphere *mspheres, int n_mspheres,
                    const rrtb_triangle *triangles, int n_triangles, int use_bvh)
 {
     if (!ctx) return RRTB_ERR_INVALID;
-    // staged moving triangles (SURVEY 8f4) belong to this call whether it succeeds or not
+    // staged moving triangles (SURVEY 8f4) and background belong to this call whether it succeeds or not
     std::vector<rrtb_mtriangle> mtri;
     mtri.swap(ctx->staged_mtriangles);
+    const bool background = ctx->staged_background;
+    const float bg[3] = {ctx->staged_bg[0], ctx->staged_bg[1], ctx->staged_bg[2]};
+    ctx->staged_background = false;
     const int n_mtriangles = (int)mtri.size();
     if (!cam || !materials || n_materials <= 0) return invalid(ctx, "scene needs a camera and at least one material");
     if (n_spheres < 0 || n_mspheres < 0 || n_triangles < 0) return invalid(ctx, "negative primitive count");
@@ -214,8 +225,11 @@ int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *m
         return invalid(ctx, "null primitive array");
     const int n = (int)n_ll;
     // everything is validated BEFORE the loaded scene is touched: a rejected call leaves it renderable
-    for (int i = 0; i < n_materials; ++i)
-        if (materials[i].type < 0 || materials[i].type > 2) return invalid(ctx, "unknown material type");
+    bool emitters = false;
+    for (int i = 0; i < n_materials; ++i) {
+        if (materials[i].type < RRTB_LAMBERTIAN || materials[i].type > RRTB_DIFFUSE_LIGHT) return invalid(ctx, "unknown material type");
+        emitters |= materials[i].type == RRTB_DIFFUSE_LIGHT;
+    }
     for (int i = 0; i < n_spheres; ++i)
         if (spheres[i].material < 0 || spheres[i].material >= n_materials) return invalid(ctx, "sphere material index out of range");
     for (int i = 0; i < n_mspheres; ++i) {
@@ -239,6 +253,9 @@ int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *m
     ctx->n_prims = n;
     ctx->use_bvh = use_bvh ? 1 : 0;
     ctx->motion = use_motion_nodes(n_mspheres + n_mtriangles, cam);
+    ctx->background = background;
+    for (int k = 0; k < 3; ++k) ctx->bg[k] = bg[k];
+    ctx->lights = emitters || background;
 
     int rc;
     const int nb = (n + 255) / 256;

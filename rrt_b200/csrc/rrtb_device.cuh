@@ -694,11 +694,21 @@ __device__ __forceinline__ void sample_unit_sphere(float x0, float x1, float &ux
     uz = z;
 }
 
-// returns true if the path continues; (dx,dy,dz) = scattered direction, (ar,ag,ab) = attenuation
+// returns true if the path continues; (dx,dy,dz) = scattered direction, (ar,ag,ab) = attenuation.
+// LIGHTS: the scene may hold emitters (RRTB_DIFFUSE_LIGHT), which never scatter: direction 0, (ar,ag,ab) = Le.  Without
+// it type 3 is not tested for (launch_render picks LIGHTS kernels for every scene that has an emitter).
+template <bool LIGHTS = false>
 __device__ __forceinline__ bool scatter(int mtype, float4 m, const Ray &r, const HitRecord &rec, uint4 rnd, float &dx,
                                         float &dy, float &dz, float &ar, float &ag, float &ab)
 {
     const float nx = rec.nx, ny = rec.ny, nz = rec.nz;
+    if (LIGHTS && mtype == RRTB_DIFFUSE_LIGHT) { // book 2 diffuse_light::scatter
+        dx = dy = dz = 0.0f;
+        ar = m.x;
+        ag = m.y;
+        ab = m.z;
+        return false;
+    }
     if (mtype == 0) { // lambertian, material.h:21-32
         float ux, uy, uz;
         sample_unit_sphere(u01(rnd.x), u01(rnd.y), ux, uy, uz);

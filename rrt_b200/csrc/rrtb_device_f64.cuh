@@ -271,10 +271,19 @@ __device__ __forceinline__ void sample_unit_sphere_d(double x0, double x1, doubl
     uz = z;
 }
 
+// LIGHTS: as scatter in rrtb_device.cuh
+template <bool LIGHTS = false>
 __device__ __forceinline__ bool scatter_d(int mtype, float4 m, const RayD &r, const HitRecordD &rec, uint4 rnd, double &dx,
                                           double &dy, double &dz, double &ar, double &ag, double &ab)
 {
     const double nx = rec.nx, ny = rec.ny, nz = rec.nz;
+    if (LIGHTS && mtype == RRTB_DIFFUSE_LIGHT) {
+        dx = dy = dz = 0.0;
+        ar = m.x;
+        ag = m.y;
+        ab = m.z;
+        return false;
+    }
     if (mtype == 0) {
         double ux, uy, uz;
         sample_unit_sphere_d(u01d(rnd.x), u01d(rnd.y), ux, uy, uz);

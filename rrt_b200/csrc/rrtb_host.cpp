@@ -129,6 +129,8 @@ struct rrtb_scene {
     std::vector<rrtb_triangle> triangles;
     std::vector<rrtb_mtriangle> mtriangles; // of `mobj` instances
     int n_objs = 0, n_obj_insts = 0;
+    bool has_background = false; // `background r g b` (grammar extension): replaces the sky
+    float background[3] = {0.f, 0.f, 0.f};
 };
 
 extern "C" {
@@ -235,12 +237,29 @@ int rrtb_scene_parse_file(const char *path, int image_width, int image_height, r
                     m.type = RRTB_DIELECTRIC;
                     m.param = to_f(r);
                 }
+                else if (type == "diffuse_light") { // grammar extension (include/rrtb.h): albedo = emitted radiance
+                    std::string r, g, b;
+                    iss >> r >> g >> b;
+                    m.type = RRTB_DIFFUSE_LIGHT;
+                    m.albedo[0] = to_f(r);
+                    m.albedo[1] = to_f(g);
+                    m.albedo[2] = to_f(b);
+                }
                 else {
                     throw ParseError{3, "ERROR: unknown material type: " + type};
                 }
                 int next = (int)sc->materials.size();
                 sc->materials.push_back(m);
                 mat_idx.insert(std::pair<std::string, int>(name, next)); // first definition of a name wins
+            }
+            else if (line.find("background") == 0) { // grammar extension (include/rrtb.h); the LAST background line wins
+                std::istringstream iss(line);
+                std::string kw, r, g, b;
+                iss >> kw >> r >> g >> b;
+                sc->background[0] = to_f(r);
+                sc->background[1] = to_f(g);
+                sc->background[2] = to_f(b);
+                sc->has_background = true;
             }
             else if (line.find("sphere") == 0) { // scene.h:295-312
                 std::istringstream iss(line);
@@ -449,11 +468,19 @@ const rrtb_msphere *rrtb_scene_mspheres(const rrtb_scene *s) { return s ? s->msp
 const rrtb_triangle *rrtb_scene_triangles(const rrtb_scene *s) { return s ? s->triangles.data() : nullptr; }
 int rrtb_scene_mtriangle_count(const rrtb_scene *s) { return s ? (int)s->mtriangles.size() : 0; }
 const rrtb_mtriangle *rrtb_scene_mtriangles(const rrtb_scene *s) { return s ? s->mtriangles.data() : nullptr; }
+int rrtb_scene_background(const rrtb_scene *s, float *rgb3)
+{
+    if (!s || !s->has_background) return 0;
+    if (rgb3)
+        for (int k = 0; k < 3; ++k) rgb3[k] = s->background[k];
+    return 1;
+}
 
 int rrtb_scene_upload(rrtb_ctx *ctx, const rrtb_scene *s, int use_bvh)
 {
     if (!ctx || !s) return RRTB_ERR_INVALID;
     int rc = rrtb_scene_stage_moving_triangles(ctx, s->mtriangles.data(), (int)s->mtriangles.size());
+    if (rc == RRTB_OK) rc = rrtb_scene_stage_background(ctx, s->has_background ? s->background : nullptr);
     if (rc != RRTB_OK) return rc;
     return rrtb_scene_set(ctx, &s->cam, s->materials.data(), (int)s->materials.size(), s->spheres.data(),
                           (int)s->spheres.size(), s->mspheres.data(), (int)s->mspheres.size(), s->triangles.data(),

@@ -22,6 +22,11 @@ struct rrtb_ctx {
     rrtb_camera cam{};
     int n_materials = 0, n_spheres = 0, n_mspheres = 0, n_triangles = 0, n_mtriangles = 0, n_prims = 0;
     std::vector<rrtb_mtriangle> staged_mtriangles; // rrtb_scene_stage_moving_triangles -> next rrtb_scene_set
+    bool staged_background = false;                // rrtb_scene_stage_background -> next rrtb_scene_set
+    float staged_bg[3] = {0.f, 0.f, 0.f};
+    bool background = false;                       // the loaded scene has a constant background bg instead of the sky
+    float bg[3] = {0.f, 0.f, 0.f};
+    bool lights = false;                           // ... or a RRTB_DIFFUSE_LIGHT material: render with the LIGHTS kernels
     int use_bvh = 1;
     double seconds_build = 0.0;
 

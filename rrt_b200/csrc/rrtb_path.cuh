@@ -46,10 +46,11 @@ struct PathF32 { // the float integrator (rrtb_device.cuh)
     {
         return hit_record<MTRI>(leaves, info, r, h);
     }
+    template <bool LIGHTS = false>
     static __device__ __forceinline__ bool bounce(int mtype, float4 m, const Ray &r, const HitRecord &rec, uint4 rnd, float &dx,
                                                   float &dy, float &dz, float &ar, float &ag, float &ab)
     {
-        return scatter(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
+        return scatter<LIGHTS>(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
     }
     static __device__ __forceinline__ float mul(float x, float y) { return x * y; }
     // sky x throughput -> fixed point (rrt.cu:68-75), clamped to fixed_clamp(spp)
@@ -61,6 +62,15 @@ struct PathF32 { // the float integrator (rrtb_device.cuh)
         fr = to_fixed(tr * cr, clamp);
         fg = to_fixed(tg * cg, clamp);
         fb = to_fixed(tb * cb, clamp);
+    }
+    // throughput x a constant radiance -> fixed point: the emitted term (Le of a RRTB_DIFFUSE_LIGHT hit, material
+    // albedo) and the background term (a segment that leaves a scene with a background), plain float products as above
+    static __device__ __forceinline__ void const_fixed(float tr, float tg, float tb, float lr, float lg, float lb, float clamp,
+                                                       unsigned long long &fr, unsigned long long &fg, unsigned long long &fb)
+    {
+        fr = to_fixed(tr * lr, clamp);
+        fg = to_fixed(tg * lg, clamp);
+        fb = to_fixed(tb * lb, clamp);
     }
     static __device__ __forceinline__ Ray camera(const DeviceCamera &cam, int W, int H, int i, int j, int sample, uint2 key)
     {
@@ -102,10 +112,11 @@ struct PathF64 { // the double integrator (rrtb_device_f64.cuh); bit-exact again
     {
         return hit_record_d(leaves, info, r, h);
     }
+    template <bool LIGHTS = false>
     static __device__ __forceinline__ bool bounce(int mtype, float4 m, const RayD &r, const HitRecordD &rec, uint4 rnd, double &dx,
                                                   double &dy, double &dz, double &ar, double &ag, double &ab)
     {
-        return scatter_d(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
+        return scatter_d<LIGHTS>(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab);
     }
     static __device__ __forceinline__ double mul(double x, double y) { return __dmul_rn(x, y); }
     static __device__ __forceinline__ void sky_fixed(const RayD &r, double tr, double tg, double tb, float clamp, unsigned long long &fr,
@@ -116,6 +127,14 @@ struct PathF64 { // the double integrator (rrtb_device_f64.cuh); bit-exact again
         fr = to_fixed_d(lr, clamp);
         fg = to_fixed_d(lg, clamp);
         fb = to_fixed_d(lb, clamp);
+    }
+    // the emitted and background terms: __dmul_rn(throughput, (double)L), as oracle/rrt_oracle_f64.c
+    static __device__ __forceinline__ void const_fixed(double tr, double tg, double tb, float lr, float lg, float lb, float clamp,
+                                                       unsigned long long &fr, unsigned long long &fg, unsigned long long &fb)
+    {
+        fr = to_fixed_d(__dmul_rn(tr, (double)lr), clamp);
+        fg = to_fixed_d(__dmul_rn(tg, (double)lg), clamp);
+        fb = to_fixed_d(__dmul_rn(tb, (double)lb), clamp);
     }
     static __device__ __forceinline__ RayD camera(const DeviceCamera &cam, int W, int H, int i, int j, int sample, uint2 key)
     {

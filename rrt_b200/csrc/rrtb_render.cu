@@ -53,9 +53,13 @@ struct RenderArgs {
     int th_fetch, th_shade, th_leaf; // pool-scheduler thresholds (lanes)
     int step_iters, th_node;         // max node visits per scheduling round / lanes needed to continue
     unsigned long long *queue;  // [0] queue head, [1] rays, [2] box tests, [3] sphere, [4] msphere, [5] triangle tests, [6] hits
+    // LIGHTS kernels only (appended, so the fields above keep their parameter offsets)
+    int background;             // != 0: a segment that leaves the scene adds throughput x bg instead of the sky
+    float bg[3];
 };
 
-template <class P, bool USE_BVH, bool COUNT_RAYS>
+// LIGHTS: the scene has emitters (RRTB_DIFFUSE_LIGHT) or a background; the other instantiations compile neither in
+template <class P, bool USE_BVH, bool COUNT_RAYS, bool LIGHTS = false>
 __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
 {
     typedef typename P::real real;
@@ -126,9 +130,10 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
             }
             // ---- shade: rrt.cu:50-76
             bool path_end = false;
-            if (h.ref < 0) { // sky x throughput (rrt.cu:68-75)
+            if (h.ref < 0) { // sky x throughput (rrt.cu:68-75), or background x throughput
                 unsigned long long fr, fg, fb;
-                P::sky_fixed(ray, thr_r, thr_g, thr_b, a.clamp, fr, fg, fb);
+                if (LIGHTS && a.background) P::const_fixed(thr_r, thr_g, thr_b, a.bg[0], a.bg[1], a.bg[2], a.clamp, fr, fg, fb);
+                else P::sky_fixed(ray, thr_r, thr_g, thr_b, a.clamp, fr, fg, fb);
                 acc_r += fr;
                 acc_g += fg;
                 acc_b += fb;
@@ -140,7 +145,7 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
                 float4 m = __ldg(&s.materials[rec.mat]);
                 int mtype = __ldg(&s.material_type[rec.mat]);
                 real dx, dy, dz, ar, ag, ab;
-                if (P::bounce(mtype, m, ray, rec, rnd, dx, dy, dz, ar, ag, ab)) {
+                if (P::template bounce<LIGHTS>(mtype, m, ray, rec, rnd, dx, dy, dz, ar, ag, ab)) {
                     thr_r = P::mul(thr_r, ar);
                     thr_g = P::mul(thr_g, ag);
                     thr_b = P::mul(thr_b, ab);
@@ -153,7 +158,16 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
                     if (++bounce >= a.max_depth) path_end = true; // exceeded depth: black (rrt.cu:78)
                 }
                 else {
-                    path_end = true; // absorbed: black (rrt.cu:61-63)
+                    if constexpr (LIGHTS) { // (if constexpr: the other instantiations keep their code exactly)
+                        if (mtype == RRTB_DIFFUSE_LIGHT) { // an emitter: throughput x Le
+                            unsigned long long fr, fg, fb;
+                            P::const_fixed(thr_r, thr_g, thr_b, m.x, m.y, m.z, a.clamp, fr, fg, fb);
+                            acc_r += fr;
+                            acc_g += fg;
+                            acc_b += fb;
+                        }
+                    }
+                    path_end = true; // absorbed: black (rrt.cu:61-63), or an emitter
                 }
             }
             if (path_end) {
@@ -300,7 +314,7 @@ __global__ void k_scatter_test(const DeviceScene s, const typename P::real *__re
     rec.obj = 0;
     uint4 rnd = make_uint4(rnd4[4 * i], rnd4[4 * i + 1], rnd4[4 * i + 2], rnd4[4 * i + 3]);
     real dx, dy, dz, ar, ag, ab;
-    bool ok = P::bounce(__ldg(&s.material_type[rec.mat]), __ldg(&s.materials[rec.mat]), r, rec, rnd, dx, dy, dz, ar, ag, ab);
+    bool ok = P::template bounce<true>(__ldg(&s.material_type[rec.mat]), __ldg(&s.materials[rec.mat]), r, rec, rnd, dx, dy, dz, ar, ag, ab);
     real *o = out8 + 8 * (size_t)i;
     o[0] = dx; o[1] = dy; o[2] = dz; o[3] = ar; o[4] = ag; o[5] = ab; o[6] = ok ? 1 : 0; o[7] = 0;
 }
@@ -422,10 +436,10 @@ static int grid_size(const rrtb_ctx *ctx, size_t n)
 }
 
 // the lane kernel: persistent, one wave, a multiple of the SM count
-template <class P, bool USE_BVH>
+template <class P, bool USE_BVH, bool LIGHTS = false>
 static int launch_lane(rrtb_ctx *ctx, const RenderArgs &args, bool cnt, int *blocks_out)
 {
-    auto kernel = cnt ? k_render<P, USE_BVH, true> : k_render<P, USE_BVH, false>;
+    auto kernel = cnt ? k_render<P, USE_BVH, true, LIGHTS> : k_render<P, USE_BVH, false, LIGHTS>;
     int per_sm = 0;
     RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, 0));
     if (per_sm < 1) per_sm = 1;
@@ -437,10 +451,10 @@ static int launch_lane(rrtb_ctx *ctx, const RenderArgs &args, bool cnt, int *blo
     return RRTB_OK;
 }
 
-template <class P, bool MTRI, bool MOTION>
+template <class P, bool MTRI, bool MOTION, bool LIGHTS = false>
 static int launch_pool(rrtb_ctx *ctx, const RenderArgs &args, bool cnt, int *blocks_out)
 {
-    auto kernel = cnt ? k_render_pool<true, NODE_UNROLL, MTRI, P, MOTION> : k_render_pool<false, NODE_UNROLL, MTRI, P, MOTION>;
+    auto kernel = cnt ? k_render_pool<true, NODE_UNROLL, MTRI, P, MOTION, LIGHTS> : k_render_pool<false, NODE_UNROLL, MTRI, P, MOTION, LIGHTS>;
     constexpr int POOL = P::POOL;
     const int smem = (int)(sizeof(WarpPoolT<typename P::real, POOL>) * POOL_WARPS);
     RRTB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -500,6 +514,8 @@ int launch_render(rrtb_ctx *ctx, const rrtb_render_params *p, uint64_t *d_accum,
     a.th_leaf = knob("RRTB_TH_LEAF", a.th_leaf, 1, 32);
 #endif
     a.queue = ctx->d_counters;
+    a.background = ctx->background ? 1 : 0;
+    for (int k = 0; k < 3; ++k) a.bg[k] = ctx->bg[k];
 
     RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_counters, 0, 8 * sizeof(unsigned long long), ctx->stream));
     RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
@@ -515,9 +531,16 @@ int launch_render(rrtb_ctx *ctx, const rrtb_render_params *p, uint64_t *d_accum,
         static const Launcher pool[3][2] = {{launch_pool<PathF32, false, false>, launch_pool<PathF32, false, true>},
                                             {launch_pool<PathF32, true, false>, launch_pool<PathF32, true, true>},
                                             {launch_pool<PathF64, true, false>, launch_pool<PathF64, true, true>}};
+        // scenes with emitters or a background (ctx->lights): the LIGHTS kernels, [precision][...] as above; the float pool
+        // kernel compiles the moving-triangle cases in, as the double one does
+        static const Launcher lane_lit[2][2] = {{launch_lane<PathF32, false, true>, launch_lane<PathF32, true, true>},
+                                                {launch_lane<PathF64, false, true>, launch_lane<PathF64, true, true>}};
+        static const Launcher pool_lit[2][2] = {{launch_pool<PathF32, true, false, true>, launch_pool<PathF32, true, true, true>},
+                                                {launch_pool<PathF64, true, false, true>, launch_pool<PathF64, true, true, true>}};
         const int f64 = p->precision == RRTB_PRECISION_F64;
         // motion: moving primitives under an open shutter, the kernels walk interpolating motion nodes
-        const Launcher launch = use_pool ? pool[f64 ? 2 : ctx->n_mtriangles > 0][ctx->motion] : lane[f64][ctx->use_bvh != 0];
+        const Launcher launch = ctx->lights ? (use_pool ? pool_lit[f64][ctx->motion] : lane_lit[f64][ctx->use_bvh != 0])
+                                            : (use_pool ? pool[f64 ? 2 : ctx->n_mtriangles > 0][ctx->motion] : lane[f64][ctx->use_bvh != 0]);
         const int rc = launch(ctx, a, p->count_rays != 0, &blocks);
         if (rc) return rc;
         launches = 1;

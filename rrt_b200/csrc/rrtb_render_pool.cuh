@@ -9,14 +9,15 @@
 //
 //   trace stack    slots whose ray awaits traversal
 //   scatter stack  slots whose segment HIT something  (hit record + material scatter next)
-//   gen stack      slots whose path ENDED (sky, absorbed, depth) or that never held one
+//   gen stack      slots whose path ENDED (sky, absorbed, depth, emitter) or that never held one
 //
 //   FETCH    idle lanes pop the trace stack, load the ray and start a traversal
 //   STEP     lanes in flight visit BVH nodes (the inner loop runs on while a vote finds enough of them),
 //            then, by vote, do one exact leaf test; a lane whose traversal ends writes (t, leaf ref) to its
 //            slot, pushes it on the scatter or the gen stack and is idle at once -- nobody waits for it
-//   SCATTER  32 hit slots, one per lane: hit record, Philox block, scatter; survivors -> trace stack
-//   GEN      32 ended slots, one per lane: sky x throughput into the accumulator (64-bit integer atomics),
+//   SCATTER  32 hit slots, one per lane: hit record, Philox block, scatter; survivors -> trace stack (LIGHTS: an
+//            emitter hit adds throughput x Le to the accumulator here and ends its path)
+//   GEN      32 ended slots, one per lane: sky (LIGHTS: or background) x throughput into the accumulator (64-bit integer atomics),
 //            then the next camera paths of the global queue (ONE warp-aggregated atomicAdd per batch),
 //            Philox block, thin-lens ray -> trace stack
 //
@@ -48,7 +49,8 @@ struct WarpPoolT { // SoA, one per warp, in dynamic shared memory
     unsigned char gq[POOL]; // gen stack
 };
 
-template <bool COUNT_RAYS, int NODE_UNROLL, bool MTRI = false, class P = PathF32, bool MOTION = false>
+// LIGHTS: the scene has emitters (RRTB_DIFFUSE_LIGHT) or a background; the other instantiations compile neither in
+template <bool COUNT_RAYS, int NODE_UNROLL, bool MTRI = false, class P = PathF32, bool MOTION = false, bool LIGHTS = false>
 __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(const RenderArgs a)
 {
     typedef typename P::real real;
@@ -133,7 +135,7 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
                 float4 m = __ldg(&s.materials[rec.mat]);
                 int mtype = __ldg(&s.material_type[rec.mat]);
                 real dx, dy, dz, ar, ag, ab;
-                if (P::bounce(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab) && bounce + 1 < a.max_depth) {
+                if (P::template bounce<LIGHTS>(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab) && bounce + 1 < a.max_depth) {
                     wp.ox[sl] = rec.px; wp.oy[sl] = rec.py; wp.oz[sl] = rec.pz;
                     wp.dx[sl] = dx; wp.dy[sl] = dy; wp.dz[sl] = dz;
                     wp.tr[sl] = P::mul(wp.tr[sl], ar); wp.tg[sl] = P::mul(wp.tg[sl], ag); wp.tb[sl] = P::mul(wp.tb[sl], ab);
@@ -141,6 +143,16 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
                     to_trace = true;
                 }
                 else { // absorbed (rrt.cu:61-63) or depth exhausted (rrt.cu:78): black, nothing to accumulate
+                    if constexpr (LIGHTS) { // ... unless an emitter ended the path: throughput x Le, accumulated here
+                        if (mtype == RRTB_DIFFUSE_LIGHT) {
+                            unsigned long long fr, fg, fb;
+                            P::const_fixed(wp.tr[sl], wp.tg[sl], wp.tb[sl], m.x, m.y, m.z, a.clamp, fr, fg, fb);
+                            unsigned long long *dst = a.accum + 3ull * (unsigned long long)wp.pixel[sl];
+                            atomicAdd(dst + 0, fr);
+                            atomicAdd(dst + 1, fg);
+                            atomicAdd(dst + 2, fb);
+                        }
+                    }
                     wp.hit_ref[sl] = SLOT_FRESH;
                     ended = true;
                 }
@@ -161,12 +173,17 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
             const int sl = mine ? wp.gq[gq_n - 1 - lane] : 0;
             gq_n -= take;
             __syncwarp();
-            if (mine && wp.hit_ref[sl] == -1) { // the segment left the scene: sky x throughput (rrt.cu:68-75)
+            if (mine && wp.hit_ref[sl] == -1) { // the segment left the scene: sky x throughput (rrt.cu:68-75), or background
                 if (COUNT_RAYS) ++rays;
-                typename P::RayT r;
-                r.dx = wp.dx[sl]; r.dy = wp.dy[sl]; r.dz = wp.dz[sl];
                 unsigned long long fr, fg, fb;
-                P::sky_fixed(r, wp.tr[sl], wp.tg[sl], wp.tb[sl], a.clamp, fr, fg, fb);
+                if (LIGHTS && a.background) {
+                    P::const_fixed(wp.tr[sl], wp.tg[sl], wp.tb[sl], a.bg[0], a.bg[1], a.bg[2], a.clamp, fr, fg, fb);
+                }
+                else {
+                    typename P::RayT r;
+                    r.dx = wp.dx[sl]; r.dy = wp.dy[sl]; r.dz = wp.dz[sl];
+                    P::sky_fixed(r, wp.tr[sl], wp.tg[sl], wp.tb[sl], a.clamp, fr, fg, fb);
+                }
                 unsigned long long *dst = a.accum + 3ull * (unsigned long long)wp.pixel[sl];
                 atomicAdd(dst + 0, fr);
                 atomicAdd(dst + 1, fg);

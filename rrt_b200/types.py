@@ -2,12 +2,13 @@
 
 The scene vocabulary is the reference's (scene.h:43-54,183-208; camera.h:40-48): spheres, moving
 spheres, world-space triangles; lambertian / metal / dielectric materials; a derived thin-lens camera.
+Beyond it: diffuse_light emitters (albedo = emitted radiance) and an optional constant background.
 """
 import ctypes as C
 
 import numpy as np
 
-LAMBERTIAN, METAL, DIELECTRIC = 0, 1, 2
+LAMBERTIAN, METAL, DIELECTRIC, DIFFUSE_LIGHT = 0, 1, 2, 3
 SHARD_TILES, SHARD_SAMPLES = 0, 1
 SCHED_AUTO, SCHED_SIMPLE, SCHED_POOL = 0, 1, 2
 
@@ -88,9 +89,10 @@ class Stats(C.Structure):
 
 class SceneArrays:
     """A scene as plain arrays, in the reference's object-id order (spheres, moving spheres, triangles;
-    rrt.cu:151-164), then the moving triangles of SURVEY 8f4."""
+    rrt.cu:151-164), then the moving triangles of SURVEY 8f4.  `background`: None renders the reference's sky,
+    an RGB triple a constant background instead (include/rrtb.h rrtb_scene_stage_background)."""
 
-    def __init__(self, camera, materials, spheres=None, mspheres=None, triangles=None, mtriangles=None):
+    def __init__(self, camera, materials, spheres=None, mspheres=None, triangles=None, mtriangles=None, background=None):
         self.camera = np.ascontiguousarray(np.asarray(camera, dtype=camera_dtype).reshape(1))
         self.materials = np.ascontiguousarray(np.asarray(materials, dtype=material_dtype))
         self.spheres = np.ascontiguousarray(
@@ -105,6 +107,7 @@ class SceneArrays:
         self.mtriangles = np.ascontiguousarray(
             np.zeros(0, mtriangle_dtype) if mtriangles is None else np.asarray(mtriangles, dtype=mtriangle_dtype)
         )
+        self.background = None if background is None else np.ascontiguousarray(np.asarray(background, dtype=np.float32).reshape(3))
 
     @property
     def n_objects(self):
@@ -121,7 +124,7 @@ class SceneArrays:
 
     # ---- (de)serialisation used by the golden fixtures (tests/golden/*.npz) ----
     def to_npz_dict(self):
-        return dict(
+        d = dict(
             camera=self.camera.view(np.uint8),
             materials=self.materials.view(np.uint8),
             spheres=self.spheres.view(np.uint8),
@@ -129,6 +132,9 @@ class SceneArrays:
             triangles=self.triangles.view(np.uint8),
             mtriangles=self.mtriangles.view(np.uint8),
         )
+        if self.background is not None:
+            d["background"] = self.background.copy()
+        return d
 
     @classmethod
     def from_npz_dict(cls, d):
@@ -145,4 +151,5 @@ class SceneArrays:
             v("mspheres", msphere_dtype),
             v("triangles", triangle_dtype),
             v("mtriangles", mtriangle_dtype),
+            background=np.asarray(d["background"], np.float32) if "background" in d else None,  # older fixtures: the sky
         )

@@ -9,15 +9,16 @@ ROOT="$(cd "$(dirname "$0")/.." && pwd)"; W=$(mktemp -d /tmp/rrtb_fuzz.XXXXXX); 
 cat > $W/drv.cpp <<EOF
 #include <stdint.h>
 #include "$ROOT/include/rrtb.h"
-extern "C" { // the two device-side entry points rrtb_host.cpp refers to (rrtb_scene_upload); never called here
+extern "C" { // the device-side entry points rrtb_host.cpp refers to (rrtb_scene_upload); never called here
 int rrtb_scene_stage_moving_triangles(rrtb_ctx *, const rrtb_mtriangle *, int32_t) { return 0; }
+int rrtb_scene_stage_background(rrtb_ctx *, const float *) { return 0; }
 int rrtb_scene_set(rrtb_ctx *, const rrtb_camera *, const rrtb_material *, int32_t, const rrtb_sphere *, int32_t, const rrtb_msphere *, int32_t,
                    const rrtb_triangle *, int32_t, int32_t) { return 0; }
 }
 int main(int argc, char **argv) {
     for (int i = 1; i < argc; ++i) {
         rrtb_scene *s = nullptr; int code = 0; char err[512];
-        if (rrtb_scene_parse_file(argv[i], 320, 200, &s, &code, err, 512) == 0 && s) { int32_t c[6]; rrtb_scene_counts(s, c); rrtb_scene_free(s); }
+        if (rrtb_scene_parse_file(argv[i], 320, 200, &s, &code, err, 512) == 0 && s) { int32_t c[6]; float bg[3]; rrtb_scene_counts(s, c); rrtb_scene_background(s, bg); rrtb_scene_free(s); }
     }
     return 0;
 }
@@ -29,7 +30,7 @@ sc, out, n = sys.argv[1], sys.argv[2], int(sys.argv[3])
 random.seed(7)
 base = [open(p).read() for p in sorted(glob.glob(os.path.join(sc, "*.txt")))]
 toks = ["camera", "material", "sphere", "moving_sphere", "obj", "obj_inst", "triangle", "mobj", "kobj", "lambertian", "metal", "dielectric",
-        "translate", "rotate", "scale", "#", "nan", "inf", "-inf", "1e39", "-1e-50", "0", "m0", "m999", "", "9999999999999999999999", "/", "o0"]
+        "translate", "rotate", "scale", "diffuse_light", "background", "#", "nan", "inf", "-inf", "1e39", "-1e-50", "0", "m0", "m999", "", "9999999999999999999999", "/", "o0"]
 for k in range(n):
     lines = random.choice(base).split("\n")
     how = random.randint(0, 5)
