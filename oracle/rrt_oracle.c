@@ -734,6 +734,11 @@ static f3 sample_unit_sphere(float x0, float x1)
 /* returns 1 if the path continues; dir/atten out */
 static int scatter_one(const rrtb_material *m, f3 d_in, f3 n, int front, const uint32_t rnd[4], f3 *dir, f3 *att)
 {
+    if (m->type == RRTB_DIFFUSE_LIGHT) { /* book 2 diffuse_light: never scatters; att = Le */
+        *dir = F3(0.0f, 0.0f, 0.0f);
+        *att = ld3(m->albedo);
+        return 0;
+    }
     if (m->type == RRTB_LAMBERTIAN) { /* material.h:21-32 */
         f3 u = sample_unit_sphere(orc_u01(rnd[0]), orc_u01(rnd[1]));
         f3 sd = add3(n, u);
@@ -811,9 +816,10 @@ void orc_path(const orc_scene *s, const orc_bvh *bvh, int W, int H, int pixel, i
     orc_radiance(s, bvh, ray7, pixel, sample, max_depth, seed, rgb, cnt);
 }
 
-/* ray_color (rrt.cu:42-79) for an explicit primary ray; (pixel, sample) only key the bounce RNG. */
-void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int pixel, int sample, int max_depth,
-                  uint64_t seed, float *rgb, orc_counters *cnt)
+/* ray_color (rrt.cu:42-79) for an explicit primary ray; (pixel, sample) only key the bounce RNG.  bg: the constant
+ * background that replaces the sky, or NULL for the sky */
+static void radiance(const orc_scene *s, const float *bg, const orc_bvh *bvh, const float *ray7, int pixel, int sample,
+                     int max_depth, uint64_t seed, float *rgb, orc_counters *cnt)
 {
     f3 o = ld3(ray7), d = ld3(ray7 + 3);
     float time = ray7[6];
@@ -824,6 +830,12 @@ void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int
         float t;
         int id = bvh ? closest_bvh(s, bvh, o, d, time, 0.001f, &t, cnt) : closest_scan(s, o, d, time, 0.001f, &t, cnt);
         if (cnt) cnt->rays++;
+        if (id < 0 && bg) {
+            rgb[0] = thr.x * bg[0];
+            rgb[1] = thr.y * bg[1];
+            rgb[2] = thr.z * bg[2];
+            return;
+        }
         if (id < 0) { /* sky, rrt.cu:68-75 */
             float uy = d.y * (1.0f / sqrtf(dot3(d, d)));
             float tt = 0.5f * (uy + 1.0f);
@@ -840,12 +852,25 @@ void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int
         uint32_t rnd[4];
         rng_block(seed, (uint32_t)pixel, (uint32_t)sample, 2u + (uint32_t)b, rnd);
         f3 dir, att;
-        if (!scatter_one(&s->materials[mat], d, ld3(rec + 3), rec[6] != 0.0f, rnd, &dir, &att)) return; /* black */
+        if (!scatter_one(&s->materials[mat], d, ld3(rec + 3), rec[6] != 0.0f, rnd, &dir, &att)) {
+            if (s->materials[mat].type == RRTB_DIFFUSE_LIGHT) { /* emitter: throughput x Le (att = Le) */
+                rgb[0] = thr.x * att.x;
+                rgb[1] = thr.y * att.y;
+                rgb[2] = thr.z * att.z;
+            }
+            return; /* else absorbed: black */
+        }
         thr = F3(thr.x * att.x, thr.y * att.y, thr.z * att.z);
         o = ld3(rec);
         d = dir;
     }
     /* exceeded depth: black (rrt.cu:78) */
+}
+
+void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int pixel, int sample, int max_depth,
+                  uint64_t seed, float *rgb, orc_counters *cnt)
+{
+    radiance(s, NULL, bvh, ray7, pixel, sample, max_depth, seed, rgb, cnt);
 }
 
 static inline uint64_t to_fixed(float x, float clamp) /* value * 2^40, round to nearest even, clamped to [0, clamp] */
@@ -857,6 +882,13 @@ static inline uint64_t to_fixed(float x, float clamp) /* value * 2^40, round to 
 
 void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, int max_depth, uint64_t seed,
                 int rank, int world, int shard_mode, float *out_rgb, uint64_t *out_fixed, orc_counters *cnt)
+{
+    orc_render_bg(s, NULL, bvh, W, H, spp, max_depth, seed, rank, world, shard_mode, out_rgb, out_fixed, cnt);
+}
+
+void orc_render_bg(const orc_scene *s, const float *bg, const orc_bvh *bvh, int W, int H, int spp, int max_depth,
+                   uint64_t seed, int rank, int world, int shard_mode, float *out_rgb, uint64_t *out_fixed,
+                   orc_counters *cnt)
 {
     orc_counters total;
     memset(&total, 0, sizeof(total));
@@ -880,8 +912,9 @@ void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, i
                 if (mine) {
                     for (int sm = 0; sm < spp; ++sm) {
                         if (world > 1 && shard_mode == RRTB_SHARD_SAMPLES && (sm % world) != rank) continue;
-                        float rgb[3];
-                        orc_path(s, bvh, W, H, pixel, sm, max_depth, seed, rgb, &local);
+                        float ray7[7], rgb[3];
+                        orc_camera_ray(&s->cam, W, H, pixel, sm, seed, ray7);
+                        radiance(s, bg, bvh, ray7, pixel, sm, max_depth, seed, rgb, &local);
                         for (int k = 0; k < 3; ++k) acc[k] += to_fixed(rgb[k], clamp);
                     }
                 }

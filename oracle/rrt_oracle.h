@@ -12,6 +12,13 @@
  * (tests/golden/, tools/make_golden.py).
  *
  * The scene structs are the public C ABI ones (include/rrtb.h) so the same arrays feed both sides.
+ *
+ * Lights (DESIGN f5) have no reference counterpart and are parity-unpinned: a RRTB_DIFFUSE_LIGHT material never
+ * scatters and ends the path with throughput x Le (Le = its albedo), and the background of orc_render_bg /
+ * orc_d_render_bg, when not NULL, replaces the sky with throughput x background.  Both terms are float products in the
+ * float integrator and one double product of the float-to-double value per channel in the double one, in the order of
+ * the product's PathF32 / PathF64 ::const_fixed.  A scene without a RRTB_DIFFUSE_LIGHT material, rendered with the
+ * sky, reaches neither term, so on it every entry point is exactly the parity-pinned estimator above.
  */
 #ifndef RRT_ORACLE_H
 #define RRT_ORACLE_H
@@ -72,7 +79,8 @@ void orc_bvh_free(orc_bvh *b);
 void orc_trace_bvh(const orc_scene *s, const orc_bvh *b, const float *rays7, int n, float t_min, int32_t *id,
                    float *t, float *rec7, orc_counters *cnt);
 
-/* material.h scatter with an explicit Philox block. in16/out8 as rrtb_scatter. */
+/* material.h scatter with an explicit Philox block. in16/out8 as rrtb_scatter.  An emitter reports direction 0,
+ * attenuation Le, not scattered. */
 void orc_scatter(const orc_scene *s, const float *in16, const uint32_t *rnd4, int n, float *out8);
 
 /* per-sample radiance clamp of a render of spp samples in all: min(2^20, 2^(23 - ceil(log2 spp))), so that a pixel's
@@ -90,6 +98,10 @@ static inline float orc_fixed_clamp(int spp)
  * Each sample's radiance is clamped to orc_fixed_clamp(spp) (spp = the whole render's, also for a shard). */
 void orc_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, int max_depth, uint64_t seed,
                 int rank, int world, int shard_mode, float *out_rgb, uint64_t *out_fixed, orc_counters *cnt);
+/* orc_render under a constant background: background[3] replaces the sky; NULL is the sky (orc_render) */
+void orc_render_bg(const orc_scene *s, const float *background, const orc_bvh *bvh, int W, int H, int spp, int max_depth,
+                   uint64_t seed, int rank, int world, int shard_mode, float *out_rgb, uint64_t *out_fixed,
+                   orc_counters *cnt);
 /* ray_color for an explicit primary ray ((pixel, sample) only key the bounce RNG) */
 void orc_radiance(const orc_scene *s, const orc_bvh *bvh, const float *ray7, int pixel, int sample, int max_depth,
                   uint64_t seed, float *rgb, orc_counters *cnt);
@@ -114,6 +126,9 @@ void orc_d_trace(const orc_scene *s, const orc_bvh *b, const double *rays7, int 
 void orc_d_scatter(const orc_scene *s, const double *in16, const uint32_t *rnd4, int n, double *out8);
 void orc_d_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, int max_depth, uint64_t seed, double *out_rgb,
                   uint64_t *out_fixed, orc_counters *cnt);
+/* orc_d_render under a constant background, as orc_render_bg */
+void orc_d_render_bg(const orc_scene *s, const float *background, const orc_bvh *bvh, int W, int H, int spp, int max_depth,
+                     uint64_t seed, double *out_rgb, uint64_t *out_fixed, orc_counters *cnt);
 
 /* color.h:8-23 */
 void orc_tonemap_rgb8(const float *rgb_sum, int W, int H, int spp, uint8_t *rgb8_topdown);

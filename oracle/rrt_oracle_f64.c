@@ -344,6 +344,11 @@ static d3 unit_sphere_d(double x0, double x1)
 /* material.h:21-32,48-57,76-109 in double; same Philox block layout as the float integrator */
 static int scatter_d(const rrtb_material *m, d3 d_in, d3 n, int front, const uint32_t rnd[4], d3 *dir, d3 *att)
 {
+    if (m->type == RRTB_DIFFUSE_LIGHT) { /* never scatters; att = (double)Le */
+        *dir = D3(0, 0, 0);
+        *att = ldf(m->albedo);
+        return 0;
+    }
     if (m->type == RRTB_LAMBERTIAN) {
         d3 u = unit_sphere_d(u01d(rnd[0]), u01d(rnd[1]));
         d3 sd = D3(n.x + u.x, n.y + u.y, n.z + u.z);
@@ -407,8 +412,9 @@ void orc_d_scatter(const orc_scene *s, const double *in16, const uint32_t *rnd4,
     }
 }
 
-static void path_d(const orc_scene *s, const orc_bvh *bvh, int W, int H, int pixel, int sample, int max_depth, uint64_t seed,
-                   double *rgb, orc_counters *cnt)
+/* bg: the constant background that replaces the sky, or NULL for the sky */
+static void path_d(const orc_scene *s, const float *bg, const orc_bvh *bvh, int W, int H, int pixel, int sample, int max_depth,
+                   uint64_t seed, double *rgb, orc_counters *cnt)
 {
     double ray7[7];
     orc_d_camera_ray(&s->cam, W, H, pixel, sample, seed, ray7);
@@ -421,6 +427,12 @@ static void path_d(const orc_scene *s, const orc_bvh *bvh, int W, int H, int pix
         double t;
         int id = closest_d(s, bvh, o, d, time, 0.001, &t);
         cnt->rays++;
+        if (id < 0 && bg) {
+            rgb[0] = thr.x * (double)bg[0];
+            rgb[1] = thr.y * (double)bg[1];
+            rgb[2] = thr.z * (double)bg[2];
+            return;
+        }
         if (id < 0) {
             double uy = d.y * (1.0 / sqrt(ddot(d, d)));
             double tt = 0.5 * (uy + 1.0);
@@ -436,7 +448,14 @@ static void path_d(const orc_scene *s, const orc_bvh *bvh, int W, int H, int pix
         uint32_t rnd[4];
         rng_block(seed, (uint32_t)pixel, (uint32_t)sample, 2u + (uint32_t)b, rnd);
         d3 dir, att;
-        if (!scatter_d(&s->materials[mat], d, ldd(rec + 3), rec[6] != 0.0, rnd, &dir, &att)) return;
+        if (!scatter_d(&s->materials[mat], d, ldd(rec + 3), rec[6] != 0.0, rnd, &dir, &att)) {
+            if (s->materials[mat].type == RRTB_DIFFUSE_LIGHT) { /* emitter: throughput x Le (att = (double)Le) */
+                rgb[0] = thr.x * att.x;
+                rgb[1] = thr.y * att.y;
+                rgb[2] = thr.z * att.z;
+            }
+            return; /* else absorbed: black */
+        }
         thr = D3(thr.x * att.x, thr.y * att.y, thr.z * att.z);
         o = ldd(rec);
         d = dir;
@@ -454,6 +473,12 @@ static inline uint64_t to_fixed_d(double x, double clamp)
 void orc_d_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp, int max_depth, uint64_t seed, double *out_rgb,
                   uint64_t *out_fixed, orc_counters *cnt)
 {
+    orc_d_render_bg(s, NULL, bvh, W, H, spp, max_depth, seed, out_rgb, out_fixed, cnt);
+}
+
+void orc_d_render_bg(const orc_scene *s, const float *bg, const orc_bvh *bvh, int W, int H, int spp, int max_depth,
+                     uint64_t seed, double *out_rgb, uint64_t *out_fixed, orc_counters *cnt)
+{
     orc_counters total;
     memset(&total, 0, sizeof(total));
     const double clamp = orc_fixed_clamp(spp);
@@ -468,7 +493,7 @@ void orc_d_render(const orc_scene *s, const orc_bvh *bvh, int W, int H, int spp,
                 uint64_t acc[3] = {0, 0, 0};
                 for (int sm = 0; sm < spp; ++sm) {
                     double rgb[3];
-                    path_d(s, bvh, W, H, pixel, sm, max_depth, seed, rgb, &local);
+                    path_d(s, bg, bvh, W, H, pixel, sm, max_depth, seed, rgb, &local);
                     for (int k = 0; k < 3; ++k) acc[k] += to_fixed_d(rgb[k], clamp);
                 }
                 for (int k = 0; k < 3; ++k) {

@@ -87,7 +87,7 @@ def oracle_lib():
 
 
 class Oracle:
-    """The CPU oracle bound to one scene."""
+    """The CPU oracle bound to one scene, emitters and the scene's background (None: the sky) included."""
 
     def __init__(self, scene: SceneArrays):
         self.lib = oracle_lib()
@@ -100,6 +100,7 @@ class Oracle:
         s.triangles, s.n_triangles = scene.triangles.ctypes.data, len(scene.triangles)
         s.mtriangles, s.n_mtriangles = scene.mtriangles.ctypes.data, len(scene.mtriangles)
         self._s = s
+        self._bg = None if scene.background is None else C.c_void_p(scene.background.ctypes.data)  # kept alive by self.scene
         self._bvh = None
 
     def __del__(self):
@@ -179,9 +180,9 @@ class Oracle:
         out = np.zeros((H, W, 3), np.float32)
         fixed = np.zeros((H, W, 3), np.uint64)
         cnt = Counters()
-        self.lib.orc_render(C.byref(self._s), self.bvh() if use_bvh else None, W, H, spp, max_depth, C.c_uint64(seed),
-                            rank, world, shard_mode, C.c_void_p(out.ctypes.data), C.c_void_p(fixed.ctypes.data),
-                            C.byref(cnt))
+        self.lib.orc_render_bg(C.byref(self._s), self._bg, self.bvh() if use_bvh else None, W, H, spp, max_depth,
+                               C.c_uint64(seed), rank, world, shard_mode, C.c_void_p(out.ctypes.data),
+                               C.c_void_p(fixed.ctypes.data), C.byref(cnt))
         return out, fixed, cnt.as_dict()
 
     # -- the double integrator (oracle/rrt_oracle_f64.c) --
@@ -216,8 +217,8 @@ class Oracle:
         out = np.zeros((H, W, 3), np.float64)
         fixed = np.zeros((H, W, 3), np.uint64)
         cnt = Counters()
-        self.lib.orc_d_render(C.byref(self._s), self.bvh() if use_bvh else None, W, H, spp, max_depth, C.c_uint64(seed),
-                              C.c_void_p(out.ctypes.data), C.c_void_p(fixed.ctypes.data), C.byref(cnt))
+        self.lib.orc_d_render_bg(C.byref(self._s), self._bg, self.bvh() if use_bvh else None, W, H, spp, max_depth,
+                                 C.c_uint64(seed), C.c_void_p(out.ctypes.data), C.c_void_p(fixed.ctypes.data), C.byref(cnt))
         return out, fixed, cnt.as_dict()
 
     def tonemap(self, rgb_sum, spp):

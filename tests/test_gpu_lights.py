@@ -21,7 +21,6 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, load_golden
-from lights_oracle import LitOracle
 from oracle_lib import Oracle
 from rrt_b200.types import DIFFUSE_LIGHT, SceneArrays, material_dtype, sphere_dtype
 from test_gpu_launch_space import POOL, S1, S2, SAMPLES, SIMPLE, TILES, _renders, _where, shard_paths
@@ -41,7 +40,7 @@ def test_anchor_sums_on_the_gpu(ctx, name, depth, precision):
     build, miss, hit = ANCHORS[name]
     W, H, spp = 33, 17, 40
     scene = build(W, H)
-    _, want, cnt = LitOracle(scene).render_f64(W, H, spp, depth, S2)
+    _, want, cnt = Oracle(scene).render_f64(W, H, spp, depth, S2)
     if depth == 1:
         hit = (0.0, 0.0, 0.0)  # the bounce off the small sphere would exceed the depth
     check_two_level(want, spp, miss, hit, (H // 2, W // 2), (0, 0))
@@ -78,7 +77,7 @@ def test_scatter_hook_on_an_emitter(ctx):
     in16[:, 13] = 1
     in16[:, 14] = (1, 0)
     rnd = (np.arange(8, dtype=np.uint64).reshape(2, 4) * 0x9E3779B9 % 2**32).astype(np.uint32)
-    orc = LitOracle(scene)
+    orc = Oracle(scene)
     got32, got64 = ctx.scatter(in16.astype(np.float32), rnd), ctx.scatter_f64(in16, rnd)
     assert got32[0].tolist() == got64[0].tolist() == [0, 0, 0, 0.75, 0.75, 0.75, 0, 0]
     assert got64.tobytes() == orc.scatter_f64(in16, rnd).tobytes()
@@ -102,7 +101,7 @@ def test_buried_light_is_not_reached_on_the_oracle():
     W, H, spp = 40, 27, 4
     for render in ("render", "render_f64"):
         a = getattr(Oracle(plain), render)(W, H, spp, 50, S1)
-        b = getattr(LitOracle(lit), render)(W, H, spp, 50, S1)
+        b = getattr(Oracle(lit), render)(W, H, spp, 50, S1)
         assert a[1].tobytes() == b[1].tobytes() and (a[2]["rays"], a[2]["hits"]) == (b[2]["rays"], b[2]["hits"])
 
 
@@ -153,7 +152,7 @@ LIT_CASES = [("cornell", 61, 45, 24, 50), ("cornell", 33, 17, 7, 3), ("fast", 61
 def test_f64_lit_render_equals_oracle(ctx, lit_scenes, case):
     name, W, H, spp, depth = case
     scene = lit_scenes[name]
-    want, _, cnt = LitOracle(scene).render_f64(W, H, spp, depth, S2)
+    want, _, cnt = Oracle(scene).render_f64(W, H, spp, depth, S2)
     for label, img, st, count in _renders(ctx, scene, W, H, spp, depth, S2, "f64", np.float64):
         assert img.tobytes() == want.tobytes(), (case, label, _where(img, want))
         if count:
@@ -169,7 +168,7 @@ def test_f32_lit_render_same_bits_on_every_scheduler(ctx, lit_scenes, case):
     for label, img, st, count in runs:
         assert img.tobytes() == first.tobytes(), (case, label, _where(img, first))
     assert len({(st["rays"], st["hits"]) for _, _, st, count in runs if count}) == 1
-    ref, _, _ = LitOracle(scene).render(W, H, spp, depth, S2)
+    ref, _, _ = Oracle(scene).render(W, H, spp, depth, S2)
     a = np.sqrt(first.astype(np.float64) / spp).clip(0, 1)
     b = np.sqrt(ref.astype(np.float64) / spp).clip(0, 1)
     close = np.abs(a - b).max(axis=2) < 1e-3
@@ -258,8 +257,8 @@ def test_staging_then_clearing_a_background_is_no_background(ctx):
     # staged: the background replaces the sky (the oracle agrees bit for bit) ...
     assert st(ctx.h, C.c_void_p(bg.ctypes.data)) == 0 and _scene_set(ctx, plain) == 0
     with_bg, _ = ctx.render(W, H, spp, 50, seed=S1, dtype=np.float64, precision="f64")
-    want, _, _ = LitOracle(SceneArrays(plain.camera, plain.materials, plain.spheres, plain.mspheres, plain.triangles,
-                                    background=bg)).render_f64(W, H, spp, 50, S1)
+    want, _, _ = Oracle(SceneArrays(plain.camera, plain.materials, plain.spheres, plain.mspheres, plain.triangles,
+                                 background=bg)).render_f64(W, H, spp, 50, S1)
     assert with_bg.tobytes() == want.tobytes() and with_bg.tobytes() != sky.tobytes()
     # ... and is consumed: the next rrtb_scene_set without a staging call has the sky again
     assert _scene_set(ctx, plain) == 0

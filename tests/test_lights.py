@@ -1,6 +1,7 @@
 """-m "not gpu": diffuse_light emitters and a constant background (include/rrtb.h RRTB_DIFFUSE_LIGHT,
-rrtb_scene_stage_background): the scene grammar, the Python scene arrays and the analytic anchors on both CPU oracles (with the lights terms of
-tests/oracle_lights, see tests/lights_oracle.py).
+rrtb_scene_stage_background): the scene grammar, the Python scene arrays, the analytic anchors on both integrators of
+the CPU oracle (which carries the emitted and background terms itself, oracle/rrt_oracle.h), and the oracle's outputs
+pinned by digest on scenes with and without lights.
 
 The anchors are scenes in which every camera path ends after at most two segments with a radiance that is one product
 of exactly representable values, so each pixel sum is known exactly:
@@ -12,13 +13,14 @@ of exactly representable values, so each pixel sum is known exactly:
 
 tests/test_gpu_lights.py renders the same scenes on the GPU and expects the same sums.
 """
+import hashlib
+import json
 import os
 
 import numpy as np
 import pytest
 
 from conftest import ROOT, load_golden
-from lights_oracle import LitOracle
 from oracle_lib import Oracle, camera_derive, ref_scene_path
 from rrt_b200.types import DIFFUSE_LIGHT, SceneArrays, material_dtype, sphere_dtype
 
@@ -194,7 +196,7 @@ def test_scene_arrays_carry_the_background():
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# C2: analytic anchors on both oracles
+# C2: analytic anchors on both integrators of the oracle
 # ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name", sorted(ANCHORS))
 @pytest.mark.parametrize("depth", [2, 50])
@@ -202,7 +204,7 @@ def test_anchor_sums_on_the_oracles(name, depth):
     build, miss, hit = ANCHORS[name]
     W, H, spp = 9, 7, 24
     scene = build(W, H)
-    orc = LitOracle(scene)
+    orc = Oracle(scene)
     ks = []
     for bvh in (True, False):
         _, f32, c32 = orc.render(W, H, spp, depth, 1984, use_bvh=bvh)
@@ -225,20 +227,20 @@ def test_anchor_at_depth_one(name):
     background still count."""
     build, miss, _ = ANCHORS[name]
     W, H, spp = 9, 7, 8
-    _, f, _ = LitOracle(build(W, H)).render_f64(W, H, spp, 1, 1984)
+    _, f, _ = Oracle(build(W, H)).render_f64(W, H, spp, 1, 1984)
     check_two_level(f, spp, miss, (0.0, 0.0, 0.0), (H // 2, W // 2), (0, 0))
 
 
 def test_anchor_clamp_on_the_oracle():
     """Le = 3 at spp = 2^21 + 1, where the per-sample clamp is 2: every pixel sums to exactly spp * fixed(2)."""
     W, H, spp = 2, 2, 2**21 + 1
-    _, f, _ = LitOracle(emitter_only_scene(W, H, 3.0)).render_f64(W, H, spp, 2, 1984, use_bvh=False)
+    _, f, _ = Oracle(emitter_only_scene(W, H, 3.0)).render_f64(W, H, spp, 2, 1984, use_bvh=False)
     assert np.all(f == spp * fixed(2.0))
 
 
 def test_scatter_reports_no_scatter_for_an_emitter():
     scene = furnace_scene(8, 4, 0.5)
-    orc = LitOracle(scene)
+    orc = Oracle(scene)
     in16 = np.zeros((2, 16))
     in16[:, 3:6] = (0, 0, -1)
     in16[:, 10:13] = (0, 0, 1)
@@ -250,22 +252,125 @@ def test_scatter_reports_no_scatter_for_an_emitter():
         assert out[1, 6] == 1 and out[1, 3] == 0.5
 
 
-@pytest.mark.parametrize("name", ["test2", "final"])
-def test_lights_oracle_without_lights_is_the_oracle(name):
-    """The oracle with lights, on a scene with neither emitter nor background, is the plain oracle bit for bit."""
-    scene, _ = load_golden(name)
-    W, H, spp = 24, 16, 3
-    a, b = Oracle(scene), LitOracle(scene)
-    for bvh in (True, False):
-        for r in ("render", "render_f64"):
-            x, y = getattr(a, r)(W, H, spp, 50, 7, use_bvh=bvh), getattr(b, r)(W, H, spp, 50, 7, use_bvh=bvh)
-            assert x[1].tobytes() == y[1].tobytes() and x[2] == y[2], (name, r, bvh)
-    x, y = a.render(W, H, spp, 50, 7, rank=1, world=3, shard_mode=0), b.render(W, H, spp, 50, 7, rank=1, world=3, shard_mode=0)
-    assert x[1].tobytes() == y[1].tobytes()
+# ---------------------------------------------------------------------------------------------------------------
+# C3: the oracle pinned on the CPU
+# ---------------------------------------------------------------------------------------------------------------
+PIN_W, PIN_H, PIN_SPP, PIN_DEPTH, PIN_SEED = 24, 16, 3, 50, 7
+
+# scene -> output -> SHA-256, made as test_oracle_outputs_are_pinned says; data, never to be regenerated by a refactor
+ORACLE_PINS = {
+    "test2": {
+        "render/bvh": "bfc47d425042f12b7d4ebb69d9fd6c1ded3f4c897e1e3020e390b9f4366d94db",
+        "render/scan": "93f80c91ee11d2ae31a5b99a0a1f34203078663771a71d8512fe55d5c35cadaa",
+        "render_f64/bvh": "f593ae3f4db6cd1d5ee1ca732b6594bf49f8873fbcf45264378278fc32ce20a2",
+        "render_f64/scan": "f593ae3f4db6cd1d5ee1ca732b6594bf49f8873fbcf45264378278fc32ce20a2",
+        "render/bvh/tile-1-of-3": "8b02411963e23111b2199a6b64fd25ede52860011e04442e2448e6be07d1729d",
+        "scatter": "aa22ae5d77459119d58754d864c6e08cc4617c79e9fc0a6db66a3303414a09d0",
+        "scatter_f64": "28b219b76ca42fcfcbbd3692cc4f7ca1aea7c94199544d2dc275df9fdb25f6e4",
+    },
+    "test3": {
+        "render/bvh": "1fd29dc0f7355fed87a691584e3c65d4550c20772876479a56e5d6412cf612b2",
+        "render/scan": "ca0eef29999db1029a5471e0230c2242f8451d9cd1d075c0a3e6961c73b9050b",
+        "render_f64/bvh": "5f85663e74e1d4d6452135663796ccac253e47b914e94a986689ebdcb3c3394d",
+        "render_f64/scan": "5f85663e74e1d4d6452135663796ccac253e47b914e94a986689ebdcb3c3394d",
+        "render/bvh/tile-1-of-3": "8d8efa896c948b6922192bc11aa7c79dfe4b42b00010057d43ee5f99c860115a",
+        "scatter": "a51d7c13f3651d972ace5d1e3b431900d82c5a601fadca46a811a22a72cefe80",
+        "scatter_f64": "3832a0526a294e25f16cc414aea71b5d2c02170bd63dcbc44cb0ff19e49d315b",
+    },
+    "final": {
+        "render/bvh": "7cd9a96279f70a997114a625c32667e891e18000ea96b855c69db55b2c369532",
+        "render/scan": "d5fd04771898a1fb4fd1fc111340c9f4c725900e0d25a517a9f13d91eb265f6e",
+        "render_f64/bvh": "ee524c3d6eb62095d38fdf56f2f1fb6d7c51ca4f904885f6b64da98de3dcfbff",
+        "render_f64/scan": "ee524c3d6eb62095d38fdf56f2f1fb6d7c51ca4f904885f6b64da98de3dcfbff",
+        "render/bvh/tile-1-of-3": "17933ca73ac0ab18cf715fe15aecd2b940e04128269b6a9236ca30664502d853",
+        "scatter": "375ae995875b777629ca807d2c25684ac3cb77eea62bf158bc06fa743527a7b7",
+        "scatter_f64": "7be9360b108167358168584f779fb8b05cf267e49ad1663d665f28fabc51c30e",
+    },
+    "background-a0.5": {
+        "render/bvh": "fbc1f6124b49706bf5a254d361cffbdb629afe9fdcfbf84c78aa618aac553670",
+        "render/scan": "b1f11552ef88672d2d351752efd957e8dbb3675fb03be26caf1ebe2cf2840d5b",
+        "render_f64/bvh": "fbc1f6124b49706bf5a254d361cffbdb629afe9fdcfbf84c78aa618aac553670",
+        "render_f64/scan": "fbc1f6124b49706bf5a254d361cffbdb629afe9fdcfbf84c78aa618aac553670",
+        "render/bvh/tile-1-of-3": "707b626a2a2fd133ad3a339002f627babd5ac0521f4637488c4c6017ece2df50",
+        "scatter": "75ed123957470cbe767b5cc047e5a3c59ac1cb67eb15302f82aca3c1ec2d64c5",
+        "scatter_f64": "2b94de0780a434e0309549f155260a9d539c38435aff717601158e6cf26e11e6",
+    },
+    "furnace-a0.5": {
+        "render/bvh": "78d196de3a7af7c6956535061b33401b3993bb12a0f8bd50cfc5889562de6902",
+        "render/scan": "6fd1e86cf82ae31988877020e72a949b9aae662e7e32c6b300bfbb929ed49474",
+        "render_f64/bvh": "c6e38d70929efc5a52f943938563c194abbc0cac05263d31688003ed196937a1",
+        "render_f64/scan": "c6e38d70929efc5a52f943938563c194abbc0cac05263d31688003ed196937a1",
+        "render/bvh/tile-1-of-3": "d228c379331595516f0e6b9a952b40eeda3ab4d0337106a4049a3fcc949b33c5",
+        "scatter": "f52c92afaa7007e77012bed647769c5189f618e231df5eb4c05a3f72baf5eda9",
+        "scatter_f64": "96acc1b7214d14167e6550d1cfce7372d2660271b16cbe5e31b8bcecce3293d7",
+    },
+    "furnace-a1": {
+        "render/bvh": "2c9ea54073d34a00586dd755089980a1727eaafcab66883523661743d923a354",
+        "render/scan": "f9c474aea6c0cb420cd9fdb4d6bd60359da9f7a4f51f07124081c58b957f4343",
+        "render_f64/bvh": "5b1dca39025261a1d644413f63c9d0deb9f365c8bd4b46c10cad453ace53dc33",
+        "render_f64/scan": "5b1dca39025261a1d644413f63c9d0deb9f365c8bd4b46c10cad453ace53dc33",
+        "render/bvh/tile-1-of-3": "b6ad88903160dcfe0ce883b97788f8b9cc2337fd9c26a35da0fed9b89606631f",
+        "scatter": "a90e2fdf22404d607c323ec66eaee0e157a0f627dbaf3e8d5eb39dbeefbb6ba9",
+        "scatter_f64": "f7b5ccbcd0a231e0ec993593b7ef029c4c07e725e7eef49aaa35369ffaf18a38",
+    },
+    "cornell": {
+        "render/bvh": "c580a9ae82c8eb3a213f555f76da3c79ae0801eabb774c0f374f145ad2842d48",
+        "render/scan": "90ad2ca0b7528ef68ece1cdac58a656d86fae5848459083a45d36d95bd1bc1b4",
+        "render_f64/bvh": "5f45fff9b36eb1fe22cf3b0285f972e32376a3e69501819964fa2c8157f19795",
+        "render_f64/scan": "5f45fff9b36eb1fe22cf3b0285f972e32376a3e69501819964fa2c8157f19795",
+        "render/bvh/tile-1-of-3": "23e2c03aa83d36d2bcb2be3d59bf5a07880fdd39d4bc5dd9dc2eac5c76e50be8",
+        "scatter": "fa3fa8029797c2b2be6eb5bf2188bf0b30b7ccb90e809e9f3e92e4e65bbbab55",
+        "scatter_f64": "b8cdd165ef4a54922a7ad3b504a2bc2b1c7be3bdd504141897b18d78fca27f4f",
+    },
+}
+
+
+def pin_scene(name):
+    """A scene of ORACLE_PINS at PIN_W x PIN_H: a golden fixture, an anchor or scenes/cornell.txt (needs the library)"""
+    if name == "cornell":
+        from rrt_b200 import Scene
+
+        return Scene.from_file(CORNELL, PIN_W, PIN_H).arrays
+    if name in ANCHORS:
+        return ANCHORS[name][0](PIN_W, PIN_H)
+    return load_golden(name)[0]
+
+
+def oracle_digests(orc):
+    """SHA-256 of each pinned output of an oracle bound to a scene: a render's fixed-point framebuffer followed by its
+    counters (JSON, sorted keys); a scatter hook's output array on 64 seeded random inputs over all of the scene's
+    materials"""
+    sha = lambda *parts: hashlib.sha256(b"".join(parts)).hexdigest()
+    W, H, spp, depth, seed = PIN_W, PIN_H, PIN_SPP, PIN_DEPTH, PIN_SEED
+    out = {}
+    for r in ("render", "render_f64"):
+        for bvh in (True, False):
+            _, f, cnt = getattr(orc, r)(W, H, spp, depth, seed, use_bvh=bvh)
+            out["%s/%s" % (r, "bvh" if bvh else "scan")] = sha(f.tobytes(), json.dumps(cnt, sort_keys=True).encode())
+    _, f, cnt = orc.render(W, H, spp, depth, seed, rank=1, world=3, shard_mode=0)  # RRTB_SHARD_TILES
+    out["render/bvh/tile-1-of-3"] = sha(f.tobytes(), json.dumps(cnt, sort_keys=True).encode())
     rng = np.random.default_rng(3)
     in16 = rng.normal(size=(64, 16))
     in16[:, 13] = rng.integers(0, 2, 64)
-    in16[:, 14] = rng.integers(0, len(scene.materials), 64)
+    in16[:, 14] = rng.integers(0, len(orc.scene.materials), 64)
     rnd = rng.integers(0, 2**32, size=(64, 4), dtype=np.uint32)
-    assert a.scatter(in16, rnd).tobytes() == b.scatter(in16, rnd).tobytes()
-    assert a.scatter_f64(in16, rnd).tobytes() == b.scatter_f64(in16, rnd).tobytes()
+    out["scatter"] = sha(orc.scatter(in16, rnd).tobytes())
+    out["scatter_f64"] = sha(orc.scatter_f64(in16, rnd).tobytes())
+    return out
+
+
+@pytest.mark.parametrize("name", list(ORACLE_PINS))
+def test_oracle_outputs_are_pinned(name, request):
+    """The oracle's framebuffers, counters and scatter outputs equal the digests of ORACLE_PINS: both integrators through
+    the LBVH and the flat scan, a tile shard and both scatter hooks, on test2, test3 and final (no lights), on the three
+    anchors and on cornell.txt (emitters, a background).
+
+    The digests were computed once with oracle_digests at commit d7e664a, the last one with a separate oracle for
+    lights: its plain oracle for test2, test3 and final, its oracle with lights for the others.  The oracle is what the
+    GPU is held to bit for bit and the only check of the lights on a machine without a GPU, so a refactor of it must
+    leave every digest as it is.  Only a change of what a path computes may change this table, in the same change as
+    the GPU integrators."""
+    if name == "cornell":
+        request.getfixturevalue("built_lib")
+    got = oracle_digests(Oracle(pin_scene(name)))
+    assert got == ORACLE_PINS[name], [k for k in got if got[k] != ORACLE_PINS[name][k]]
