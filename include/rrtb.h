@@ -283,9 +283,15 @@ int rrtb_bvh_download(rrtb_ctx *ctx, uint32_t *morton, uint32_t *perm, int32_t *
  * widened to float), 4 child refs as int bits, 4 unused.  Child ref >= 0: node index; < 0: ~((sorted position << 2) |
  * primitive type); an unused child slot has h = -inf.  Node 0 is the root; a parent always precedes its children.
  * Test hook: the tree is derived data (closest hit does not depend on it); it is checked for being a partition of
- * the primitives whose boxes enclose them (tests/test_gpu_edge_cases.py). */
+ * the primitives whose boxes enclose them (tests/test_gpu_edge_cases.py) and, raw, word for word against the CPU
+ * reference of the build (tests/test_wide_tree.py). */
 int rrtb_wide_size(rrtb_ctx *ctx, int32_t *n_nodes, int32_t *width);
 int rrtb_wide_download(rrtb_ctx *ctx, float *nodes, int32_t max_nodes);
+/* The same nodes as the device holds them, word for word: 24 uint32 per node (rrtb_device.cuh "Traversal node": float
+ * centres, fp16 half-extent pairs rounded up, refs, 2 zero words) or, in scenes traversed through motion nodes, 40 per
+ * node ("Motion node": centres and half extents at both ends of the shutter).  *words_per_node (may be NULL) gets 24 or
+ * 40; `words` holds max_nodes nodes of that size.  Node indices are the build's own (atomic) numbering. */
+int rrtb_wide_download_raw(rrtb_ctx *ctx, uint32_t *words, int32_t max_nodes, int32_t *words_per_node);
 /* Philox4x32-10 known-answer hook: out[4*i..] = philox(ctr[4*i..], key) computed on the device. */
 int rrtb_philox(rrtb_ctx *ctx, const uint32_t *ctr4, int n, uint32_t key0, uint32_t key1, uint32_t *out4);
 /* material::scatter (material.h:21-32,50-57,76-96) on the device for explicit inputs.

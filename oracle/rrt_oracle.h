@@ -79,6 +79,49 @@ void orc_bvh_free(orc_bvh *b);
 void orc_trace_bvh(const orc_scene *s, const orc_bvh *b, const float *rays7, int n, float t_min, int32_t *id,
                    float *t, float *rec7, orc_counters *cnt);
 
+/* the traversal tree of the product (rrt_oracle_wide.c): the SAH rebuild of the LBVH's lower subtrees, the refit of
+ * the Morton top, the 4-wide collapse and its node encoding, restated in float in the GPU's operation order */
+typedef struct orc_wide_counters {
+    int32_t sort_small;        /* 1: one-block bitonic sort (n <= 2048), 0: radix sort */
+    int32_t rebuild_shape;     /* k_sah_rebuild<1024> (n <= 4096) or <256>; 0: no rebuild (n < 3) */
+    int32_t n_roots;           /* rebuilt subtrees */
+    int32_t block_splits;      /* binned splits of runs of more than 128 by the whole block (shape 1024 only) */
+    int32_t block_median_coincident, block_median_budget; /* ... of them median splits: no plane / depth budget */
+    int32_t warp_splits;       /* binned splits by one warp (runs of 5 or more) */
+    int32_t warp_median_coincident, warp_median_budget;
+    int32_t small_splits;      /* exact splits of runs of 2..4 boxes */
+    int32_t small_halved;      /* ... of them halved: no finite cost or depth budget */
+    int32_t refit_parent;      /* leaves directly under a node of more than 512 leaves (k_refit_upper parent rule) */
+    int32_t refit_grandparent; /* leaves of a 2-leaf node under a node of more than 512 leaves (grandparent rule) */
+    int32_t max_binary_depth;  /* deepest leaf of the binary traversal tree, root = 0 */
+    int32_t max_wide_depth;    /* deepest 4-wide node, root = 0 */
+    float pad;                 /* the traversal-box padding the nodes were encoded with: 2^-20 max(largest |coordinate| of
+                                * a primitive box, max_k |origin_k| + lens radius), computed here (tests compare it with
+                                * orc_bvh.pad) */
+} orc_wide_counters;
+
+typedef struct orc_wide {
+    int32_t n_nodes, words_per_node; /* 24 words per node, 40 per motion node (rrtb_device.cuh) */
+    uint32_t *words;                 /* [n_nodes * words_per_node], canonical order: pre-order, children in slot order */
+    int32_t n_tasks, n_items;
+    int32_t *tasks; /* [n_tasks * 7] per split: path (0 block, 1 warp, 2 exact), first item, count, choice (axis * 32 + bin,
+                     * the left mask of an exact split, -1 for a binned median split), how (0 SAH, 1 no plane / no
+                     * finite cost, 2 depth budget), level below the subtree root, budget (63 - canonical depth of the
+                     * subtree root) */
+    int32_t *items;     /* the sorted positions of each split's run, in run order */
+    float *prim_box01;  /* [12 n] object-id order: lo, hi at camera time0, lo, hi at camera time1 (k_prepare) */
+    int32_t *left2, *right2; /* [max(n - 1, 1)] the binary traversal tree the collapse reads (rebuilt subtrees and the
+                              * Morton top; the canonical LBVH for n < 3): >= 0 node, < 0 leaf ~sorted position */
+    float *node_box2;        /* [6 max(n - 1, 1)] its node boxes, min xyz, max xyz */
+    orc_wide_counters cnt;
+} orc_wide;
+
+/* motion: 40-word motion nodes with both ends of the shutter (the caller applies the library's rule) */
+orc_wide *orc_wide_build(const orc_scene *s, int motion);
+void orc_wide_free(orc_wide *w);
+/* float -> IEEE half rounded toward +inf, bits (the half extents of the traversal nodes) */
+uint16_t orc_f16_up(float h);
+
 /* material.h scatter with an explicit Philox block. in16/out8 as rrtb_scatter.  An emitter reports direction 0,
  * attenuation Le, not scattered. */
 void orc_scatter(const orc_scene *s, const float *in16, const uint32_t *rnd4, int n, float *out8);

@@ -17,7 +17,7 @@ SYMBOLS = [
     "rrtb_scene_set", "rrtb_scene_stage_moving_triangles", "rrtb_scene_stage_background", "rrtb_camera_set", "rrtb_render", "rrtb_render_f64", "rrtb_render_device", "rrtb_resolve_device",
     "rrtb_accumulate_device", "rrtb_frame_create", "rrtb_frame_export", "rrtb_frame_import", "rrtb_frame_attach", "rrtb_frame_detach",
     "rrtb_render_shard", "rrtb_frame_download", "rrtb_render_group", "rrtb_host_alloc", "rrtb_host_free", "rrtb_trace_closest", "rrtb_trace_closest_f64", "rrtb_camera_rays", "rrtb_camera_rays_f64",
-    "rrtb_bvh_size", "rrtb_bvh_download", "rrtb_wide_size", "rrtb_wide_download", "rrtb_philox", "rrtb_scatter", "rrtb_scatter_f64", "rrtb_probe_issue_rate", "rrtb_scene_parse_file", "rrtb_scene_free", "rrtb_scene_counts",
+    "rrtb_bvh_size", "rrtb_bvh_download", "rrtb_wide_size", "rrtb_wide_download", "rrtb_wide_download_raw", "rrtb_philox", "rrtb_scatter", "rrtb_scatter_f64", "rrtb_probe_issue_rate", "rrtb_scene_parse_file", "rrtb_scene_free", "rrtb_scene_counts",
     "rrtb_scene_camera", "rrtb_scene_materials", "rrtb_scene_spheres", "rrtb_scene_mspheres",
     "rrtb_scene_triangles", "rrtb_scene_mtriangle_count", "rrtb_scene_mtriangles", "rrtb_scene_background", "rrtb_scene_upload", "rrtb_camera_derive", "rrtb_tonemap_rgb8", "rrtb_tonemap_rgb8_f64", "rrtb_write_png",
 ]
@@ -81,6 +81,7 @@ def load():
         "rrtb_bvh_download": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp]),
         "rrtb_wide_size": (C.c_int, [vp, P(i32), P(i32)]),
         "rrtb_wide_download": (C.c_int, [vp, vp, i32]),
+        "rrtb_wide_download_raw": (C.c_int, [vp, vp, i32, P(i32)]),
         "rrtb_philox": (C.c_int, [vp, vp, C.c_int, u32, u32, vp]),
         "rrtb_scatter": (C.c_int, [vp, vp, vp, C.c_int, vp]),
         "rrtb_probe_issue_rate": (C.c_int, [vp, P(C.c_double), P(C.c_double)]),

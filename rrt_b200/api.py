@@ -352,6 +352,16 @@ class Context:
         return dict(c=raw[:, 0:3 * w].reshape(-1, 3, w).copy(), h=raw[:, 3 * w:6 * w].reshape(-1, 3, w).copy(),
                     ref=raw[:, 6 * w:7 * w].copy().view(np.int32))
 
+    def wide_raw(self):
+        """The traversal nodes as the device holds them: [m, 24] uint32, or [m, 40] for motion nodes (include/rrtb.h
+        rrtb_wide_download_raw), in the build's own node numbering."""
+        n = C.c_int32()
+        self._check(self.lib.rrtb_wide_size(self.h, C.byref(n), None))
+        raw = np.zeros((n.value, 40), np.uint32)
+        wpn = C.c_int32()
+        self._check(self.lib.rrtb_wide_download_raw(self.h, _vp(raw), n.value, C.byref(wpn)))
+        return raw.reshape(-1)[:n.value * wpn.value].reshape(n.value, wpn.value).copy()
+
     def philox(self, ctr4, key0, key1):
         ctr4 = np.ascontiguousarray(ctr4, dtype=np.uint32).reshape(-1, 4)
         out = np.zeros_like(ctr4)

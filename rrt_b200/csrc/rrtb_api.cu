@@ -999,6 +999,19 @@ int rrtb_wide_download(rrtb_ctx *ctx, float *nodes, int32_t max_nodes)
     return RRTB_OK;
 }
 
+int rrtb_wide_download_raw(rrtb_ctx *ctx, uint32_t *words, int32_t max_nodes, int32_t *words_per_node)
+{
+    if (!ctx || !words || max_nodes < 0) return RRTB_ERR_INVALID;
+    int32_t n_nodes = 0;
+    int rc = rrtb_wide_size(ctx, &n_nodes, nullptr);
+    if (rc) return rc;
+    if (n_nodes > max_nodes) return invalid(ctx, "wide-node buffer too small");
+    const int wpn = ctx->motion ? 4 * RRTB_MOTION_NODE_F4 : 4 * RRTB_NODE_F4;
+    if (words_per_node) *words_per_node = wpn;
+    RRTB_CUDA(ctx, cudaMemcpy(words, ctx->d_wnodes, sizeof(uint32_t) * (size_t)wpn * n_nodes, cudaMemcpyDeviceToHost));
+    return RRTB_OK;
+}
+
 int rrtb_philox(rrtb_ctx *ctx, const uint32_t *ctr4, int n, uint32_t key0, uint32_t key1, uint32_t *out4)
 {
     if (!ctx || !ctr4 || !out4 || n < 0) return RRTB_ERR_INVALID;

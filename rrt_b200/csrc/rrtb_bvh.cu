@@ -527,6 +527,24 @@ __global__ void __launch_bounds__(TPB) k_sah_select(int n, const int *__restrict
     if (size >= 3 && size <= SAH_MAX && psize > SAH_MAX) roots[atomicAdd(&st->n_roots, 1)] = i;
 }
 
+// The arithmetic of the SAH rebuild and of the collapse, written so that each product, sum and quotient rounds once:
+// ptxas would otherwise contract products and sums into FMAs where it chooses, and the tree would then depend on the
+// compiler.  oracle/rrt_oracle_wide.c restates these definitions as plain C built with -ffp-contract=off.
+//   area_rn      x*y + y*z + z*x, half the surface area of a box of extents x, y, z
+//   sah_cost_rn  a0*n0 + a1*n1, the SAH cost of a split into boxes of areas a0, a1 holding n0, n1 primitives
+//   sah_bin      the bin of twice a centroid, c2 = lo + hi, among SAH_BINS over [cmin, cmin + SAH_BINS / scale]
+__device__ __forceinline__ float area_rn(float x, float y, float z)
+{
+    return __fadd_rn(__fadd_rn(__fmul_rn(x, y), __fmul_rn(y, z)), __fmul_rn(z, x));
+}
+__device__ __forceinline__ float sah_cost_rn(float a0, int n0, float a1, int n1)
+{
+    return __fadd_rn(__fmul_rn(a0, (float)n0), __fmul_rn(a1, (float)n1));
+}
+__device__ __forceinline__ float centroid2(const float *box, int k) { return __fadd_rn(box[k], box[3 + k]); }
+__device__ __forceinline__ float sah_scale(float cmin, float cmax) { return cmax > cmin ? __fdiv_rn((float)SAH_BINS, __fsub_rn(cmax, cmin)) : 0.f; }
+__device__ __forceinline__ int sah_bin(float c2, float cmin, float scale) { return min(SAH_BINS - 1, (int)__fmul_rn(__fsub_rn(c2, cmin), scale)); }
+
 // order-preserving float <-> int (for atomicMin / atomicMax on shared memory)
 __device__ __forceinline__ int f2o(float f)
 {
@@ -584,9 +602,9 @@ __device__ __forceinline__ void sah_choose(const int (*bn3)[SAH_BINS][7], int la
             rhi[c] = __shfl_down_sync(0xffffffffu, shi[c], 1);
         }
         if (lane < 31 && pc > 0 && rc > 0) {
-            const float x0 = phi[0] - plo[0], y0 = phi[1] - plo[1], z0 = phi[2] - plo[2];
-            const float x1 = rhi[0] - rlo[0], y1 = rhi[1] - rlo[1], z1 = rhi[2] - rlo[2];
-            const float ck = (x0 * y0 + y0 * z0 + z0 * x0) * (float)pc + (x1 * y1 + y1 * z1 + z1 * x1) * (float)rc;
+            const float a0 = area_rn(__fsub_rn(phi[0], plo[0]), __fsub_rn(phi[1], plo[1]), __fsub_rn(phi[2], plo[2]));
+            const float a1 = area_rn(__fsub_rn(rhi[0], rlo[0]), __fsub_rn(rhi[1], rlo[1]), __fsub_rn(rhi[2], rlo[2]));
+            const float ck = sah_cost_rn(a0, pc, a1, rc);
             if (ck < cost) {
                 cost = ck;
                 best = k * 32 + lane;
@@ -619,8 +637,7 @@ __device__ __forceinline__ void sah_bins_clear(int (*bn3)[SAH_BINS][7], int lane
 __device__ __forceinline__ void sah_bins_add(int (*bn3)[SAH_BINS][7], const float *box, const float *cmin, const float *scale)
 {
     for (int k = 0; k < 3; ++k) {
-        const float c = box[k] + box[3 + k];
-        int *bn = bn3[k][min(SAH_BINS - 1, (int)((c - cmin[k]) * scale[k]))];
+        int *bn = bn3[k][sah_bin(centroid2(box, k), cmin[k], scale[k])];
         atomicAdd(&bn[0], 1);
         for (int c3 = 0; c3 < 3; ++c3) {
             atomicMin(&bn[1 + c3], f2o(box[c3]));
@@ -729,7 +746,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                 for (int c = 0; c < 6; ++c) box[c] = sbox[l][c];
                 if (warp * 32 < cnt) { // centroid bounds (twice the centroid: lo + hi)
                     for (int k = 0; k < 3; ++k) {
-                        const float c = box[k] + box[3 + k];
+                        const float c = centroid2(box, k);
                         const float mn = warp_min(valid ? c : inf), mx = warp_max(valid ? c : -inf);
                         if (lane == 0) {
                             atomicMin(&s_cmin[k], f2o(mn));
@@ -742,7 +759,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                 for (int k = 0; k < 3; ++k) {
                     const float cmax = o2f(s_cmax[k]);
                     cmin[k] = o2f(s_cmin[k]);
-                    scale[k] = cmax > cmin[k] ? (float)SAH_BINS / (cmax - cmin[k]) : 0.f;
+                    scale[k] = sah_scale(cmin[k], cmax);
                 }
                 if (valid) sah_bins_add(bins[0], box, cmin, scale);
                 __syncthreads();
@@ -762,7 +779,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                 bool go_left = false;
                 if (valid) {
                     if (s_median) go_left = tid < cnt / 2;
-                    else go_left = min(SAH_BINS - 1, (int)((box[ax] + box[3 + ax] - cmin[ax]) * scale[ax])) <= sp;
+                    else go_left = sah_bin(centroid2(box, ax), cmin[ax], scale[ax]) <= sp;
                 }
                 const unsigned ml = __ballot_sync(0xffffffffu, go_left), mr = __ballot_sync(0xffffffffu, valid && !go_left);
                 if (lane == 0) {
@@ -828,9 +845,9 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                             }
                         }
                         const int na = __popc(mask & ((1u << cnt) - 1u));
-                        const float x0 = ahi[0] - alo[0], y0 = ahi[1] - alo[1], z0 = ahi[2] - alo[2];
-                        const float x1 = bhi[0] - blo[0], y1 = bhi[1] - blo[1], z1 = bhi[2] - blo[2];
-                        cost = (x0 * y0 + y0 * z0 + z0 * x0) * (float)na + (x1 * y1 + y1 * z1 + z1 * x1) * (float)(cnt - na);
+                        const float a0 = area_rn(__fsub_rn(ahi[0], alo[0]), __fsub_rn(ahi[1], alo[1]), __fsub_rn(ahi[2], alo[2]));
+                        const float a1 = area_rn(__fsub_rn(bhi[0], blo[0]), __fsub_rn(bhi[1], blo[1]), __fsub_rn(bhi[2], blo[2]));
+                        cost = sah_cost_rn(a0, na, a1, cnt - na);
                     }
                     int best = lane;
                     for (int o = 4; o > 0; o >>= 1) {
@@ -860,7 +877,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                     for (int i = b + lane; i < e; i += 32) {
                         const int l = sidx[cur][i];
                         for (int k = 0; k < 3; ++k) {
-                            const float c = sbox[l][k] + sbox[l][3 + k];
+                            const float c = centroid2(sbox[l], k);
                             cmin[k] = fminf(cmin[k], c);
                             cmax[k] = fmaxf(cmax[k], c);
                         }
@@ -869,7 +886,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                     for (int k = 0; k < 3; ++k) {
                         cmin[k] = warp_min(cmin[k]);
                         cmax[k] = warp_max(cmax[k]);
-                        scale[k] = cmax[k] > cmin[k] ? (float)SAH_BINS / (cmax[k] - cmin[k]) : 0.f;
+                        scale[k] = sah_scale(cmin[k], cmax[k]);
                     }
                     sah_bins_clear(bins[warp], lane);
                     __syncwarp();
@@ -891,10 +908,7 @@ __global__ void __launch_bounds__(NT) k_sah_rebuild(const uint64_t *__restrict__
                         bool go_left = false;
                         if (valid) {
                             if (median) go_left = (i - b) < cnt / 2;
-                            else {
-                                const float c = sbox[l][ax] + sbox[l][3 + ax];
-                                go_left = min(SAH_BINS - 1, (int)((c - cmin[ax]) * scale[ax])) <= sp;
-                            }
+                            else go_left = sah_bin(centroid2(sbox[l], ax), cmin[ax], scale[ax]) <= sp;
                         }
                         const unsigned ml = __ballot_sync(0xffffffffu, go_left), mr = __ballot_sync(0xffffffffu, valid && !go_left);
                         if (go_left) sidx[cur ^ 1][b + nl + __popc(ml & lt)] = (unsigned short)l;
@@ -1003,8 +1017,8 @@ __global__ void __launch_bounds__(TPB) k_refit_upper(const uint64_t *__restrict_
 // (the roundings of c and of hi-c / c-lo are <= 2^-23 * magnitude, pad is 2^-20 * magnitude)
 __device__ __forceinline__ void center_half(float lo, float hi, float pad, float &c, float &h)
 {
-    c = 0.5f * (lo + hi);
-    h = fmaxf(hi - c, c - lo) + pad;
+    c = __fmul_rn(0.5f, __fadd_rn(lo, hi));
+    h = __fadd_rn(fmaxf(__fsub_rn(hi, c), __fsub_rn(c, lo)), pad);
 }
 
 __device__ __forceinline__ int prim_type(int id, int ns, int nms, int nt)
@@ -1047,8 +1061,7 @@ __device__ __forceinline__ float f16_pair_up(float lo, float hi) { return __uint
 
 __device__ __forceinline__ float box_area6(const float *b)
 {
-    const float x = b[3] - b[0], y = b[4] - b[1], z = b[5] - b[2];
-    return x * y + y * z + z * x;
+    return area_rn(__fsub_rn(b[3], b[0]), __fsub_rn(b[4], b[1]), __fsub_rn(b[5], b[2]));
 }
 
 __device__ __forceinline__ void collapse_one(int i, int b, const uint64_t *__restrict__ keys, int n, int ns, int nms, int nt,

@@ -56,6 +56,29 @@ class _OrcBvh(C.Structure):
     ]
 
 
+_WIDE_COUNTERS = ("sort_small", "rebuild_shape", "n_roots", "block_splits", "block_median_coincident", "block_median_budget",
+                  "warp_splits", "warp_median_coincident", "warp_median_budget", "small_splits", "small_halved",
+                  "refit_parent", "refit_grandparent", "max_binary_depth", "max_wide_depth")
+
+
+class _OrcWideCounters(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in _WIDE_COUNTERS] + [("pad", C.c_float)]
+
+
+class _OrcWide(C.Structure):
+    _fields_ = [
+        ("n_nodes", C.c_int32), ("words_per_node", C.c_int32),
+        ("words", C.POINTER(C.c_uint32)),
+        ("n_tasks", C.c_int32), ("n_items", C.c_int32),
+        ("tasks", C.POINTER(C.c_int32)),
+        ("items", C.POINTER(C.c_int32)),
+        ("prim_box01", C.POINTER(C.c_float)),
+        ("left2", C.POINTER(C.c_int32)), ("right2", C.POINTER(C.c_int32)),
+        ("node_box2", C.POINTER(C.c_float)),
+        ("cnt", _OrcWideCounters),
+    ]
+
+
 class Counters(C.Structure):
     _fields_ = [(k, C.c_uint64) for k in ("rays", "box_tests", "sphere_tests", "msphere_tests", "triangle_tests", "hits", "paths")]
 
@@ -67,7 +90,7 @@ def build_oracle():
     if os.environ.get("RRTB_ORACLE_LIB"):  # e.g. oracle/liboracle_ubsan.so (`make -C oracle ubsan`): the checker under UBSan
         return os.environ["RRTB_ORACLE_LIB"]
     so = os.path.join(ORACLE_DIR, "liboracle.so")
-    src = [os.path.join(ORACLE_DIR, f) for f in ("rrt_oracle.c", "rrt_oracle_f64.c", "rrt_oracle.h")]
+    src = [os.path.join(ORACLE_DIR, f) for f in ("rrt_oracle.c", "rrt_oracle_f64.c", "rrt_oracle_wide.c", "rrt_oracle.h")]
     if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):
         subprocess.check_call(["make", "-C", ORACLE_DIR, "oracle"], stdout=subprocess.DEVNULL)
     return so
@@ -83,6 +106,11 @@ def oracle_lib():
         _oracle.orc_bvh_build.restype = C.POINTER(_OrcBvh)
         _oracle.orc_u01.restype = C.c_float
         _oracle.orc_u01.argtypes = [C.c_uint32]
+        _oracle.orc_wide_build.restype = C.POINTER(_OrcWide)
+        _oracle.orc_wide_build.argtypes = [C.c_void_p, C.c_int]
+        _oracle.orc_wide_free.argtypes = [C.POINTER(_OrcWide)]
+        _oracle.orc_f16_up.restype = C.c_uint16
+        _oracle.orc_f16_up.argtypes = [C.c_float]
     return _oracle
 
 
@@ -128,6 +156,33 @@ class Oracle:
             prim_box=g(b.prim_box, 6 * n, np.float32).reshape(-1, 6),
             pad=float(b.pad),
         )
+
+    def wide_tree(self, motion):
+        """The 4-wide traversal tree of rrt_oracle_wide.c: dict(words=[m, 24 or 40] uint32 in canonical order (pre-order,
+        children in slot order), counters=dict, tasks=[k, 7] int32 (path, first item, count, choice, how, level, budget:
+        see rrt_oracle.h orc_wide), items=int32 sorted positions, prim_box01=[n, 12] float32, and the binary traversal
+        tree the collapse reads: left2 / right2 [n - 1] int32, node_box2 [n - 1, 6] float32).  `motion`: 40-word motion
+        nodes (the library's rule: 8 or more moving primitives and an open shutter)."""
+        p = self.lib.orc_wide_build(C.byref(self._s), 1 if motion else 0)
+        assert p, "orc_wide_build: empty scene"
+        try:
+            w = p.contents
+            g = lambda ptr, cnt, dt: np.ctypeslib.as_array(ptr, shape=(cnt,)).astype(dt, copy=True) if cnt else np.zeros(0, dt)
+            ni = max(self.scene.n_objects - 1, 0)
+            cnt = {k: int(getattr(w.cnt, k)) for k in _WIDE_COUNTERS}
+            cnt["pad"] = float(w.cnt.pad)
+            return dict(
+                words=g(w.words, w.n_nodes * w.words_per_node, np.uint32).reshape(w.n_nodes, w.words_per_node),
+                counters=cnt,
+                tasks=g(w.tasks, 7 * w.n_tasks, np.int32).reshape(-1, 7),
+                items=g(w.items, w.n_items, np.int32),
+                prim_box01=g(w.prim_box01, 12 * self.scene.n_objects, np.float32).reshape(-1, 12),
+                left2=g(w.left2, ni, np.int32),
+                right2=g(w.right2, ni, np.int32),
+                node_box2=g(w.node_box2, 6 * ni, np.float32).reshape(-1, 6),
+            )
+        finally:
+            self.lib.orc_wide_free(p)
 
     # -- rays --
     def camera_rays(self, W, H, pixels, sample, seed):
@@ -227,6 +282,11 @@ class Oracle:
         out = np.zeros((H, W, 3), np.uint8)
         self.lib.orc_tonemap_rgb8(C.c_void_p(rgb_sum.ctypes.data), W, H, spp, C.c_void_p(out.ctypes.data))
         return out
+
+
+def f16_up(h):
+    """orc_f16_up: the bits of float h as IEEE half, rounded toward +inf"""
+    return int(oracle_lib().orc_f16_up(float(h)))
 
 
 def philox(ctr4, key0, key1):
