@@ -3,7 +3,8 @@
 // Replaces render_init + cuda_render (rrt.cu:81-122) and ray_color (rrt.cu:42-79).  k_render below is the
 // one-path-per-lane kernel of the flat scan and RRTB_SCHED_SIMPLE; the LBVH default is the pool scheduler of
 // rrtb_render_pool.cuh.  Both kernels and the hooks are written once over the path policy of rrtb_path.cuh and
-// instantiated for the float and the double integrator.
+// instantiated for the float and the double integrator; both kernels shade a segment with hit_step / miss_fixed and
+// map a work item to its pixel and sample with local_pixel / global_sample below.
 //
 // Scheduling.  The reference runs one thread per PIXEL, so a warp lives until its slowest pixel has
 // finished all spp samples of up to max_depth bounces.  Here the kernel is PERSISTENT: the grid is
@@ -58,6 +59,103 @@ struct RenderArgs {
     float bg[3];
 };
 
+// ---- the rules of a work item and of a path segment, shared by the lane kernel and the pool scheduler ----------------
+// The pool passes its slot fields to the reference parameters, so that each is read from shared memory only where used.
+
+// The pixel (i, j) of pixel-in-tile `pit` of 8x4-pixel tile `tile` (row-major, tiles_x per row).
+__device__ __forceinline__ void tile_pixel(int tile, int tiles_x, unsigned pit, int &i, int &j)
+{
+    int ty = (int)__fdividef((float)tile, (float)tiles_x); // float estimate, off by <= 1 below 2^28 pixels ...
+    int tx = tile - ty * tiles_x;
+    if (tx < 0) { // ... corrected exactly in integers
+        --ty;
+        tx += tiles_x;
+    }
+    else if (tx >= tiles_x) {
+        ++ty;
+        tx -= tiles_x;
+    }
+    i = tx * 8 + (int)(pit & 7u);
+    j = ty * 4 + (int)(pit >> 3);
+}
+
+// The pixel of pixel-in-tile `pit` of this rank's local tile `ltile`; false for a padding pixel of an edge tile.
+__device__ __forceinline__ bool local_pixel(const RenderArgs &a, int ltile, unsigned pit, int &i, int &j)
+{
+    tile_pixel(a.shard_mode == RRTB_SHARD_TILES ? ltile * a.world + a.rank : ltile, a.tiles_x, pit, i, j);
+    return i < a.W && j < a.H;
+}
+
+// The sample of this rank's local sample `ls`, the key of its Philox streams.
+__device__ __forceinline__ int global_sample(const RenderArgs &a, int ls)
+{
+    return a.shard_mode == RRTB_SHARD_SAMPLES ? ls * a.world + a.rank : ls;
+}
+
+// A segment that leaves the scene adds background x throughput (LIGHTS, a scene with a background), else sky x
+// throughput (rrt.cu:68-75); the sky reads only the ray's direction.
+template <class P, bool LIGHTS>
+__device__ __forceinline__ ulonglong3 miss_fixed(const RenderArgs &a, const typename P::RayT &ray, const typename P::real &tr,
+                                                 const typename P::real &tg, const typename P::real &tb)
+{
+    ulonglong3 f;
+    if (LIGHTS && a.background) P::const_fixed(tr, tg, tb, a.bg[0], a.bg[1], a.bg[2], a.clamp, f.x, f.y, f.z);
+    else P::sky_fixed(ray, tr, tg, tb, a.clamp, f.x, f.y, f.z);
+    return f;
+}
+
+// A segment that hit something (rrt.cu:50-63): hit record, Philox block (pixel, sample, 2 + bounce), scatter.  True:
+// the path goes on, with `ray` and the throughput updated.  False: it ends; an emitter (LIGHTS) hands its last term,
+// throughput x Le, to `emit`, called behind the material test alone so that the pool's atomics need no test of their
+// own.  A scattered path ends here when its next segment would exceed max_depth (rrt.cu:78);
+// such a segment would add nothing, so ending the path one segment later gives the same image.
+template <class P, bool MTRI, bool LIGHTS, class Emit>
+__device__ __forceinline__ bool hit_step(const RenderArgs &a, const float4 *__restrict__ leaves, const LeafAux info,
+                                         typename P::RayT &ray, const typename P::HitT &h, const int &pixel, const int &sample,
+                                         int bounce, typename P::real &tr, typename P::real &tg, typename P::real &tb,
+                                         const Emit &emit)
+{
+    const typename P::RecT rec = P::template record<MTRI>(leaves, info, ray, h);
+    const uint4 rnd = philox4x32_10(make_uint4((uint32_t)pixel, (uint32_t)sample, 2u + (uint32_t)bounce, 0u), a.key);
+    const float4 m = __ldg(&a.scene.materials[rec.mat]);
+    const int mtype = __ldg(&a.scene.material_type[rec.mat]);
+    typename P::real dx, dy, dz, ar, ag, ab;
+    const bool go_on = P::template bounce<LIGHTS>(mtype, m, ray, rec, rnd, dx, dy, dz, ar, ag, ab) && bounce + 1 < a.max_depth;
+    if (go_on) {
+        ray.ox = rec.px; ray.oy = rec.py; ray.oz = rec.pz;
+        ray.dx = dx; ray.dy = dy; ray.dz = dz;
+        tr = P::mul(tr, ar); tg = P::mul(tg, ag); tb = P::mul(tb, ab);
+    }
+    else if constexpr (LIGHTS) { // (if constexpr: the other instantiations keep their code exactly)
+        if (mtype == RRTB_DIFFUSE_LIGHT) {
+            ulonglong3 f;
+            P::const_fixed(tr, tg, tb, m.x, m.y, m.z, a.clamp, f.x, f.y, f.z);
+            emit(f);
+        }
+    }
+    return go_on;
+}
+
+// Adds a fixed-point triple to a pixel's sums (64-bit integer atomics: the order of arrival does not matter).
+__device__ __forceinline__ void accumulate(const RenderArgs &a, int pixel, ulonglong3 f)
+{
+    unsigned long long *dst = a.accum + 3ull * (unsigned long long)pixel;
+    atomicAdd(dst + 0, f.x);
+    atomicAdd(dst + 1, f.y);
+    atomicAdd(dst + 2, f.z);
+}
+
+// Counting build: the warp's sums of {rays, box, sphere, msphere, triangle tests, hits} into queue[1..6].
+__device__ __forceinline__ void flush_counters(const RenderArgs &a, unsigned long long rays, const TravCounters &tc,
+                                               unsigned long long hits)
+{
+    unsigned long long v[6] = {rays, tc.box, tc.sph, tc.msph, tc.tri, hits};
+    for (int k = 0; k < 6; ++k) {
+        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+        if ((threadIdx.x & 31u) == 0 && v[k]) atomicAdd(a.queue + 1 + k, v[k]);
+    }
+}
+
 // LIGHTS: the scene has emitters (RRTB_DIFFUSE_LIGHT) or a background; the other instantiations compile neither in
 template <class P, bool USE_BVH, bool COUNT_RAYS, bool LIGHTS = false>
 __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
@@ -70,7 +168,7 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
 
     // lane state
     int pixel = -1, ls = 0, ls_end = 0; // current item: pixel, local sample cursor, end
-    unsigned long long acc_r = 0, acc_g = 0, acc_b = 0;
+    ulonglong3 acc = make_ulonglong3(0ull, 0ull, 0ull); // the item's radiance so far, fixed point
     typename P::RayT ray;
     real thr_r = 1, thr_g = 1, thr_b = 1;
     int bounce = 0;
@@ -99,10 +197,8 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
                     unsigned long long tile_chunk = item >> 5;
                     int chunk = (int)(tile_chunk % (unsigned long long)a.n_chunks);
                     int ltile = (int)(tile_chunk / (unsigned long long)a.n_chunks);
-                    int tile = a.shard_mode == RRTB_SHARD_TILES ? ltile * a.world + a.rank : ltile;
-                    int ty = tile / a.tiles_x, tx = tile - ty * a.tiles_x;
-                    int i = tx * 8 + (int)(pit & 7u), j = ty * 4 + (int)(pit >> 3);
-                    if (i < a.W && j < a.H) {
+                    int i, j;
+                    if (local_pixel(a, ltile, pit, i, j)) {
                         pixel = j * a.W + i;
                         ls = chunk * CHUNK;
                         ls_end = min(ls + CHUNK, a.n_local_samples);
@@ -114,7 +210,7 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
         if (__all_sync(0xffffffffu, done)) break;
 
         if (pixel >= 0) {
-            const int sample = a.shard_mode == RRTB_SHARD_SAMPLES ? ls * a.world + a.rank : ls;
+            const int sample = global_sample(a, ls);
             if (!in_path) { // ---- generate: rrt.cu:112-114 + camera.h:31-38
                 ray = P::camera(a.cam, a.W, a.H, pixel % a.W, pixel / a.W, sample, a.key);
                 thr_r = thr_g = thr_b = 1;
@@ -129,67 +225,21 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
                 if (h.ref >= 0) ++hits;
             }
             // ---- shade: rrt.cu:50-76
-            bool path_end = false;
-            if (h.ref < 0) { // sky x throughput (rrt.cu:68-75), or background x throughput
-                unsigned long long fr, fg, fb;
-                if (LIGHTS && a.background) P::const_fixed(thr_r, thr_g, thr_b, a.bg[0], a.bg[1], a.bg[2], a.clamp, fr, fg, fb);
-                else P::sky_fixed(ray, thr_r, thr_g, thr_b, a.clamp, fr, fg, fb);
-                acc_r += fr;
-                acc_g += fg;
-                acc_b += fb;
-                path_end = true;
+            const auto add = [&](ulonglong3 f) { acc.x += f.x; acc.y += f.y; acc.z += f.z; };
+            if (h.ref < 0) add(miss_fixed<P, LIGHTS>(a, ray, thr_r, thr_g, thr_b));
+            else if (hit_step<P, true, LIGHTS>(a, leaves, info, ray, h, pixel, sample, bounce, thr_r, thr_g, thr_b, add)) {
+                ++bounce;
+                continue; // the path goes on
             }
-            else {
-                typename P::RecT rec = P::template record<true>(leaves, info, ray, h);
-                uint4 rnd = philox4x32_10(make_uint4((uint32_t)pixel, (uint32_t)sample, 2u + (uint32_t)bounce, 0u), a.key);
-                float4 m = __ldg(&s.materials[rec.mat]);
-                int mtype = __ldg(&s.material_type[rec.mat]);
-                real dx, dy, dz, ar, ag, ab;
-                if (P::template bounce<LIGHTS>(mtype, m, ray, rec, rnd, dx, dy, dz, ar, ag, ab)) {
-                    thr_r = P::mul(thr_r, ar);
-                    thr_g = P::mul(thr_g, ag);
-                    thr_b = P::mul(thr_b, ab);
-                    ray.ox = rec.px;
-                    ray.oy = rec.py;
-                    ray.oz = rec.pz;
-                    ray.dx = dx;
-                    ray.dy = dy;
-                    ray.dz = dz;
-                    if (++bounce >= a.max_depth) path_end = true; // exceeded depth: black (rrt.cu:78)
-                }
-                else {
-                    if constexpr (LIGHTS) { // (if constexpr: the other instantiations keep their code exactly)
-                        if (mtype == RRTB_DIFFUSE_LIGHT) { // an emitter: throughput x Le
-                            unsigned long long fr, fg, fb;
-                            P::const_fixed(thr_r, thr_g, thr_b, m.x, m.y, m.z, a.clamp, fr, fg, fb);
-                            acc_r += fr;
-                            acc_g += fg;
-                            acc_b += fb;
-                        }
-                    }
-                    path_end = true; // absorbed: black (rrt.cu:61-63), or an emitter
-                }
-            }
-            if (path_end) {
-                in_path = false;
-                if (++ls >= ls_end) { // ---- flush the chunk
-                    unsigned long long *dst = a.accum + 3ull * (unsigned long long)pixel;
-                    atomicAdd(dst + 0, acc_r);
-                    atomicAdd(dst + 1, acc_g);
-                    atomicAdd(dst + 2, acc_b);
-                    acc_r = acc_g = acc_b = 0;
-                    pixel = -1;
-                }
+            in_path = false;
+            if (++ls >= ls_end) { // ---- flush the chunk
+                accumulate(a, pixel, acc);
+                acc = make_ulonglong3(0ull, 0ull, 0ull);
+                pixel = -1;
             }
         }
     }
-    if (COUNT_RAYS) {
-        unsigned long long v[6] = {rays, tc.box, tc.sph, tc.msph, tc.tri, hits};
-        for (int k = 0; k < 6; ++k) {
-            for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-            if (lane == 0 && v[k]) atomicAdd(a.queue + 1 + k, v[k]);
-        }
-    }
+    if (COUNT_RAYS) flush_counters(a, rays, tc, hits);
 }
 
 } // namespace rrtb
@@ -216,8 +266,8 @@ __global__ void __launch_bounds__(256) k_resolve_tiles(const unsigned long long 
     const int lane = threadIdx.x & 31;
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     for (int tile = rank + warp * world; tile < n_tiles; tile += n_warps * world) {
-        const int ty = tile / tiles_x, tx = tile - ty * tiles_x;
-        const int i = tx * 8 + (lane & 7), j = ty * 4 + (lane >> 3);
+        int i, j;
+        tile_pixel(tile, tiles_x, lane, i, j);
         if (i < W && j < H) {
             const size_t k = 3 * ((size_t)j * W + i);
             out[k + 0] = (T)((double)acc[k + 0] * 9.094947017729282e-13); // 2^-40; float: one rounding, as k_resolve

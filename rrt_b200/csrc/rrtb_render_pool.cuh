@@ -15,9 +15,9 @@
 //   STEP     lanes in flight visit BVH nodes (the inner loop runs on while a vote finds enough of them),
 //            then, by vote, do one exact leaf test; a lane whose traversal ends writes (t, leaf ref) to its
 //            slot, pushes it on the scatter or the gen stack and is idle at once -- nobody waits for it
-//   SCATTER  32 hit slots, one per lane: hit record, Philox block, scatter; survivors -> trace stack (LIGHTS: an
-//            emitter hit adds throughput x Le to the accumulator here and ends its path)
-//   GEN      32 ended slots, one per lane: sky (LIGHTS: or background) x throughput into the accumulator (64-bit integer atomics),
+//   SCATTER  32 hit slots, one per lane: hit_step (hit record, Philox block, scatter); survivors -> trace stack
+//            (LIGHTS: an emitter hit adds throughput x Le to the accumulator here and ends its path)
+//   GEN      32 ended slots, one per lane: miss_fixed, sky (LIGHTS: or background) x throughput, into the accumulator,
 //            then the next camera paths of the global queue (ONE warp-aggregated atomicAdd per batch),
 //            Philox block, thin-lens ray -> trace stack
 //
@@ -130,29 +130,15 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
                     ++rays;
                     ++hits;
                 }
-                typename P::RecT rec = P::template record<MTRI>(leaves, info, r, h);
-                uint4 rnd = philox4x32_10(make_uint4((uint32_t)wp.pixel[sl], (uint32_t)wp.sample[sl], 2u + (uint32_t)bounce, 0u), a.key);
-                float4 m = __ldg(&s.materials[rec.mat]);
-                int mtype = __ldg(&s.material_type[rec.mat]);
-                real dx, dy, dz, ar, ag, ab;
-                if (P::template bounce<LIGHTS>(mtype, m, r, rec, rnd, dx, dy, dz, ar, ag, ab) && bounce + 1 < a.max_depth) {
-                    wp.ox[sl] = rec.px; wp.oy[sl] = rec.py; wp.oz[sl] = rec.pz;
-                    wp.dx[sl] = dx; wp.dy[sl] = dy; wp.dz[sl] = dz;
-                    wp.tr[sl] = P::mul(wp.tr[sl], ar); wp.tg[sl] = P::mul(wp.tg[sl], ag); wp.tb[sl] = P::mul(wp.tb[sl], ab);
+                const auto emit = [&](ulonglong3 f) { accumulate(a, wp.pixel[sl], f); };
+                if (hit_step<P, MTRI, LIGHTS>(a, leaves, info, r, h, wp.pixel[sl], wp.sample[sl], bounce, wp.tr[sl], wp.tg[sl],
+                                              wp.tb[sl], emit)) { // the throughput is updated in the slot
+                    wp.ox[sl] = r.ox; wp.oy[sl] = r.oy; wp.oz[sl] = r.oz;
+                    wp.dx[sl] = r.dx; wp.dy[sl] = r.dy; wp.dz[sl] = r.dz;
                     wp.bounce[sl] = bounce + 1;
                     to_trace = true;
                 }
-                else { // absorbed (rrt.cu:61-63) or depth exhausted (rrt.cu:78): black, nothing to accumulate
-                    if constexpr (LIGHTS) { // ... unless an emitter ended the path: throughput x Le, accumulated here
-                        if (mtype == RRTB_DIFFUSE_LIGHT) {
-                            unsigned long long fr, fg, fb;
-                            P::const_fixed(wp.tr[sl], wp.tg[sl], wp.tb[sl], m.x, m.y, m.z, a.clamp, fr, fg, fb);
-                            unsigned long long *dst = a.accum + 3ull * (unsigned long long)wp.pixel[sl];
-                            atomicAdd(dst + 0, fr);
-                            atomicAdd(dst + 1, fg);
-                            atomicAdd(dst + 2, fb);
-                        }
-                    }
+                else { // absorbed, out of depth or an emitter (whose term `emit` has accumulated)
                     wp.hit_ref[sl] = SLOT_FRESH;
                     ended = true;
                 }
@@ -173,21 +159,12 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
             const int sl = mine ? wp.gq[gq_n - 1 - lane] : 0;
             gq_n -= take;
             __syncwarp();
-            if (mine && wp.hit_ref[sl] == -1) { // the segment left the scene: sky x throughput (rrt.cu:68-75), or background
+            if (mine && wp.hit_ref[sl] == -1) { // the segment left the scene
                 if (COUNT_RAYS) ++rays;
-                unsigned long long fr, fg, fb;
-                if (LIGHTS && a.background) {
-                    P::const_fixed(wp.tr[sl], wp.tg[sl], wp.tb[sl], a.bg[0], a.bg[1], a.bg[2], a.clamp, fr, fg, fb);
-                }
-                else {
-                    typename P::RayT r;
-                    r.dx = wp.dx[sl]; r.dy = wp.dy[sl]; r.dz = wp.dz[sl];
-                    P::sky_fixed(r, wp.tr[sl], wp.tg[sl], wp.tb[sl], a.clamp, fr, fg, fb);
-                }
-                unsigned long long *dst = a.accum + 3ull * (unsigned long long)wp.pixel[sl];
-                atomicAdd(dst + 0, fr);
-                atomicAdd(dst + 1, fg);
-                atomicAdd(dst + 2, fb);
+                typename P::RayT r; // the miss term reads only the direction
+                r.dx = wp.dx[sl]; r.dy = wp.dy[sl]; r.dz = wp.dz[sl];
+                const ulonglong3 f = miss_fixed<P, LIGHTS>(a, r, wp.tr[sl], wp.tg[sl], wp.tb[sl]);
+                accumulate(a, wp.pixel[sl], f);
             }
             // next camera paths: one warp-aggregated atomic on the global queue
             bool to_trace = false;
@@ -215,20 +192,9 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
                         ls -= a.n_local_samples;
                         ++ltile;
                     }
-                    const int tile = a.shard_mode == RRTB_SHARD_TILES ? ltile * a.world + a.rank : ltile;
-                    int ty = (int)__fdividef((float)tile, (float)a.tiles_x); // float estimate, off by <= 1 ...
-                    int tx = tile - ty * a.tiles_x;
-                    if (tx < 0) { // ... corrected exactly in integers
-                        --ty;
-                        tx += a.tiles_x;
-                    }
-                    else if (tx >= a.tiles_x) {
-                        ++ty;
-                        tx -= a.tiles_x;
-                    }
-                    const int i = tx * 8 + (int)(pit & 7u), j = ty * 4 + (int)(pit >> 3);
-                    if (i < a.W && j < a.H) { // else: padding pixel of an edge tile, the slot asks again
-                        const int sample = a.shard_mode == RRTB_SHARD_SAMPLES ? ls * a.world + a.rank : ls;
+                    int i, j;
+                    if (local_pixel(a, ltile, pit, i, j)) { // else: padding pixel of an edge tile, the slot asks again
+                        const int sample = global_sample(a, ls);
                         typename P::RayT r = P::camera(a.cam, a.W, a.H, i, j, sample, a.key); // rrt.cu:112-114, camera.h:31-38
                         wp.ox[sl] = r.ox; wp.oy[sl] = r.oy; wp.oz[sl] = r.oz;
                         wp.dx[sl] = r.dx; wp.dy[sl] = r.dy; wp.dz[sl] = r.dz;
@@ -296,13 +262,7 @@ __global__ void __launch_bounds__(RENDER_TPB, P::BLOCKS_PER_SM) k_render_pool(co
             }
         }
     }
-    if (COUNT_RAYS) {
-        unsigned long long v[6] = {rays, tc.box, tc.sph, tc.msph, tc.tri, hits};
-        for (int k = 0; k < 6; ++k) {
-            for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-            if (lane == 0 && v[k]) atomicAdd(a.queue + 1 + k, v[k]);
-        }
-    }
+    if (COUNT_RAYS) flush_counters(a, rays, tc, hits);
 }
 
 } // namespace rrtb
