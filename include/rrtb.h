@@ -202,6 +202,30 @@ int rrtb_render(rrtb_ctx *ctx, const rrtb_render_params *p, float *out_rgb, rrtb
  * of the `rrtd` drop-in; rays, RNG and intersection arithmetic are those of rrtb_render. */
 int rrtb_render_f64(rrtb_ctx *ctx, const rrtb_render_params *p, double *out_rgb, rrtb_stats *stats);
 
+/* ---- first-hit AOVs (arbitrary output variables: denoiser guides, compositing) ------------------------------------
+ * For each pixel and sample s = 0 .. spp-1 the sample's PRIMARY SEGMENT: the camera ray of the beauty render (same
+ * Philox streams, lens sample and shutter time) and one closest-hit query with t_min = 0.001.  So the AOVs of samples
+ * 0 .. k-1 are those of the first segments of the beauty render's samples 0 .. k-1, whatever spp either uses.
+ * Per sample, on a hit / a miss:
+ *   albedo    the material's attenuation clamped per channel to [0, 1]: lambertian and metal the albedo, dielectric
+ *             (1, 1, 1), RRTB_DIFFUSE_LIGHT its Le                                                  / 0
+ *   normal    the hit record's face-forwarded normal (the one shading uses, against the ray)        / 0
+ *   depth     Euclidean distance from the ray origin to the hit point, t |d|                        / not counted
+ *   coverage  1                                                                                      / 0
+ * A miss reports 0, not the sky or the background: coverage tells where the background shows.  Per pixel the outputs
+ * are float means: albedo, normal and coverage the sum over the spp samples / spp, depth the sum over the samples that
+ * hit / their count (0 if none hit).  Each sum is a double accumulated in sample order 0 .. spp-1 (a miss leaves it as
+ * it is), divided once (correctly rounded) and rounded once to float.  The per-sample values are the integrator's:
+ * RRTB_PRECISION_F32 float t, normal and distance (sqrt and fma correctly rounded) widened to double when added,
+ * RRTB_PRECISION_F64 double throughout.  So the buffers do not depend on the grid, the scheduling, tree or flat scan,
+ * or the tile shard. */
+/* first-hit AOVs of the shard (p->rank, p->world) of a W x H image: HOST float buffers, bottom-up like rrtb_render;
+ * albedo3 / normal3 = 3*W*H, depth / coverage = W*H; pixels outside the shard are 0.  p->precision picks the integrator;
+ * p->max_depth and p->scheduler are ignored; p->shard_mode must be RRTB_SHARD_TILES.  stats: seconds_render is the AOV
+ * kernel's device time, paths and (count_rays) rays the primary segments, hits those that hit. */
+int rrtb_render_aov(rrtb_ctx *ctx, const rrtb_render_params *p, float *albedo3, float *normal3, float *depth,
+                    float *coverage, rrtb_stats *stats);
+
 /* Device-resident entry points (used by the multi-GPU host and bench.py):
  *   d_accum : DEVICE pointer (this GPU's memory, or a peer GPU's mapped over NVLink) to 3*W*H
  *             uint64 fixed-point accumulators (value * 2^40), pre-zeroed by the caller.  The kernel
@@ -347,6 +371,9 @@ int rrtb_tonemap_rgb8(const float *rgb_sum, int width, int height, int spp, uint
 int rrtb_tonemap_rgb8_f64(const double *rgb_sum, int width, int height, int spp, uint8_t *rgb8);
 /* PNG writer used where the reference calls stbi_write_png (main.cpp:164). */
 int rrtb_write_png(const char *path, int width, int height, const uint8_t *rgb8);
+/* PFM (Portable Float Map): channels 3 ("PF") or 1 ("Pf"), little endian (scale -1.0); PFM rows run bottom to top,
+ * which is this library's framebuffer order, so no flip */
+int rrtb_write_pfm(const char *path, int width, int height, int channels, const float *data);
 
 #ifdef __cplusplus
 }

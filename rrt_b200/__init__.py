@@ -4,6 +4,6 @@ The product is the CUDA library rrt_b200/librrtb200.so (C ABI: include/rrtb.h, s
 the drop-in `rrt` executable (rrt_b200/host).  This package is the thin ctypes binding over the C ABI
 (the reference's "add pybind11" to-do, README.md:66) used by the tests and bench.py.
 """
-from .api import Context, PinnedBuffer, Rrt, Scene, SceneError, camera_derive, render_group, tonemap, write_png  # noqa: F401
+from .api import Context, PinnedBuffer, Rrt, Scene, SceneError, camera_derive, render_group, tonemap, write_pfm, write_png  # noqa: F401
 from ._lib import RrtbError, LIB_PATH  # noqa: F401
 from .types import SceneArrays, RenderParams, Stats  # noqa: F401

@@ -14,12 +14,12 @@ LIB_PATH = os.environ.get("RRTB_LIB") or os.path.join(_HERE, "librrtb200.so")  #
 # every symbol include/rrtb.h declares (tests/test_abi.py checks the header against this list)
 SYMBOLS = [
     "rrtb_abi_version", "rrtb_create", "rrtb_destroy", "rrtb_last_error", "rrtb_device_info",
-    "rrtb_scene_set", "rrtb_scene_stage_moving_triangles", "rrtb_scene_stage_background", "rrtb_camera_set", "rrtb_render", "rrtb_render_f64", "rrtb_render_device", "rrtb_resolve_device",
+    "rrtb_scene_set", "rrtb_scene_stage_moving_triangles", "rrtb_scene_stage_background", "rrtb_camera_set", "rrtb_render", "rrtb_render_f64", "rrtb_render_aov", "rrtb_render_device", "rrtb_resolve_device",
     "rrtb_accumulate_device", "rrtb_frame_create", "rrtb_frame_export", "rrtb_frame_import", "rrtb_frame_attach", "rrtb_frame_detach",
     "rrtb_render_shard", "rrtb_frame_download", "rrtb_render_group", "rrtb_host_alloc", "rrtb_host_free", "rrtb_trace_closest", "rrtb_trace_closest_f64", "rrtb_camera_rays", "rrtb_camera_rays_f64",
     "rrtb_bvh_size", "rrtb_bvh_download", "rrtb_wide_size", "rrtb_wide_download", "rrtb_wide_download_raw", "rrtb_philox", "rrtb_scatter", "rrtb_scatter_f64", "rrtb_probe_issue_rate", "rrtb_scene_parse_file", "rrtb_scene_free", "rrtb_scene_counts",
     "rrtb_scene_camera", "rrtb_scene_materials", "rrtb_scene_spheres", "rrtb_scene_mspheres",
-    "rrtb_scene_triangles", "rrtb_scene_mtriangle_count", "rrtb_scene_mtriangles", "rrtb_scene_background", "rrtb_scene_upload", "rrtb_camera_derive", "rrtb_tonemap_rgb8", "rrtb_tonemap_rgb8_f64", "rrtb_write_png",
+    "rrtb_scene_triangles", "rrtb_scene_mtriangle_count", "rrtb_scene_mtriangles", "rrtb_scene_background", "rrtb_scene_upload", "rrtb_camera_derive", "rrtb_tonemap_rgb8", "rrtb_tonemap_rgb8_f64", "rrtb_write_png", "rrtb_write_pfm",
 ]
 
 STATUS = {0: "RRTB_OK", -1: "RRTB_ERR_INVALID", -2: "RRTB_ERR_NO_DEVICE", -3: "RRTB_ERR_CUDA", -4: "RRTB_ERR_NO_SCENE",
@@ -59,6 +59,7 @@ def load():
         "rrtb_camera_set": (C.c_int, [vp, vp]),
         "rrtb_render": (C.c_int, [vp, P(RenderParams), vp, P(Stats)]),
         "rrtb_render_f64": (C.c_int, [vp, P(RenderParams), vp, P(Stats)]),
+        "rrtb_render_aov": (C.c_int, [vp, P(RenderParams), vp, vp, vp, vp, P(Stats)]),
         "rrtb_render_device": (C.c_int, [vp, P(RenderParams), vp, P(Stats)]),
         "rrtb_resolve_device": (C.c_int, [vp, vp, vp, C.c_size_t]),
         "rrtb_accumulate_device": (C.c_int, [vp, vp, vp, C.c_size_t]),
@@ -101,6 +102,7 @@ def load():
         "rrtb_tonemap_rgb8": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp]),
         "rrtb_tonemap_rgb8_f64": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp]),
         "rrtb_write_png": (C.c_int, [C.c_char_p, C.c_int, C.c_int, vp]),
+        "rrtb_write_pfm": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_int, vp]),
     }
     for name in SYMBOLS:
         fn = getattr(lib, name)  # raises AttributeError if the library does not export it

@@ -239,6 +239,18 @@ class Context:
         self._check(fn(self.h, C.byref(p), C.c_void_p(out.ctypes.data), C.byref(st)))
         return out, st.as_dict()
 
+    def render_aov(self, width, height, spp, seed=1984, rank=0, world=1, count_rays=False, precision="f32"):
+        """First-hit AOVs (include/rrtb.h rrtb_render_aov) of tile shard (rank, world): dict of float32 MEANS albedo
+        [H, W, 3], normal [H, W, 3], depth [H, W], coverage [H, W] (row 0 = bottom scanline; pixels of other shards 0),
+        and the stats."""
+        p = self.params(width, height, spp, 1, seed, rank, world, 0, count_rays, 0, precision)
+        out = dict(albedo=np.zeros((height, width, 3), np.float32), normal=np.zeros((height, width, 3), np.float32),
+                   depth=np.zeros((height, width), np.float32), coverage=np.zeros((height, width), np.float32))
+        st = Stats()
+        self._check(self.lib.rrtb_render_aov(self.h, C.byref(p), _vp(out["albedo"]), _vp(out["normal"]), _vp(out["depth"]),
+                                             _vp(out["coverage"]), C.byref(st)))
+        return out, st.as_dict()
+
     def render_device(self, params, accum_ptr):
         """Device-resident path: adds this shard into the uint64 accumulator at device address accum_ptr."""
         st = Stats()
@@ -409,6 +421,16 @@ def write_png(path, rgb8):
         raise RrtbError(rc, "rrtb_write_png(%s)" % path)
 
 
+def write_pfm(path, array):
+    """rrtb_write_pfm: a float32 [H, W, 3] or [H, W] array (row 0 = bottom, the framebuffer order) as a little-endian PFM."""
+    lib = _lib.load()
+    a = np.ascontiguousarray(array, dtype=np.float32)
+    assert a.ndim in (2, 3) and (a.ndim == 2 or a.shape[2] in (1, 3)), a.shape
+    rc = lib.rrtb_write_pfm(str(path).encode(), a.shape[1], a.shape[0], 1 if a.ndim == 2 else a.shape[2], _vp(a))
+    if rc != 0:
+        raise RrtbError(rc, "rrtb_write_pfm(%s)" % path)
+
+
 class Rrt:
     """Mirror of the reference's `class Rrt` (rrt.h:14-48; CUDA build signature with threads_x/threads_y).
 
@@ -437,3 +459,10 @@ class Rrt:
         self.fb, self.stats = self.ctx.render(self.image_width, self.image_height, self.samples_per_pixel, self.max_depth, self.seed,
                                               count_rays=True, dtype=np.float64 if f64 else np.float32, precision=self.precision)
         return self.fb
+
+    def render_aov(self, the_scene):
+        """First-hit AOVs of the scene at this renderer's size, samples, seed and precision: (dict of albedo, normal,
+        depth, coverage means, as Context.render_aov), stats."""
+        self.ctx.set_scene(the_scene, self.bvh)
+        return self.ctx.render_aov(self.image_width, self.image_height, self.samples_per_pixel, self.seed, count_rays=True,
+                                   precision=self.precision)

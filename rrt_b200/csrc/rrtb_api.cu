@@ -119,6 +119,7 @@ void rrtb_destroy(rrtb_ctx *ctx)
     if (ctx->d_counters) cudaFree(ctx->d_counters);
     if (ctx->d_accum) cudaFree(ctx->d_accum);
     if (ctx->d_rgb) cudaFree(ctx->d_rgb);
+    if (ctx->d_aov) cudaFree(ctx->d_aov);
     if (ctx->peer_is_ipc) {
         if (ctx->peer_frame) cudaIpcCloseMemHandle(ctx->peer_frame);
         if (ctx->peer_sum) cudaIpcCloseMemHandle(ctx->peer_sum);
@@ -516,6 +517,28 @@ int rrtb_render(rrtb_ctx *ctx, const rrtb_render_params *p, float *out_rgb, rrtb
 int rrtb_render_f64(rrtb_ctx *ctx, const rrtb_render_params *p, double *out_rgb, rrtb_stats *stats)
 {
     return render_host(ctx, p, out_rgb, stats, true);
+}
+
+int rrtb_render_aov(rrtb_ctx *ctx, const rrtb_render_params *p, float *albedo3, float *normal3, float *depth, float *coverage,
+                    rrtb_stats *stats)
+{
+    int rc = check_render(ctx, p);
+    if (rc) return rc;
+    // a pixel's double sums split over sample shards would not add up to one GPU's bits
+    if (p->shard_mode != RRTB_SHARD_TILES) return invalid(ctx, "rrtb_render_aov shards by tiles only (RRTB_SHARD_TILES)");
+    if (!albedo3 || !normal3 || !depth || !coverage) return invalid(ctx, "null output buffer");
+    RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t n = (size_t)p->width * p->height;
+    if ((rc = dev_reserve(ctx, ctx->d_aov, 8 * n))) return rc;
+    rrtb_stats local;
+    memset(&local, 0, sizeof(local));
+    if ((rc = launch_aov(ctx, p, ctx->d_aov, &local))) return rc;
+    if ((rc = copy_to_host(ctx, albedo3, ctx->d_aov, 3 * n * sizeof(float)))) return rc;
+    if ((rc = copy_to_host(ctx, normal3, ctx->d_aov + 3 * n, 3 * n * sizeof(float)))) return rc;
+    if ((rc = copy_to_host(ctx, depth, ctx->d_aov + 6 * n, n * sizeof(float)))) return rc;
+    if ((rc = copy_to_host(ctx, coverage, ctx->d_aov + 7 * n, n * sizeof(float)))) return rc;
+    if (stats) *stats = local;
+    return RRTB_OK;
 }
 
 // ---- multi-GPU frame (SURVEY 8e) ---------------------------------------------------------------------------------

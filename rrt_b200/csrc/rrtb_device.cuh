@@ -789,6 +789,26 @@ __device__ __forceinline__ void sky(const Ray &r, float &cr, float &cg, float &c
     cb = fmaf(t, 1.0f, w);
 }
 
+// ---- first-hit AOVs (rrtb_render_aov) ------------------------------------------------------------------------
+// The albedo of a hit: the material's attenuation (lambertian and metal: the albedo, dielectric: 1, an emitter: its Le),
+// clamped per channel to [0, 1].
+__device__ __forceinline__ void aov_albedo(int mtype, float4 m, float &r, float &g, float &b)
+{
+    if (mtype == RRTB_DIELECTRIC) {
+        r = g = b = 1.0f;
+        return;
+    }
+    r = fminf(fmaxf(m.x, 0.0f), 1.0f);
+    g = fminf(fmaxf(m.y, 0.0f), 1.0f);
+    b = fminf(fmaxf(m.z, 0.0f), 1.0f);
+}
+
+// Euclidean distance from the ray's origin to its point at t: t |d| (camera directions are not unit length)
+__device__ __forceinline__ float ray_distance(const Ray &r, float t)
+{
+    return __fmul_rn(t, __fsqrt_rn(__fmaf_rn(r.dz, r.dz, __fmaf_rn(r.dy, r.dy, __fmul_rn(r.dx, r.dx)))));
+}
+
 // The per-sample radiance clamp of a render of spp samples in all (every shard uses the same value):
 // C = min(2^20, 2^(23 - ceil(log2 spp))), a power of two, so that spp * C * 2^40 <= 2^63 and no pixel sum can wrap,
 // whatever the albedos.  spp <= 2^23 (rrtb_render_params.spp): C >= 1, so radiance <= 1 (sky through albedos

@@ -363,6 +363,12 @@ __device__ __forceinline__ void sky_d(const RayD &r, double tr, double tg, doubl
     cb = __dmul_rn(tb, __fma_rn(t, 1.0, w));
 }
 
+// ray_distance of rrtb_device.cuh in double
+__device__ __forceinline__ double ray_distance_d(const RayD &r, double t)
+{
+    return __dmul_rn(t, __dsqrt_rn(ddot3(r.dx, r.dy, r.dz, r.dx, r.dy, r.dz)));
+}
+
 // radiance -> 2^40 fixed point, clamped to [0, clamp] (to_fixed in rrtb_device.cuh)
 __device__ __forceinline__ unsigned long long to_fixed_d(double x, double clamp)
 {

@@ -565,4 +565,25 @@ int rrtb_write_png(const char *path, int width, int height, const uint8_t *rgb8)
     return ok ? RRTB_OK : RRTB_ERR_IO;
 }
 
+
+// PFM (Portable Float Map): "PF" (3 channels) or "Pf" (1), width height, scale -1.0 (little endian), then the rows bottom
+// to top, which is the framebuffer's own order.  The floats are written byte by byte, so the file is the same on any host.
+int rrtb_write_pfm(const char *path, int width, int height, int channels, const float *data)
+{
+    if (!path || !data || width <= 0 || height <= 0 || (channels != 1 && channels != 3)) return RRTB_ERR_INVALID;
+    const size_t n = (size_t)width * height * channels;
+    std::vector<uint8_t> raw(4 * n);
+    for (size_t k = 0; k < n; ++k) {
+        uint32_t b;
+        memcpy(&b, data + k, 4);
+        for (int q = 0; q < 4; ++q) raw[4 * k + q] = (uint8_t)(b >> (8 * q));
+    }
+    FILE *f = fopen(path, "wb");
+    if (!f) return RRTB_ERR_IO;
+    bool ok = fprintf(f, "%s\n%d %d\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height) > 0;
+    ok = fwrite(raw.data(), 1, raw.size(), f) == raw.size() && ok;
+    ok = fclose(f) == 0 && ok;
+    return ok ? RRTB_OK : RRTB_ERR_IO;
+}
+
 } // extern "C"

@@ -72,6 +72,7 @@ struct rrtb_ctx {
     unsigned long long *d_accum = nullptr;    // host-path accumulator (3*W*H)
     float *d_rgb = nullptr;                   // host-path float framebuffer
     size_t accum_elems = 0;
+    float *d_aov = nullptr;                   // rrtb_render_aov's output, 8*W*H floats (grow-only)
     unsigned char *d_stage = nullptr;         // raw scene structs of the last upload (input of k_prepare; kept for rebuilds)
     size_t stage_off[4] = {0, 0, 0, 0};       // byte offsets of the sphere / msphere / triangle / mtriangle arrays in d_stage
     float build_cam_mag = 0.f;                // camera magnitude the traversal-box padding was computed with
@@ -114,6 +115,8 @@ DeviceScene device_scene(const rrtb_ctx *ctx);
 DeviceCamera device_camera(const rrtb_camera &c, int W, int H);
 int launch_render(rrtb_ctx *ctx, const rrtb_render_params *p, uint64_t *d_accum, rrtb_stats *stats, bool defer = false);
 int finish_render(rrtb_ctx *ctx, rrtb_stats *stats);
+// first-hit AOVs of a tile shard into d_out (8*W*H floats, planar: albedo, normal, depth, coverage); synchronises
+int launch_aov(rrtb_ctx *ctx, const rrtb_render_params *p, float *d_out, rrtb_stats *stats);
 int launch_resolve_tiles(rrtb_ctx *ctx, const uint64_t *d_accum, void *d_out, const rrtb_render_params *p, bool f64);
 int launch_accumulate_atomic(rrtb_ctx *ctx, uint64_t *d_dst, const uint64_t *d_src, size_t n);
 int launch_accumulate(rrtb_ctx *ctx, uint64_t *d_dst, const uint64_t *d_src, size_t n);

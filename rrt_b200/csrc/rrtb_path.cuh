@@ -76,6 +76,9 @@ struct PathF32 { // the float integrator (rrtb_device.cuh)
     {
         return camera_ray(cam, W, H, i, j, sample, key);
     }
+    // first-hit AOVs: the clamped albedo of a hit and the distance to it
+    static __device__ __forceinline__ void albedo(int mtype, float4 m, float &r, float &g, float &b) { aov_albedo(mtype, m, r, g, b); }
+    static __device__ __forceinline__ float distance(const Ray &r, float t) { return ray_distance(r, t); }
 };
 
 struct PathF64 { // the double integrator (rrtb_device_f64.cuh); bit-exact against oracle/rrt_oracle_f64.c
@@ -140,6 +143,16 @@ struct PathF64 { // the double integrator (rrtb_device_f64.cuh); bit-exact again
     {
         return camera_ray_d(cam, W, H, i, j, sample, key);
     }
+    // the albedo is clamped in float and widened: exact, and the same as clamping the widened value
+    static __device__ __forceinline__ void albedo(int mtype, float4 m, double &r, double &g, double &b)
+    {
+        float fr, fg, fb;
+        aov_albedo(mtype, m, fr, fg, fb);
+        r = fr;
+        g = fg;
+        b = fb;
+    }
+    static __device__ __forceinline__ double distance(const RayD &r, double t) { return ray_distance_d(r, t); }
 };
 
 template <typename real>

@@ -242,6 +242,84 @@ __global__ void __launch_bounds__(RENDER_TPB, 2) k_render(const RenderArgs a)
     if (COUNT_RAYS) flush_counters(a, rays, tc, hits);
 }
 
+// ---- first-hit AOVs (rrtb_render_aov) -----------------------------------------------------------------------------
+// The primary segment of every sample of a pixel: camera ray, one closest-hit query, and on a hit the clamped albedo,
+// the face-forwarded normal of the hit record and the distance t |d|.  A lane owns one pixel and runs its samples in
+// order, summing in double (a miss leaves the sums as they are), so the means depend on neither the grid nor the tree.
+struct AovArgs {
+    DeviceScene scene;
+    DeviceCamera cam;
+    int W, H, spp;
+    uint2 key;
+    int rank, world, tiles_x;
+    int n_local_tiles;         // tiles owned by this rank (RRTB_SHARD_TILES)
+    float *out;                // planar: albedo 3*W*H, normal 3*W*H, depth W*H, coverage W*H
+    unsigned long long *queue; // [0] tile queue head, [1..6] the counters of RenderArgs::queue
+};
+
+// persistent: each warp draws one 8x4-pixel tile at a time off the queue, lane = pixel in tile
+template <class P, bool USE_BVH, bool COUNT_RAYS>
+__global__ void __launch_bounds__(RENDER_TPB, 2) k_render_aov(const AovArgs a)
+{
+    typedef typename P::real real;
+    const unsigned lane = threadIdx.x & 31u;
+    const DeviceScene &s = a.scene;
+    const float4 *__restrict__ leaves = USE_BVH ? s.leaves : s.flat_leaves;
+    const LeafAux info = USE_BVH ? LeafAux{s.leaf_info, s.leaf_ext} : LeafAux{s.flat_info, s.flat_ext};
+    const size_t n = (size_t)a.W * a.H;
+    unsigned long long rays = 0, hits = 0;
+    TravCounters tc = {0ull, 0ull, 0ull, 0ull};
+
+    while (true) {
+        unsigned long long ltile = 0;
+        if (lane == 0) ltile = atomicAdd(a.queue, 1ull);
+        ltile = __shfl_sync(0xffffffffu, ltile, 0);
+        if (ltile >= (unsigned long long)a.n_local_tiles) break;
+        int i, j;
+        tile_pixel((int)ltile * a.world + a.rank, a.tiles_x, lane, i, j);
+        if (i >= a.W || j >= a.H) continue; // padding pixel of an edge tile
+        double al[3] = {0.0, 0.0, 0.0}, nm[3] = {0.0, 0.0, 0.0}, dist = 0.0;
+        int n_hit = 0;
+        for (int smp = 0; smp < a.spp; ++smp) {
+            const typename P::RayT ray = P::camera(a.cam, a.W, a.H, i, j, smp, a.key);
+            const real t_min = (real)0.001;
+            const typename P::HitT h = USE_BVH ? closest_bvh<P, COUNT_RAYS>(s, ray, t_min, tc) : closest_scan<P, COUNT_RAYS>(s, ray, t_min, tc);
+            if (COUNT_RAYS) {
+                ++rays;
+                if (h.ref >= 0) ++hits;
+            }
+            if (h.ref < 0) continue;
+            const typename P::RecT rec = P::template record<true>(leaves, info, ray, h);
+            real ar, ag, ab;
+            P::albedo(__ldg(&s.material_type[rec.mat]), __ldg(&s.materials[rec.mat]), ar, ag, ab);
+            al[0] = __dadd_rn(al[0], (double)ar);
+            al[1] = __dadd_rn(al[1], (double)ag);
+            al[2] = __dadd_rn(al[2], (double)ab);
+            nm[0] = __dadd_rn(nm[0], (double)rec.nx);
+            nm[1] = __dadd_rn(nm[1], (double)rec.ny);
+            nm[2] = __dadd_rn(nm[2], (double)rec.nz);
+            dist = __dadd_rn(dist, (double)P::distance(ray, h.t));
+            ++n_hit;
+        }
+        // each mean: one correctly rounded division, one rounding to float
+        const double spp = (double)a.spp;
+        const size_t p = (size_t)j * a.W + i;
+        for (int k = 0; k < 3; ++k) {
+            a.out[3 * p + k] = __double2float_rn(__ddiv_rn(al[k], spp));
+            a.out[3 * n + 3 * p + k] = __double2float_rn(__ddiv_rn(nm[k], spp));
+        }
+        a.out[6 * n + p] = n_hit ? __double2float_rn(__ddiv_rn(dist, (double)n_hit)) : 0.0f;
+        a.out[7 * n + p] = __double2float_rn(__ddiv_rn((double)n_hit, spp));
+    }
+    if (COUNT_RAYS) { // the warp's sums of {rays, box, sphere, msphere, triangle tests, hits} into queue[1..6], as flush_counters
+        unsigned long long v[6] = {rays, tc.box, tc.sph, tc.msph, tc.tri, hits};
+        for (int k = 0; k < 6; ++k) {
+            for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+            if (lane == 0 && v[k]) atomicAdd(a.queue + 1 + k, v[k]);
+        }
+    }
+}
+
 } // namespace rrtb
 #include "rrtb_render_pool.cuh"
 namespace rrtb {
@@ -648,6 +726,51 @@ int finish_render(rrtb_ctx *ctx, rrtb_stats *stats)
 #endif
     }
     return RRTB_OK;
+}
+
+// the AOV kernel: persistent, one wave, at most one warp per owned tile
+template <class P, bool USE_BVH>
+static int launch_aov_kernel(rrtb_ctx *ctx, const AovArgs &a, bool cnt)
+{
+    auto kernel = cnt ? k_render_aov<P, USE_BVH, true> : k_render_aov<P, USE_BVH, false>;
+    int per_sm = 0;
+    RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, 0));
+    if (per_sm < 1) per_sm = 1;
+    const int want = (a.n_local_tiles + RENDER_TPB / 32 - 1) / (RENDER_TPB / 32);
+    const int blocks = min(ctx->sm_count * per_sm, max(want, 1));
+    kernel<<<blocks, RENDER_TPB, 0, ctx->stream>>>(a);
+    return RRTB_OK;
+}
+
+int launch_aov(rrtb_ctx *ctx, const rrtb_render_params *p, float *d_out, rrtb_stats *stats)
+{
+    const ShardGeometry g = shard_geometry(p); // p->shard_mode is RRTB_SHARD_TILES (rrtb_render_aov)
+    AovArgs a;
+    a.scene = device_scene(ctx);
+    a.cam = device_camera(ctx->cam, p->width, p->height);
+    a.W = p->width;
+    a.H = p->height;
+    a.spp = p->spp;
+    a.key = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
+    a.rank = g.rank;
+    a.world = g.world;
+    a.tiles_x = g.tiles_x;
+    a.n_local_tiles = g.n_local_tiles;
+    a.out = d_out;
+    a.queue = ctx->d_counters;
+    RRTB_CUDA(ctx, cudaMemsetAsync(d_out, 0, 8 * sizeof(float) * (size_t)p->width * p->height, ctx->stream)); // pixels of other shards
+    RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_counters, 0, 8 * sizeof(unsigned long long), ctx->stream));
+    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    typedef int (*Launcher)(rrtb_ctx *, const AovArgs &, bool);
+    static const Launcher launch[2][2] = {{launch_aov_kernel<PathF32, false>, launch_aov_kernel<PathF32, true>},
+                                          {launch_aov_kernel<PathF64, false>, launch_aov_kernel<PathF64, true>}};
+    const int rc = launch[p->precision == RRTB_PRECISION_F64][ctx->use_bvh != 0](ctx, a, p->count_rays != 0);
+    if (rc) return rc;
+    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    RRTB_CUDA(ctx, cudaGetLastError());
+    ctx->pending = *p;
+    ctx->pending_launches = 1;
+    return finish_render(ctx, stats); // device time, counters and primary segments (stats.paths) as for a render
 }
 
 template <typename T>

@@ -7,6 +7,8 @@
 //                    -I <list>  frame batch (reference README.md:64 to-do "input list of scenes to render")
 //                    -G <n>     n GPUs of this box: one context + one host thread per GPU, each renders its
 //                               interleaved tiles; the shards are disjoint, so summing them is exact
+//                    -A <prefix> linear float PFMs after the render: <prefix>.color.pfm (sum / spp) and the first-hit
+//                               AOVs <prefix>.{albedo,normal,depth,coverage}.pfm (rrtb_render_aov, on the first device)
 //   usage + exit 1   on any unknown argument                       (main.cpp:33-51)
 //   exit 1 "no scene loaded" / 2 cannot open / 3 unknown material / 4 missing camera|materials|objects
 //                                                                  (main.cpp:126-127, scene.h:220-223,287-290,431-442)
@@ -65,6 +67,8 @@ static void usage(const char *argv)
     std::cerr << "  -G <n>              : render on n GPUs (devices D..D+n-1), interleaved 8x4-pixel tiles (1)\n";
     std::cerr << "  -I list.txt         : frame batch: one '<scene.txt> <out.png>' per line; scenes that differ only\n";
     std::cerr << "                        in their camera reuse the uploaded scene and its BVH\n";
+    std::cerr << "  -A <prefix>         : also write <prefix>.color.pfm (linear mean) and the first-hit AOVs\n";
+    std::cerr << "                        <prefix>.albedo.pfm, .normal.pfm, .depth.pfm, .coverage.pfm (not with -I)\n";
     std::exit(1);
 }
 
@@ -169,6 +173,7 @@ int main(int argc, char *argv[])
     std::string batch_list;
     int n_gpus = 1;
     bool count_rays = false;
+    std::string aov_prefix;
 
     // Only the first letter after '-' is examined, as in the reference (so "-input" == "-i").
     for (int i = 1; i < argc; ++i) {
@@ -196,8 +201,10 @@ int main(int argc, char *argv[])
         else if (c == 'I') batch_list = next();
         else if (c == 'G') n_gpus = atoi(next());
         else if (c == 'R') count_rays = true;
+        else if (c == 'A') aov_prefix = next();
         else usage(argv[i]);
     }
+    if (aov_prefix != "" && batch_list != "") usage("-A (with -I)");
 
     if (batch_list != "")
         return run_batch(batch_list, image_width, image_height, num_samples, max_depth, use_bvh, num_threads_x, num_threads_y,
@@ -284,6 +291,26 @@ int main(int argc, char *argv[])
         if (rrtb_write_png(png_filename, image_width, image_height, rgb.data()) != RRTB_OK) {
             std::cerr << "ERROR: could not write " << png_filename << std::endl;
             std::exit(1);
+        }
+    }
+    if (aov_prefix != "") { // linear PFMs: the beauty mean, then the first-hit AOVs at the same samples, seed and precision
+        const size_t n = (size_t)image_width * image_height;
+        std::vector<float> color(3 * n), albedo(3 * n), normal(3 * n), depth(n), coverage(n);
+        for (size_t k = 0; k < n; ++k)
+            for (int c = 0; c < 3; ++c) color[3 * k + c] = (float)(fb[k].e[c] / (FP_T)num_samples);
+        rrt.render_aov(albedo.data(), normal.data(), depth.data(), coverage.data());
+        const struct {
+            const char *name;
+            int channels;
+            const float *data;
+        } pfm[5] = {{".color.pfm", 3, color.data()}, {".albedo.pfm", 3, albedo.data()}, {".normal.pfm", 3, normal.data()},
+                    {".depth.pfm", 1, depth.data()}, {".coverage.pfm", 1, coverage.data()}};
+        for (const auto &f : pfm) {
+            const std::string path = aov_prefix + f.name;
+            if (rrtb_write_pfm(path.c_str(), image_width, image_height, f.channels, f.data) != RRTB_OK) {
+                std::cerr << "ERROR: could not write " << path << std::endl;
+                std::exit(1);
+            }
         }
     }
     rrtb_scene_free(the_scene);

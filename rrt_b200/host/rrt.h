@@ -111,6 +111,24 @@ class Rrt {
         return fb.data();
     }
 
+    // First-hit AOVs (rrtb_render_aov) of the uploaded scene at this object's size, samples, seed and precision: float
+    // means, bottom-up; albedo3 / normal3 hold 3*W*H floats, depth / coverage W*H.
+    void render_aov(float *albedo3, float *normal3, float *depth, float *coverage)
+    {
+        rrtb_render_params p{};
+        p.width = image_width;
+        p.height = image_height;
+        p.spp = samples_per_pixel;
+        p.max_depth = max_depth;
+        p.seed = seed;
+        p.rank = rank;
+        p.world = world;
+        p.shard_mode = RRTB_SHARD_TILES;
+        p.precision = RRTB_FP_PRECISION;
+        rrtb_stats st;
+        rrtb_check(rrtb_render_aov(ctx, &p, albedo3, normal3, depth, coverage, &st), ctx, "rrtb_render_aov");
+    }
+
     bool count_rays = false;
     bool warmed = false;
 
