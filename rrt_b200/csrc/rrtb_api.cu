@@ -28,8 +28,12 @@ int cuda_fail(rrtb_ctx *ctx, cudaError_t e, const char *expr, const char *file, 
     return RRTB_ERR_CUDA;
 }
 
-int prepare_and_build(rrtb_ctx *ctx, const rrtb_sphere *d_sph, const rrtb_msphere *d_msph, const rrtb_triangle *d_tri,
-                      const rrtb_mtriangle *d_mtri);
+int read_back(rrtb_ctx *ctx, void *dst, const void *d_src, size_t bytes)
+{
+    RRTB_CUDA(ctx, cudaMemcpyAsync(dst, d_src, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return RRTB_OK;
+}
 
 static int invalid(rrtb_ctx *ctx, const char *msg)
 {
@@ -37,25 +41,60 @@ static int invalid(rrtb_ctx *ctx, const char *msg)
     return RRTB_ERR_INVALID;
 }
 
-// grow-only device buffer: reallocated only when the request exceeds what the member already holds
-template <typename T>
-static int dev_reserve(rrtb_ctx *ctx, T *&p, size_t count)
+static int require_scene(rrtb_ctx *ctx, const char *msg)
 {
-    if (count == 0) count = 1;
-    const size_t bytes = count * sizeof(T);
-    size_t &cap = ctx->capacity[(const void *)&p];
-    if (p && cap >= bytes) return RRTB_OK;
-    if (p) {
-        cudaFree(p);
-        p = nullptr;
-        cap = 0;
+    if (ctx->has_scene) return RRTB_OK;
+    ctx->err = msg;
+    return RRTB_ERR_NO_SCENE;
+}
+
+static void frame_drop_mapping(rrtb_ctx *ctx)
+{
+    if (ctx->peer_is_ipc) {
+        if (ctx->peer_frame) cudaIpcCloseMemHandle(ctx->peer_frame);
+        if (ctx->peer_sum) cudaIpcCloseMemHandle(ctx->peer_sum);
     }
-    RRTB_CUDA(ctx, cudaMalloc((void **)&p, bytes));
-    cap = bytes;
+    ctx->peer_frame = nullptr;
+    ctx->peer_sum = nullptr;
+    ctx->peer_is_ipc = false;
+}
+
+// Builds the acceleration structure from the raw scene in d_stage and marks the scene renderable.  `upload()` enqueues
+// what the build reads that is not on the device yet; stats.seconds_build times it together with the build.
+template <typename Upload>
+static int build_scene(rrtb_ctx *ctx, Upload &&upload)
+{
+    cudaStream_t st = ctx->stream;
+    ctx->has_scene = false; // until the build below has succeeded
+    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
+    int rc = upload();
+    if (rc || (rc = prepare_and_build(ctx))) return rc;
+    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev1, st));
+    // did the collapse kernel's work list drain (CollapseState::stuck == 0)?  Read back behind the build into pinned
+    // memory: it costs no synchronisation of its own
+    if ((rc = ctx->h_state.reserve(ctx, 4))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_collapse, 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    RRTB_CUDA(ctx, cudaStreamSynchronize(st)); // the caller's host arrays may go away after this
+    float ms = 0.f;
+    RRTB_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    ctx->seconds_build = ms * 1e-3;
+    if (ctx->h_state[3]) {
+        ctx->err = "internal error: the 4-wide collapse did not terminate (inconsistent tree)";
+        return RRTB_ERR_CUDA;
+    }
+    ctx->has_scene = true;
     return RRTB_OK;
 }
 
 } // namespace rrtb
+
+rrtb_ctx::~rrtb_ctx()
+{
+    rrtb::frame_drop_mapping(this);
+    for (cudaEvent_t e : {ev0, ev1, ev2, ev3, ev_copy[0], ev_copy[1]})
+        if (e) cudaEventDestroy(e);
+    if (stream) cudaStreamDestroy(stream);
+}
 
 using namespace rrtb;
 
@@ -83,7 +122,7 @@ int rrtb_create(rrtb_ctx **out, int device)
     }
     rrtb_ctx *ctx = new rrtb_ctx();
     ctx->device = device;
-    auto fail = [&](int rc) {
+    auto fail = [&](int rc) { // the destructor releases what was created so far
         {
             std::lock_guard<std::mutex> lk(g_mutex);
             g_create_error = ctx->err;
@@ -105,8 +144,8 @@ int rrtb_create(rrtb_ctx **out, int device)
     CREATE_CUDA(cudaEventCreate(&ctx->ev1));
     CREATE_CUDA(cudaEventCreate(&ctx->ev2));
     CREATE_CUDA(cudaEventCreate(&ctx->ev3));
-    CREATE_CUDA(cudaMalloc((void **)&ctx->d_counters, 8 * sizeof(unsigned long long)));
 #undef CREATE_CUDA
+    if (int rc = ctx->d_counters.reserve(ctx, 8)) return fail(rc);
     *out = ctx;
     return RRTB_OK;
 }
@@ -115,22 +154,6 @@ void rrtb_destroy(rrtb_ctx *ctx)
 {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    free_scene(ctx);
-    if (ctx->d_counters) cudaFree(ctx->d_counters);
-    if (ctx->d_accum) cudaFree(ctx->d_accum);
-    if (ctx->d_rgb) cudaFree(ctx->d_rgb);
-    if (ctx->d_aov) cudaFree(ctx->d_aov);
-    if (ctx->peer_is_ipc) {
-        if (ctx->peer_frame) cudaIpcCloseMemHandle(ctx->peer_frame);
-        if (ctx->peer_sum) cudaIpcCloseMemHandle(ctx->peer_sum);
-    }
-    if (ctx->d_frame) cudaFree(ctx->d_frame);
-    if (ctx->d_sum) cudaFree(ctx->d_sum);
-    if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-    if (ctx->h_state) cudaFreeHost(ctx->h_state);
-    for (cudaEvent_t e : {ctx->ev0, ctx->ev1, ctx->ev2, ctx->ev3, ctx->ev_copy[0], ctx->ev_copy[1]})
-        if (e) cudaEventDestroy(e);
-    if (ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
 
@@ -168,25 +191,6 @@ int rrtb_device_info(rrtb_ctx *ctx, int64_t *out4, char *name, int name_len)
 // spheres: 26.1 Grays/s with motion nodes, 28.5 with shutter-spanning boxes), many do (64 fast spheres: less than half the
 // exact tests per ray), so they are used from 8 moving primitives on, under an open shutter.
 static bool use_motion_nodes(int n_moving, const rrtb_camera *cam) { return n_moving >= 8 && cam->time0 != cam->time1; }
-
-// The collapse kernel's work list drained (CollapseState::stuck == 0)?  fetch_collapse_state enqueues the read-back
-// behind the build (pinned destination: it costs no synchronisation of its own), check_collapse reads it after the
-// stream has been synchronised.
-static int fetch_collapse_state(rrtb_ctx *ctx)
-{
-    if (!ctx->h_state) RRTB_CUDA(ctx, cudaHostAlloc((void **)&ctx->h_state, 4 * sizeof(int), cudaHostAllocPortable));
-    RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_collapse, 4 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    return RRTB_OK;
-}
-
-static int check_collapse(rrtb_ctx *ctx)
-{
-    if (ctx->h_state[3]) {
-        ctx->err = "internal error: the 4-wide collapse did not terminate (inconsistent tree)";
-        return RRTB_ERR_CUDA;
-    }
-    return RRTB_OK;
-}
 
 int rrtb_scene_stage_moving_triangles(rrtb_ctx *ctx, const rrtb_mtriangle *mtriangles, int n_mtriangles)
 {
@@ -265,41 +269,41 @@ int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *m
     const size_t b_msph = (sizeof(rrtb_msphere) * (size_t)n_mspheres + 15) & ~(size_t)15;
     const size_t b_tri = (sizeof(rrtb_triangle) * (size_t)n_triangles + 15) & ~(size_t)15;
     const size_t b_mtri = (sizeof(rrtb_mtriangle) * (size_t)n_mtriangles + 15) & ~(size_t)15;
-    if ((rc = dev_reserve(ctx, ctx->d_prim, (size_t)3 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_prim_info, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_materials, (size_t)n_materials))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_material_type, (size_t)n_materials))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_prim_box, (size_t)6 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_morton, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_keys, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_keys_tmp, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_left, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_right, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_parent, (size_t)2 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_node_box, (size_t)6 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_visit, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_range, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_left2, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_right2, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_parent2, (size_t)2 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_node_box2, (size_t)6 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_sah_roots, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_wnodes, (size_t)(n_mspheres + n_mtriangles > 0 ? RRTB_MOTION_NODE_F4 : RRTB_NODE_F4) * n))) return rc;
+    if ((rc = ctx->d_prim.reserve(ctx, (size_t)3 * n))) return rc;
+    if ((rc = ctx->d_prim_info.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_materials.reserve(ctx, (size_t)n_materials))) return rc;
+    if ((rc = ctx->d_material_type.reserve(ctx, (size_t)n_materials))) return rc;
+    if ((rc = ctx->d_prim_box.reserve(ctx, (size_t)6 * n))) return rc;
+    if ((rc = ctx->d_morton.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_keys.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_keys_tmp.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_left.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_right.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_parent.reserve(ctx, (size_t)2 * n))) return rc;
+    if ((rc = ctx->d_node_box.reserve(ctx, (size_t)6 * n))) return rc;
+    if ((rc = ctx->d_visit.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_range.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_left2.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_right2.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_parent2.reserve(ctx, (size_t)2 * n))) return rc;
+    if ((rc = ctx->d_node_box2.reserve(ctx, (size_t)6 * n))) return rc;
+    if ((rc = ctx->d_sah_roots.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_wnodes.reserve(ctx, (size_t)(n_mspheres + n_mtriangles > 0 ? RRTB_MOTION_NODE_F4 : RRTB_NODE_F4) * n))) return rc;
     if (n_mspheres + n_mtriangles > 0) { // room for the end-of-shutter boxes whatever this camera's shutter is (rrtb_camera_set may open it)
-        if ((rc = dev_reserve(ctx, ctx->d_prim_box01, (size_t)12 * n))) return rc;
-        if ((rc = dev_reserve(ctx, ctx->d_node_box01, (size_t)12 * n))) return rc;
+        if ((rc = ctx->d_prim_box01.reserve(ctx, (size_t)12 * n))) return rc;
+        if ((rc = ctx->d_node_box01.reserve(ctx, (size_t)12 * n))) return rc;
     }
-    if ((rc = dev_reserve(ctx, ctx->d_wq, (size_t)n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_collapse, (size_t)16))) return rc; // CollapseState, SahState
-    if ((rc = dev_reserve(ctx, ctx->d_leaves, (size_t)3 * n))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_leaf_info, (size_t)n))) return rc;
+    if ((rc = ctx->d_wq.reserve(ctx, (size_t)n))) return rc;
+    if ((rc = ctx->d_collapse.reserve(ctx, (size_t)16))) return rc; // CollapseState, SahState
+    if ((rc = ctx->d_leaves.reserve(ctx, (size_t)3 * n))) return rc;
+    if ((rc = ctx->d_leaf_info.reserve(ctx, (size_t)n))) return rc;
     if (n_mtriangles > 0) { // edge rates of moving triangles (SURVEY 8f4): two float4 per slot, only for scenes that have them
-        if ((rc = dev_reserve(ctx, ctx->d_prim_ext, (size_t)2 * n))) return rc;
-        if ((rc = dev_reserve(ctx, ctx->d_leaf_ext, (size_t)2 * n))) return rc;
+        if ((rc = ctx->d_prim_ext.reserve(ctx, (size_t)2 * n))) return rc;
+        if ((rc = ctx->d_leaf_ext.reserve(ctx, (size_t)2 * n))) return rc;
     }
-    if ((rc = dev_reserve(ctx, ctx->d_reduce, (size_t)nb * 7 + 16))) return rc;
-    if ((rc = dev_reserve(ctx, ctx->d_hist, (size_t)256 * n_seg + (size_t)(256 * n_seg + 4095) / 4096 + 1))) return rc; // + chunk sums
-    if ((rc = dev_reserve(ctx, ctx->d_stage, b_sph + b_msph + b_tri + b_mtri))) return rc;
+    if ((rc = ctx->d_reduce.reserve(ctx, (size_t)nb * 7 + 16))) return rc;
+    if ((rc = ctx->d_hist.reserve(ctx, (size_t)256 * n_seg + (size_t)(256 * n_seg + 4095) / 4096 + 1))) return rc; // + chunk sums
+    if ((rc = ctx->d_stage.reserve(ctx, b_sph + b_msph + b_tri + b_mtri))) return rc;
 
     // materials -> (albedo.xyz, param) + type
     std::vector<float4> mats((size_t)n_materials);
@@ -315,42 +319,30 @@ int rrtb_scene_set(rrtb_ctx *ctx, const rrtb_camera *cam, const rrtb_material *m
     ctx->stage_off[1] = b_sph;
     ctx->stage_off[2] = b_sph + b_msph;
     ctx->stage_off[3] = b_sph + b_msph + b_tri;
-    rrtb_sphere *d_sph = (rrtb_sphere *)ctx->d_stage;
-    rrtb_msphere *d_msph = (rrtb_msphere *)(ctx->d_stage + b_sph);
-    rrtb_triangle *d_tri = (rrtb_triangle *)(ctx->d_stage + b_sph + b_msph);
-    rrtb_mtriangle *d_mtri = (rrtb_mtriangle *)(ctx->d_stage + b_sph + b_msph + b_tri);
-    cudaStream_t st = ctx->stream;
-    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
-    if (n_mtriangles > 0) RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_prim_ext, 0, sizeof(float4) * 2 * (size_t)n, st)); // static primitives: no rates
-    RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->d_materials, mats.data(), sizeof(float4) * n_materials, cudaMemcpyHostToDevice, st));
-    RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->d_material_type, mtypes.data(), sizeof(int) * n_materials, cudaMemcpyHostToDevice, st));
-    if (n_spheres)
-        RRTB_CUDA(ctx, cudaMemcpyAsync(d_sph, spheres, sizeof(rrtb_sphere) * (size_t)n_spheres, cudaMemcpyHostToDevice, st));
-    if (n_mspheres)
-        RRTB_CUDA(ctx, cudaMemcpyAsync(d_msph, mspheres, sizeof(rrtb_msphere) * (size_t)n_mspheres, cudaMemcpyHostToDevice, st));
-    if (n_triangles)
-        RRTB_CUDA(ctx, cudaMemcpyAsync(d_tri, triangles, sizeof(rrtb_triangle) * (size_t)n_triangles, cudaMemcpyHostToDevice, st));
-    if (n_mtriangles)
-        RRTB_CUDA(ctx, cudaMemcpyAsync(d_mtri, mtri.data(), sizeof(rrtb_mtriangle) * (size_t)n_mtriangles, cudaMemcpyHostToDevice, st));
-    if ((rc = prepare_and_build(ctx, d_sph, d_msph, d_tri, d_mtri))) return rc;
-    RRTB_CUDA(ctx, cudaEventRecord(ctx->ev1, st));
-    if ((rc = fetch_collapse_state(ctx))) return rc;
-    RRTB_CUDA(ctx, cudaStreamSynchronize(st)); // the host arrays (and mats / mtri above) may go away after this
-    float ms = 0.f;
-    RRTB_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    ctx->seconds_build = ms * 1e-3;
-    if ((rc = check_collapse(ctx))) return rc;
-    ctx->has_scene = true;
-    return RRTB_OK;
+    return build_scene(ctx, [&]() -> int {
+        cudaStream_t st = ctx->stream;
+        unsigned char *stage = ctx->d_stage;
+        if (n_mtriangles > 0) RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_prim_ext, 0, sizeof(float4) * 2 * (size_t)n, st)); // static primitives: no rates
+        RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->d_materials, mats.data(), sizeof(float4) * n_materials, cudaMemcpyHostToDevice, st));
+        RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->d_material_type, mtypes.data(), sizeof(int) * n_materials, cudaMemcpyHostToDevice, st));
+        if (n_spheres)
+            RRTB_CUDA(ctx, cudaMemcpyAsync(stage, spheres, sizeof(rrtb_sphere) * (size_t)n_spheres, cudaMemcpyHostToDevice, st));
+        if (n_mspheres)
+            RRTB_CUDA(ctx, cudaMemcpyAsync(stage + b_sph, mspheres, sizeof(rrtb_msphere) * (size_t)n_mspheres, cudaMemcpyHostToDevice, st));
+        if (n_triangles)
+            RRTB_CUDA(ctx, cudaMemcpyAsync(stage + b_sph + b_msph, triangles, sizeof(rrtb_triangle) * (size_t)n_triangles,
+                                           cudaMemcpyHostToDevice, st));
+        if (n_mtriangles)
+            RRTB_CUDA(ctx, cudaMemcpyAsync(stage + b_sph + b_msph + b_tri, mtri.data(), sizeof(rrtb_mtriangle) * (size_t)n_mtriangles,
+                                           cudaMemcpyHostToDevice, st));
+        return RRTB_OK;
+    });
 }
 
 int rrtb_camera_set(rrtb_ctx *ctx, const rrtb_camera *cam)
 {
     if (!ctx || !cam) return RRTB_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "no scene";
-        return RRTB_ERR_NO_SCENE;
-    }
+    if (int rc = require_scene(ctx, "no scene")) return rc;
     // Two things of the acceleration structure depend on the camera: the boxes of moving primitives span its shutter
     // interval (rrt.cu:169), and the padding of the traversal boxes scales with the largest coordinate a ray can
     // start from.  When either changes, the LBVH is rebuilt from the raw scene kept on the device (no upload).
@@ -360,23 +352,9 @@ int rrtb_camera_set(rrtb_ctx *ctx, const rrtb_camera *cam)
     const bool farther = mag > ctx->build_cam_mag;
     ctx->cam = *cam;
     ctx->motion = use_motion_nodes(ctx->n_mspheres + ctx->n_mtriangles, cam);
-    if (shutter || farther) {
-        RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-        ctx->has_scene = false;
-        RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-        int rc = prepare_and_build(ctx, (const rrtb_sphere *)(ctx->d_stage + ctx->stage_off[0]), (const rrtb_msphere *)(ctx->d_stage + ctx->stage_off[1]),
-                                   (const rrtb_triangle *)(ctx->d_stage + ctx->stage_off[2]), (const rrtb_mtriangle *)(ctx->d_stage + ctx->stage_off[3]));
-        if (rc) return rc;
-        RRTB_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-        if ((rc = fetch_collapse_state(ctx))) return rc;
-        RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        float ms = 0.f;
-        RRTB_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-        ctx->seconds_build = ms * 1e-3;
-        if ((rc = check_collapse(ctx))) return rc;
-        ctx->has_scene = true;
-    }
-    return RRTB_OK;
+    if (!(shutter || farther)) return RRTB_OK;
+    RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
+    return build_scene(ctx, [] { return RRTB_OK; }); // the raw scene is on the device already
 }
 
 // Device -> host copy of a result.  A pinned destination (rrtb_host_alloc, cudaHostRegister) is written by DMA
@@ -393,10 +371,7 @@ static int copy_to_host(rrtb_ctx *ctx, void *dst, const void *d_src, size_t byte
         return RRTB_OK;
     }
     const size_t CH = (size_t)4 << 20;
-    if (!ctx->h_pinned) {
-        RRTB_CUDA(ctx, cudaHostAlloc(&ctx->h_pinned, 2 * CH, cudaHostAllocPortable));
-        ctx->h_pinned_bytes = 2 * CH;
-    }
+    if (int rc = ctx->h_pinned.reserve(ctx, 2 * CH)) return rc;
     if (!ctx->ev_copy[0]) {
         RRTB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_copy[0], cudaEventDisableTiming));
         RRTB_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_copy[1], cudaEventDisableTiming));
@@ -406,41 +381,23 @@ static int copy_to_host(rrtb_ctx *ctx, void *dst, const void *d_src, size_t byte
         if (k < n_chunks) {
             if (k >= 2) RRTB_CUDA(ctx, cudaEventSynchronize(ctx->ev_copy[k & 1])); // (its memcpy below is done too: same thread)
             const size_t len = (k + 1 == n_chunks) ? bytes - k * CH : CH;
-            RRTB_CUDA(ctx, cudaMemcpyAsync((char *)ctx->h_pinned + (k & 1) * CH, (const char *)d_src + k * CH, len,
+            RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + (k & 1) * CH, (const char *)d_src + k * CH, len,
                                            cudaMemcpyDeviceToHost, ctx->stream));
             RRTB_CUDA(ctx, cudaEventRecord(ctx->ev_copy[k & 1], ctx->stream));
         }
         if (k >= 1) {
             const size_t j = k - 1, len = (j + 1 == n_chunks) ? bytes - j * CH : CH;
             RRTB_CUDA(ctx, cudaEventSynchronize(ctx->ev_copy[j & 1]));
-            memcpy((char *)dst + j * CH, (const char *)ctx->h_pinned + (j & 1) * CH, len);
+            memcpy((char *)dst + j * CH, ctx->h_pinned + (j & 1) * CH, len);
         }
     }
-    return RRTB_OK;
-}
-
-// accumulator of the host / frame paths: grow-only, 3*W*H 64-bit sums
-static int reserve_accum(rrtb_ctx *ctx, size_t n)
-{
-    if (ctx->accum_elems >= n) return RRTB_OK;
-    if (ctx->d_accum) cudaFree(ctx->d_accum);
-    if (ctx->d_rgb) cudaFree(ctx->d_rgb);
-    ctx->d_accum = nullptr;
-    ctx->d_rgb = nullptr;
-    ctx->accum_elems = 0;
-    RRTB_CUDA(ctx, cudaMalloc((void **)&ctx->d_accum, n * sizeof(unsigned long long)));
-    RRTB_CUDA(ctx, cudaMalloc((void **)&ctx->d_rgb, n * sizeof(double))); // room for the f64 resolve too
-    ctx->accum_elems = n;
     return RRTB_OK;
 }
 
 static int check_render(rrtb_ctx *ctx, const rrtb_render_params *p)
 {
     if (!ctx || !p) return RRTB_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "render before rrtb_scene_set";
-        return RRTB_ERR_NO_SCENE;
-    }
+    if (int rc = require_scene(ctx, "render before rrtb_scene_set")) return rc;
     if (p->width < 2 || p->height < 2) return invalid(ctx, "image must be at least 2x2 (u = (i+xi)/(W-1), rrt.cu:112)");
     if (p->spp < 1 || p->max_depth < 0) return invalid(ctx, "spp must be >= 1 and max_depth >= 0");
     if (p->spp > rrtb::MAX_SPP) return invalid(ctx, "spp must be <= 2^23 (64-bit fixed-point pixel sums, rrtb_device.cuh fixed_clamp)");
@@ -487,16 +444,15 @@ static int render_host(rrtb_ctx *ctx, const rrtb_render_params *p, void *out_rgb
     if (!out_rgb) return invalid(ctx, "null output buffer");
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)3 * p->width * p->height;
-    if ((rc = reserve_accum(ctx, n))) return rc;
+    if ((rc = ctx->d_accum.reserve(ctx, n)) || (rc = ctx->d_rgb.reserve(ctx, n))) return rc;
     RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_accum, 0, n * sizeof(unsigned long long), ctx->stream));
     rrtb_stats local;
     memset(&local, 0, sizeof(local));
-    rc = launch_render(ctx, p, (uint64_t *)ctx->d_accum, &local);
+    rc = launch_render(ctx, p, ctx->d_accum, &local);
     if (rc) return rc;
     cudaEvent_t e0 = ctx->ev0, e1 = ctx->ev1;
     RRTB_CUDA(ctx, cudaEventRecord(e0, ctx->stream));
-    rc = f64 ? launch_resolve(ctx, (const uint64_t *)ctx->d_accum, (double *)ctx->d_rgb, n)
-             : launch_resolve(ctx, (const uint64_t *)ctx->d_accum, ctx->d_rgb, n);
+    rc = f64 ? launch_resolve(ctx, ctx->d_accum, ctx->d_rgb.get(), n) : launch_resolve(ctx, ctx->d_accum, (float *)ctx->d_rgb.get(), n);
     if (rc) return rc;
     if ((rc = copy_to_host(ctx, out_rgb, ctx->d_rgb, n * (f64 ? sizeof(double) : sizeof(float))))) return rc;
     RRTB_CUDA(ctx, cudaEventRecord(e1, ctx->stream));
@@ -529,7 +485,7 @@ int rrtb_render_aov(rrtb_ctx *ctx, const rrtb_render_params *p, float *albedo3, 
     if (!albedo3 || !normal3 || !depth || !coverage) return invalid(ctx, "null output buffer");
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)p->width * p->height;
-    if ((rc = dev_reserve(ctx, ctx->d_aov, 8 * n))) return rc;
+    if ((rc = ctx->d_aov.reserve(ctx, 8 * n))) return rc;
     rrtb_stats local;
     memset(&local, 0, sizeof(local));
     if ((rc = launch_aov(ctx, p, ctx->d_aov, &local))) return rc;
@@ -550,17 +506,6 @@ struct FrameHandle { // what crosses the process boundary (RRTB_FRAME_HANDLE_BYT
 static_assert(sizeof(FrameHandle) <= RRTB_FRAME_HANDLE_BYTES, "handle blob too small");
 } // namespace
 
-static void frame_drop_mapping(rrtb_ctx *ctx)
-{
-    if (ctx->peer_is_ipc) {
-        if (ctx->peer_frame) cudaIpcCloseMemHandle(ctx->peer_frame);
-        if (ctx->peer_sum) cudaIpcCloseMemHandle(ctx->peer_sum);
-    }
-    ctx->peer_frame = nullptr;
-    ctx->peer_sum = nullptr;
-    ctx->peer_is_ipc = false;
-}
-
 int rrtb_frame_create(rrtb_ctx *ctx, int width, int height, int frame_f64)
 {
     if (!ctx) return RRTB_ERR_INVALID;
@@ -568,16 +513,8 @@ int rrtb_frame_create(rrtb_ctx *ctx, int width, int height, int frame_f64)
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     frame_drop_mapping(ctx);
     const size_t n = (size_t)3 * width * height;
-    if (ctx->frame_elems < n) { // cudaMalloc'ed directly (not sub-allocated): the pair must be exportable through CUDA IPC
-        if (ctx->d_frame) cudaFree(ctx->d_frame);
-        if (ctx->d_sum) cudaFree(ctx->d_sum);
-        ctx->d_frame = nullptr;
-        ctx->d_sum = nullptr;
-        ctx->frame_elems = 0;
-        RRTB_CUDA(ctx, cudaMalloc(&ctx->d_frame, n * sizeof(double)));
-        RRTB_CUDA(ctx, cudaMalloc((void **)&ctx->d_sum, n * sizeof(unsigned long long)));
-        ctx->frame_elems = n;
-    }
+    int rc;
+    if ((rc = ctx->d_frame.reserve(ctx, n)) || (rc = ctx->d_sum.reserve(ctx, n))) return rc;
     ctx->frame_w = width;
     ctx->frame_h = height;
     ctx->frame_f64 = frame_f64 ? 1 : 0;
@@ -621,7 +558,7 @@ int rrtb_frame_import(rrtb_ctx *ctx, const void *handle)
         ctx->peer_frame = nullptr;
         return cuda_fail(ctx, e, "cudaIpcOpenMemHandle(sum)", __FILE__, __LINE__);
     }
-    ctx->peer_sum = (unsigned long long *)sum;
+    ctx->peer_sum = (uint64_t *)sum;
     ctx->peer_is_ipc = true;
     ctx->frame_w = h.width;
     ctx->frame_h = h.height;
@@ -666,17 +603,17 @@ static int enqueue_shard(rrtb_ctx *ctx, const rrtb_render_params *p)
     int rc = check_render(ctx, p);
     if (rc) return rc;
     void *frame = ctx->peer_frame ? ctx->peer_frame : ctx->d_frame;
-    unsigned long long *sum = ctx->peer_frame ? ctx->peer_sum : ctx->d_sum;
+    uint64_t *sum = ctx->peer_frame ? ctx->peer_sum : ctx->d_sum;
     if (!frame) return invalid(ctx, "no frame: call rrtb_frame_create (owner) or rrtb_frame_import / rrtb_frame_attach first");
     if (p->width != ctx->frame_w || p->height != ctx->frame_h) return invalid(ctx, "render size differs from the frame's");
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)3 * p->width * p->height;
-    if ((rc = reserve_accum(ctx, n))) return rc;
+    if ((rc = ctx->d_accum.reserve(ctx, n))) return rc;
     RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_accum, 0, n * sizeof(unsigned long long), ctx->stream));
-    if ((rc = launch_render(ctx, p, (uint64_t *)ctx->d_accum, nullptr, true))) return rc;
+    if ((rc = launch_render(ctx, p, ctx->d_accum, nullptr, true))) return rc;
     RRTB_CUDA(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
-    if (p->shard_mode == RRTB_SHARD_TILES) rc = launch_resolve_tiles(ctx, (const uint64_t *)ctx->d_accum, frame, p, ctx->frame_f64 != 0);
-    else rc = launch_accumulate_atomic(ctx, (uint64_t *)sum, (const uint64_t *)ctx->d_accum, n);
+    if (p->shard_mode == RRTB_SHARD_TILES) rc = launch_resolve_tiles(ctx, ctx->d_accum, frame, p, ctx->frame_f64 != 0);
+    else rc = launch_accumulate_atomic(ctx, sum, ctx->d_accum, n);
     if (rc) return rc;
     RRTB_CUDA(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
     return RRTB_OK;
@@ -712,8 +649,8 @@ int rrtb_frame_download(rrtb_ctx *ctx, int shard_mode, void *out_rgb)
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)3 * ctx->frame_w * ctx->frame_h;
     if (shard_mode == RRTB_SHARD_SAMPLES) { // the ranks added their partial sums: resolve them, then clear for the next frame
-        int rc = ctx->frame_f64 ? launch_resolve(ctx, (const uint64_t *)ctx->d_sum, (double *)ctx->d_frame, n)
-                                : launch_resolve(ctx, (const uint64_t *)ctx->d_sum, (float *)ctx->d_frame, n);
+        int rc = ctx->frame_f64 ? launch_resolve(ctx, ctx->d_sum, ctx->d_frame.get(), n)
+                                : launch_resolve(ctx, ctx->d_sum, (float *)ctx->d_frame.get(), n);
         if (rc) return rc;
         RRTB_CUDA(ctx, cudaMemsetAsync(ctx->d_sum, 0, n * sizeof(unsigned long long), ctx->stream));
     }
@@ -797,39 +734,25 @@ int rrtb_probe_issue_rate(rrtb_ctx *ctx, double *ffma_lane_instr_per_s, double *
 
 // ---- test hooks: one body per hook, for the float (real = float) and the double integrator --------------------
 namespace {
-struct DevBuf {
-    void *p = nullptr;
-    ~DevBuf()
-    {
-        if (p) cudaFree(p);
-    }
-};
-
-#define HOOK_ALLOC(buf, bytes) RRTB_CUDA(ctx, cudaMalloc(&(buf).p, (bytes) ? (bytes) : 1))
-
 template <typename real>
 int trace_hook(rrtb_ctx *ctx, const real *rays7, int n, real t_min, int mode, int32_t *id, real *t, real *rec7)
 {
     if (!ctx || !rays7 || !id || !t || n < 0) return RRTB_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "trace before rrtb_scene_set";
-        return RRTB_ERR_NO_SCENE;
-    }
+    int rc;
+    if ((rc = require_scene(ctx, "trace before rrtb_scene_set"))) return rc;
     if (!(t_min >= (real)0)) return invalid(ctx, "t_min must be >= 0 (the reference uses 0.001, rrt.cu:49)");
     if (n == 0) return RRTB_OK;
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-    DevBuf dr, di, dt, drec;
-    HOOK_ALLOC(dr, sizeof(real) * 7 * (size_t)n);
-    HOOK_ALLOC(di, sizeof(int) * (size_t)n);
-    HOOK_ALLOC(dt, sizeof(real) * (size_t)n);
-    if (rec7) HOOK_ALLOC(drec, sizeof(real) * 7 * (size_t)n);
-    RRTB_CUDA(ctx, cudaMemcpyAsync(dr.p, rays7, sizeof(real) * 7 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = launch_trace(ctx, (const real *)dr.p, n, t_min, mode ? 1 : 0, (int32_t *)di.p, (real *)dt.p,
-                          rec7 ? (real *)drec.p : nullptr);
-    if (rc) return rc;
-    RRTB_CUDA(ctx, cudaMemcpyAsync(id, di.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    RRTB_CUDA(ctx, cudaMemcpyAsync(t, dt.p, sizeof(real) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    if (rec7) RRTB_CUDA(ctx, cudaMemcpyAsync(rec7, drec.p, sizeof(real) * 7 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    DeviceArray<real> dr, dt, drec;
+    DeviceArray<int32_t> di;
+    if ((rc = dr.reserve(ctx, 7 * (size_t)n)) || (rc = di.reserve(ctx, n)) || (rc = dt.reserve(ctx, n)) ||
+        (rec7 && (rc = drec.reserve(ctx, 7 * (size_t)n))))
+        return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(dr, rays7, sizeof(real) * 7 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = launch_trace<real>(ctx, dr, n, t_min, mode ? 1 : 0, di, dt, drec))) return rc; // drec: null without rec7
+    RRTB_CUDA(ctx, cudaMemcpyAsync(id, di, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    RRTB_CUDA(ctx, cudaMemcpyAsync(t, dt, sizeof(real) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (rec7) RRTB_CUDA(ctx, cudaMemcpyAsync(rec7, drec, sizeof(real) * 7 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return RRTB_OK;
 }
@@ -838,19 +761,16 @@ template <typename real>
 int camera_rays_hook(rrtb_ctx *ctx, const rrtb_render_params *p, const int32_t *pix, int n, int sample, real *rays7)
 {
     if (!ctx || !p || !pix || !rays7 || n < 0) return RRTB_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "camera rays before rrtb_scene_set";
-        return RRTB_ERR_NO_SCENE;
-    }
+    int rc;
+    if ((rc = require_scene(ctx, "camera rays before rrtb_scene_set"))) return rc;
     if (n == 0) return RRTB_OK;
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-    DevBuf dp, dr;
-    HOOK_ALLOC(dp, sizeof(int) * (size_t)n);
-    HOOK_ALLOC(dr, sizeof(real) * 7 * (size_t)n);
-    RRTB_CUDA(ctx, cudaMemcpyAsync(dp.p, pix, sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = launch_camera_rays(ctx, p, (const int32_t *)dp.p, n, sample, (real *)dr.p);
-    if (rc) return rc;
-    RRTB_CUDA(ctx, cudaMemcpyAsync(rays7, dr.p, sizeof(real) * 7 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    DeviceArray<int32_t> dp;
+    DeviceArray<real> dr;
+    if ((rc = dp.reserve(ctx, n)) || (rc = dr.reserve(ctx, 7 * (size_t)n))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(dp, pix, sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = launch_camera_rays<real>(ctx, p, dp, n, sample, dr))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(rays7, dr, sizeof(real) * 7 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return RRTB_OK;
 }
@@ -859,25 +779,22 @@ template <typename real>
 int scatter_hook(rrtb_ctx *ctx, const real *in16, const uint32_t *rnd4, int n, real *out8)
 {
     if (!ctx || !in16 || !rnd4 || !out8 || n < 0) return RRTB_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "scatter before rrtb_scene_set";
-        return RRTB_ERR_NO_SCENE;
-    }
+    int rc;
+    if ((rc = require_scene(ctx, "scatter before rrtb_scene_set"))) return rc;
     if (n == 0) return RRTB_OK;
     for (int i = 0; i < n; ++i) { // the kernel indexes the material arrays with in16[14]
         const real m = in16[16 * (size_t)i + 14];
         if (!(m >= (real)0 && m < (real)ctx->n_materials)) return invalid(ctx, "scatter: material index out of range");
     }
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-    DevBuf di, dr, dout;
-    HOOK_ALLOC(di, sizeof(real) * 16 * (size_t)n);
-    HOOK_ALLOC(dr, 16 * (size_t)n);
-    HOOK_ALLOC(dout, sizeof(real) * 8 * (size_t)n);
-    RRTB_CUDA(ctx, cudaMemcpyAsync(di.p, in16, sizeof(real) * 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    RRTB_CUDA(ctx, cudaMemcpyAsync(dr.p, rnd4, 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = launch_scatter(ctx, (const real *)di.p, (const uint32_t *)dr.p, n, (real *)dout.p);
-    if (rc) return rc;
-    RRTB_CUDA(ctx, cudaMemcpyAsync(out8, dout.p, sizeof(real) * 8 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    DeviceArray<real> di, dout;
+    DeviceArray<uint32_t> dr;
+    if ((rc = di.reserve(ctx, 16 * (size_t)n)) || (rc = dr.reserve(ctx, 4 * (size_t)n)) || (rc = dout.reserve(ctx, 8 * (size_t)n)))
+        return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(di, in16, sizeof(real) * 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    RRTB_CUDA(ctx, cudaMemcpyAsync(dr, rnd4, 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = launch_scatter<real>(ctx, di, dr, n, dout))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(out8, dout, sizeof(real) * 8 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return RRTB_OK;
 }
@@ -932,21 +849,20 @@ int rrtb_bvh_download(rrtb_ctx *ctx, uint32_t *morton, uint32_t *perm, int32_t *
     if (!ctx->has_scene) return RRTB_ERR_NO_SCENE;
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)ctx->n_prims, ni = n > 0 ? n - 1 : 0;
-    if (morton) RRTB_CUDA(ctx, cudaMemcpy(morton, ctx->d_morton, 4 * n, cudaMemcpyDeviceToHost));
+    int rc;
+    if (morton && (rc = read_back(ctx, morton, ctx->d_morton, 4 * n))) return rc;
     if (perm) {
         std::vector<uint64_t> keys(n);
-        RRTB_CUDA(ctx, cudaMemcpy(keys.data(), ctx->d_keys, 8 * n, cudaMemcpyDeviceToHost));
+        if ((rc = read_back(ctx, keys.data(), ctx->d_keys, 8 * n))) return rc;
         for (size_t k = 0; k < n; ++k) perm[k] = (uint32_t)keys[k];
     }
-    if (left && ni) RRTB_CUDA(ctx, cudaMemcpy(left, ctx->d_left, 4 * ni, cudaMemcpyDeviceToHost));
-    if (right && ni) RRTB_CUDA(ctx, cudaMemcpy(right, ctx->d_right, 4 * ni, cudaMemcpyDeviceToHost));
-    if (parent) RRTB_CUDA(ctx, cudaMemcpy(parent, ctx->d_parent, 4 * (2 * n - 1), cudaMemcpyDeviceToHost));
+    if (left && ni && (rc = read_back(ctx, left, ctx->d_left, 4 * ni))) return rc;
+    if (right && ni && (rc = read_back(ctx, right, ctx->d_right, 4 * ni))) return rc;
+    if (parent && (rc = read_back(ctx, parent, ctx->d_parent, 4 * (2 * n - 1)))) return rc;
     if (node_box && ni) {
-        int rc = refit_canonical(ctx);
-        if (rc) return rc;
-        RRTB_CUDA(ctx, cudaMemcpy(node_box, ctx->d_node_box, 4 * 6 * ni, cudaMemcpyDeviceToHost));
+        if ((rc = refit_canonical(ctx)) || (rc = read_back(ctx, node_box, ctx->d_node_box, 4 * 6 * ni))) return rc;
     }
-    if (prim_box) RRTB_CUDA(ctx, cudaMemcpy(prim_box, ctx->d_prim_box, 4 * 6 * n, cudaMemcpyDeviceToHost));
+    if (prim_box && (rc = read_back(ctx, prim_box, ctx->d_prim_box, 4 * 6 * n))) return rc;
     return RRTB_OK;
 }
 
@@ -956,8 +872,7 @@ int rrtb_wide_size(rrtb_ctx *ctx, int32_t *n_nodes, int32_t *width)
     if (width) *width = RRTB_WIDTH;
     if (!ctx->has_scene) return RRTB_ERR_NO_SCENE;
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-    RRTB_CUDA(ctx, cudaMemcpy(n_nodes, ctx->d_collapse, sizeof(int), cudaMemcpyDeviceToHost)); // CollapseState::n_alloc
-    return RRTB_OK;
+    return read_back(ctx, n_nodes, ctx->d_collapse, sizeof(int)); // CollapseState::n_alloc
 }
 
 // IEEE half precision -> float (the half extents of the traversal nodes, rrtb_device.cuh "Traversal node")
@@ -989,7 +904,7 @@ int rrtb_wide_download(rrtb_ctx *ctx, float *nodes, int32_t max_nodes)
     // both ends of the shutter ("Motion node"); hand them back decoded, the motion node as the UNION of its two boxes
     const int words = ctx->motion ? 40 : 24;
     std::vector<uint32_t> raw((size_t)words * n_nodes);
-    RRTB_CUDA(ctx, cudaMemcpy(raw.data(), ctx->d_wnodes, sizeof(uint32_t) * raw.size(), cudaMemcpyDeviceToHost));
+    if ((rc = read_back(ctx, raw.data(), ctx->d_wnodes, sizeof(uint32_t) * raw.size()))) return rc;
     auto f = [](uint32_t b) {
         float x;
         memcpy(&x, &b, 4);
@@ -1031,8 +946,7 @@ int rrtb_wide_download_raw(rrtb_ctx *ctx, uint32_t *words, int32_t max_nodes, in
     if (n_nodes > max_nodes) return invalid(ctx, "wide-node buffer too small");
     const int wpn = ctx->motion ? 4 * RRTB_MOTION_NODE_F4 : 4 * RRTB_NODE_F4;
     if (words_per_node) *words_per_node = wpn;
-    RRTB_CUDA(ctx, cudaMemcpy(words, ctx->d_wnodes, sizeof(uint32_t) * (size_t)wpn * n_nodes, cudaMemcpyDeviceToHost));
-    return RRTB_OK;
+    return read_back(ctx, words, ctx->d_wnodes, sizeof(uint32_t) * (size_t)wpn * n_nodes);
 }
 
 int rrtb_philox(rrtb_ctx *ctx, const uint32_t *ctr4, int n, uint32_t key0, uint32_t key1, uint32_t *out4)
@@ -1040,13 +954,12 @@ int rrtb_philox(rrtb_ctx *ctx, const uint32_t *ctr4, int n, uint32_t key0, uint3
     if (!ctx || !ctr4 || !out4 || n < 0) return RRTB_ERR_INVALID;
     if (n == 0) return RRTB_OK;
     RRTB_CUDA(ctx, cudaSetDevice(ctx->device));
-    DevBuf dc, dout;
-    HOOK_ALLOC(dc, 16 * (size_t)n);
-    HOOK_ALLOC(dout, 16 * (size_t)n);
-    RRTB_CUDA(ctx, cudaMemcpyAsync(dc.p, ctr4, 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = launch_philox(ctx, (const uint32_t *)dc.p, n, key0, key1, (uint32_t *)dout.p);
-    if (rc) return rc;
-    RRTB_CUDA(ctx, cudaMemcpyAsync(out4, dout.p, 16 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    DeviceArray<uint32_t> dc, dout;
+    int rc;
+    if ((rc = dc.reserve(ctx, 4 * (size_t)n)) || (rc = dout.reserve(ctx, 4 * (size_t)n))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(dc, ctr4, 16 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = launch_philox(ctx, dc, n, key0, key1, dout))) return rc;
+    RRTB_CUDA(ctx, cudaMemcpyAsync(out4, dout, 16 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     RRTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return RRTB_OK;
 }

@@ -1225,19 +1225,22 @@ __global__ void __launch_bounds__(TPB) k_flatten_leaves(const uint64_t *__restri
     }
 }
 
-// exposed to rrtb_api.cu (scene upload): raw struct arrays are staged by the caller
-int prepare_and_build(rrtb_ctx *ctx, const rrtb_sphere *d_sph, const rrtb_msphere *d_msph, const rrtb_triangle *d_tri,
-                      const rrtb_mtriangle *d_mtri)
+// exposed to rrtb_api.cu (scene upload and rebuild): the raw struct arrays are staged in d_stage by the caller
+int prepare_and_build(rrtb_ctx *ctx)
 {
     const int n = ctx->n_prims;
     const int ns = ctx->n_spheres, nms = ctx->n_mspheres, nt = ctx->n_triangles;
     const int nb = (n + TPB - 1) / TPB;
     cudaStream_t st = ctx->stream;
     BuildConsts *bc = (BuildConsts *)(ctx->d_reduce + (size_t)nb * 7);
+    const rrtb_sphere *d_sph = (const rrtb_sphere *)(ctx->d_stage + ctx->stage_off[0]);
+    const rrtb_msphere *d_msph = (const rrtb_msphere *)(ctx->d_stage + ctx->stage_off[1]);
+    const rrtb_triangle *d_tri = (const rrtb_triangle *)(ctx->d_stage + ctx->stage_off[2]);
+    const rrtb_mtriangle *d_mtri = (const rrtb_mtriangle *)(ctx->d_stage + ctx->stage_off[3]);
 
     k_prepare<<<nb, TPB, 0, st>>>(d_sph, ns, d_msph, nms, d_tri, nt, d_mtri, ctx->n_mtriangles, ctx->cam.time0, ctx->cam.time1, ctx->d_prim,
-                                  ctx->n_mtriangles > 0 ? ctx->d_prim_ext : nullptr, ctx->d_prim_info, ctx->d_prim_box,
-                                  ctx->motion ? ctx->d_prim_box01 : nullptr, ctx->d_reduce);
+                                  ctx->n_mtriangles > 0 ? ctx->d_prim_ext.get() : nullptr, ctx->d_prim_info, ctx->d_prim_box,
+                                  ctx->motion ? ctx->d_prim_box01.get() : nullptr, ctx->d_reduce);
     float cam_mag = 0.f;
     for (int k = 0; k < 3; ++k) cam_mag = fmaxf(cam_mag, fabsf(ctx->cam.origin[k]) + ctx->cam.lens_radius);
     ctx->build_cam_mag = cam_mag;
@@ -1315,15 +1318,15 @@ int prepare_and_build(rrtb_ctx *ctx, const rrtb_sphere *d_sph, const rrtb_mspher
         int m1 = -1;
         RRTB_CUDA(ctx, cudaMemcpyAsync(ctx->d_parent, &m1, sizeof(int), cudaMemcpyHostToDevice, st));
     }
-    CollapseState *cs = (CollapseState *)ctx->d_collapse;
+    CollapseState *cs = (CollapseState *)ctx->d_collapse.get();
     k_collapse_init<<<nb, TPB, 0, st>>>(ctx->d_wq, n, cs);
     const int want_blocks = (max(n - 1, 1) + TPB - 1) / TPB;
     k_collapse4<<<min(want_blocks, ctx->sm_count * 4), TPB, 0, st>>>(ctx->d_keys, n, ns, nms, nt, t_left, t_right,
-                                                                     ctx->d_prim_box, t_node_box, ctx->motion ? ctx->d_prim_box01 : nullptr,
-                                                                     ctx->motion ? ctx->d_node_box01 : nullptr, bc, ctx->d_wq, cs, ctx->d_wnodes);
+                                                                     ctx->d_prim_box, t_node_box, ctx->motion ? ctx->d_prim_box01.get() : nullptr,
+                                                                     ctx->motion ? ctx->d_node_box01.get() : nullptr, bc, ctx->d_wq, cs, ctx->d_wnodes);
     const bool has_ext = ctx->n_mtriangles > 0;
-    k_flatten_leaves<<<nb, TPB, 0, st>>>(ctx->d_keys, n, ctx->d_prim, ctx->d_prim_info, has_ext ? ctx->d_prim_ext : nullptr, ctx->d_leaves,
-                                         ctx->d_leaf_info, has_ext ? ctx->d_leaf_ext : nullptr);
+    k_flatten_leaves<<<nb, TPB, 0, st>>>(ctx->d_keys, n, ctx->d_prim, ctx->d_prim_info, has_ext ? ctx->d_prim_ext.get() : nullptr, ctx->d_leaves,
+                                         ctx->d_leaf_info, has_ext ? ctx->d_leaf_ext.get() : nullptr);
     RRTB_CUDA(ctx, cudaGetLastError());
     return RRTB_OK;
 }
@@ -1341,21 +1344,6 @@ int refit_canonical(rrtb_ctx *ctx)
     RRTB_CUDA(ctx, cudaStreamSynchronize(st));
     ctx->canonical_boxes = true;
     return RRTB_OK;
-}
-
-void free_scene(rrtb_ctx *ctx)
-{
-    auto F = [](auto *&p) {
-        if (p) cudaFree(p);
-        p = nullptr;
-    };
-    F(ctx->d_prim); F(ctx->d_prim_info); F(ctx->d_materials); F(ctx->d_material_type); F(ctx->d_prim_box);
-    F(ctx->d_morton); F(ctx->d_keys); F(ctx->d_keys_tmp); F(ctx->d_left); F(ctx->d_right); F(ctx->d_parent);
-    F(ctx->d_node_box); F(ctx->d_visit); F(ctx->d_wnodes); F(ctx->d_wq); F(ctx->d_collapse); F(ctx->d_leaves);
-    F(ctx->d_leaf_info); F(ctx->d_prim_ext); F(ctx->d_leaf_ext); F(ctx->d_prim_box01); F(ctx->d_node_box01); F(ctx->d_range); F(ctx->d_left2); F(ctx->d_right2); F(ctx->d_parent2);
-    F(ctx->d_node_box2); F(ctx->d_sah_roots); F(ctx->d_reduce); F(ctx->d_hist); F(ctx->d_stage);
-    ctx->capacity.clear();
-    ctx->has_scene = false;
 }
 
 } // namespace rrtb

@@ -4,13 +4,69 @@
 #include <stdint.h>
 
 #include <string>
-#include <unordered_map>
 #include <vector>
 
 #include "../../include/rrtb.h"
 #include "rrtb_device.cuh"
 
+namespace rrtb {
+
+// error helper: records the reference-style message (rrt.cu:31-40) and returns RRTB_ERR_CUDA
+int cuda_fail(rrtb_ctx *ctx, cudaError_t e, const char *expr, const char *file, int line);
+
+#define RRTB_CUDA(ctx, expr)                                                              \
+    do {                                                                                  \
+        cudaError_t _e = (expr);                                                          \
+        if (_e != cudaSuccess) return ::rrtb::cuda_fail((ctx), _e, #expr, __FILE__, __LINE__); \
+    } while (0)
+
+// One owning allocation of Ts: device memory (cudaMalloc), or pinned host memory (cudaHostAlloc) when PINNED.  Grow-only:
+// reserve() reallocates, without keeping the contents, only when the request exceeds the count already held, so a frame
+// loop that re-sends its scene pays no cudaMalloc / cudaFree.  Converts to T* for kernel arguments and pointer
+// arithmetic; get() for a cast to another pointer type.
+template <typename T, bool PINNED>
+class CudaArray {
+  public:
+    CudaArray() = default;
+    CudaArray(const CudaArray &) = delete;
+    CudaArray &operator=(const CudaArray &) = delete;
+    ~CudaArray() { release(); }
+    operator T *() const { return p_; }
+    T *get() const { return p_; }
+
+    int reserve(rrtb_ctx *ctx, size_t count)
+    {
+        if (count == 0) count = 1;
+        if (count <= cap_) return RRTB_OK;
+        release();
+        void *p = nullptr;
+        RRTB_CUDA(ctx, PINNED ? cudaHostAlloc(&p, count * sizeof(T), cudaHostAllocPortable) : cudaMalloc(&p, count * sizeof(T)));
+        p_ = (T *)p;
+        cap_ = count;
+        return RRTB_OK;
+    }
+
+  private:
+    void release()
+    {
+        if (p_ && PINNED) cudaFreeHost(p_);
+        else if (p_) cudaFree(p_);
+        p_ = nullptr;
+        cap_ = 0;
+    }
+    T *p_ = nullptr;
+    size_t cap_ = 0;
+};
+template <typename T> using DeviceArray = CudaArray<T, false>;
+template <typename T> using PinnedArray = CudaArray<T, true>;
+
+} // namespace rrtb
+
+// A new per-context buffer is one DeviceArray member: it is reserved where it is used and freed with the context.
 struct rrtb_ctx {
+    template <typename T> using DeviceArray = rrtb::DeviceArray<T>;
+    template <typename T> using PinnedArray = rrtb::PinnedArray<T>;
+
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr, ev3 = nullptr, ev_copy[2] = {nullptr, nullptr};
@@ -31,83 +87,74 @@ struct rrtb_ctx {
     double seconds_build = 0.0;
 
     // device: canonical primitive arrays (object-id order)
-    float4 *d_prim = nullptr;       // [3*n] leaf records in object-id order (== flat_leaves)
-    int2 *d_prim_info = nullptr;    // [n]   (object id, material)
-    float4 *d_materials = nullptr;  // [nm]
-    int *d_material_type = nullptr; // [nm]
+    DeviceArray<float4> d_prim;       // [3*n] leaf records in object-id order (== flat_leaves)
+    DeviceArray<int2> d_prim_info;    // [n]   (object id, material)
+    DeviceArray<float4> d_materials;  // [nm]
+    DeviceArray<int> d_material_type; // [nm]
     // device: canonical LBVH arrays (rrtb_bvh_download)
-    float *d_prim_box = nullptr;    // [6n]
-    uint32_t *d_morton = nullptr;   // [n]
-    uint64_t *d_keys = nullptr;     // [n] sorted (code << 32 | id)
-    uint64_t *d_keys_tmp = nullptr; // [n]
-    int *d_left = nullptr, *d_right = nullptr; // [n-1]
-    int *d_parent = nullptr;        // [2n-1]
-    float *d_node_box = nullptr;    // [6(n-1)]
-    bool canonical_boxes = false;   // d_node_box holds the refit of the canonical tree (else: refit_canonical on demand)
+    DeviceArray<float> d_prim_box;    // [6n]
+    DeviceArray<uint32_t> d_morton;   // [n]
+    DeviceArray<uint64_t> d_keys;     // [n] sorted (code << 32 | id)
+    DeviceArray<uint64_t> d_keys_tmp; // [n]
+    DeviceArray<int> d_left, d_right; // [n-1]
+    DeviceArray<int> d_parent;        // [2n-1]
+    DeviceArray<float> d_node_box;    // [6(n-1)]
+    bool canonical_boxes = false;     // d_node_box holds the refit of the canonical tree (else: refit_canonical on demand)
     // scenes with motion (moving primitives and an open shutter): boxes at the two ends of the shutter, for the
     // interpolating traversal nodes (rrtb_device.cuh "Motion node")
     bool motion = false;
-    float *d_prim_box01 = nullptr;  // [12n]
-    float *d_node_box01 = nullptr;  // [12(n-1)]
-    int *d_visit = nullptr;         // [n-1]
+    DeviceArray<float> d_prim_box01;  // [12n]
+    DeviceArray<float> d_node_box01;  // [12(n-1)]
+    DeviceArray<int> d_visit;         // [n-1]
     // SAH-rebuilt copy of the topology, for the traversal tree only (rrtb_bvh.cu k_sah_rebuild)
-    int2 *d_range = nullptr;        // [n-1] sorted positions covered by each canonical internal node
-    int *d_left2 = nullptr, *d_right2 = nullptr; // [n-1]
-    int *d_parent2 = nullptr;       // [2n-1]
-    float *d_node_box2 = nullptr;   // [6(n-1)]
-    int *d_sah_roots = nullptr;     // [n] roots of the subtrees to rebuild
+    DeviceArray<int2> d_range;        // [n-1] sorted positions covered by each canonical internal node
+    DeviceArray<int> d_left2, d_right2; // [n-1]
+    DeviceArray<int> d_parent2;       // [2n-1]
+    DeviceArray<float> d_node_box2;   // [6(n-1)]
+    DeviceArray<int> d_sah_roots;     // [n] roots of the subtrees to rebuild
     // device: traversal structures
-    float4 *d_wnodes = nullptr;     // [8*max(n-1,1)] 4-wide traversal nodes (rrtb_bvh.cu k_collapse4)
-    int *d_wq = nullptr;            // [n] collapse work list: binary node that roots wide node i
-    int *d_collapse = nullptr;      // CollapseState (wide-node count, ticket, leaves emitted)
-    float4 *d_leaves = nullptr;     // [3n] leaf order
-    int2 *d_leaf_info = nullptr;    // [n]
-    float4 *d_prim_ext = nullptr;   // [2n] edge rates of moving triangles, object-id order (allocated when the scene has any)
-    float4 *d_leaf_ext = nullptr;   // [2n] the same in leaf order
+    DeviceArray<float4> d_wnodes;     // [8*max(n-1,1)] 4-wide traversal nodes (rrtb_bvh.cu k_collapse4)
+    DeviceArray<int> d_wq;            // [n] collapse work list: binary node that roots wide node i
+    DeviceArray<int> d_collapse;      // CollapseState (wide-node count, ticket, leaves emitted)
+    DeviceArray<float4> d_leaves;     // [3n] leaf order
+    DeviceArray<int2> d_leaf_info;    // [n]
+    DeviceArray<float4> d_prim_ext;   // [2n] edge rates of moving triangles, object-id order (allocated when the scene has any)
+    DeviceArray<float4> d_leaf_ext;   // [2n] the same in leaf order
     // scratch
-    float *d_reduce = nullptr;      // block partials + build constants
-    unsigned int *d_hist = nullptr; // radix histograms
-    size_t hist_elems = 0;
-    unsigned long long *d_counters = nullptr; // [0] work queue head, [1] ray counter
-    unsigned long long *d_accum = nullptr;    // host-path accumulator (3*W*H)
-    float *d_rgb = nullptr;                   // host-path float framebuffer
-    size_t accum_elems = 0;
-    float *d_aov = nullptr;                   // rrtb_render_aov's output, 8*W*H floats (grow-only)
-    unsigned char *d_stage = nullptr;         // raw scene structs of the last upload (input of k_prepare; kept for rebuilds)
-    size_t stage_off[4] = {0, 0, 0, 0};       // byte offsets of the sphere / msphere / triangle / mtriangle arrays in d_stage
-    float build_cam_mag = 0.f;                // camera magnitude the traversal-box padding was computed with
-    rrtb_render_params pending{};             // the render enqueued by launch_render, for finish_render
+    DeviceArray<float> d_reduce;      // block partials + build constants
+    DeviceArray<unsigned int> d_hist; // radix histograms
+    DeviceArray<unsigned long long> d_counters; // [0] work queue head, [1] ray counter
+    DeviceArray<uint64_t> d_accum;    // host-path accumulator (3*W*H)
+    DeviceArray<double> d_rgb;        // host-path framebuffer, 3*W*H doubles' worth of room (float or double resolve)
+    DeviceArray<float> d_aov;         // rrtb_render_aov's output, 8*W*H floats
+    DeviceArray<unsigned char> d_stage; // raw scene structs of the last upload (input of k_prepare; kept for rebuilds)
+    size_t stage_off[4] = {0, 0, 0, 0}; // byte offsets of the sphere / msphere / triangle / mtriangle arrays in d_stage
+    float build_cam_mag = 0.f;        // camera magnitude the traversal-box padding was computed with
+    rrtb_render_params pending{};     // the render enqueued by launch_render, for finish_render
     int pending_launches = 0;
     // multi-GPU frame (SURVEY 8e): the owner (rank 0) holds the float/double frame every rank's resolve epilogue stores its
-    // tiles into, and the 64-bit sum buffer sample shards add into; other ranks hold peer mappings of both
-    void *d_frame = nullptr;                  // owner: 3*W*H doubles' worth of room (float or double frame)
-    unsigned long long *d_sum = nullptr;      // owner: 3*W*H fixed-point sums of a sample-sharded frame
-    size_t frame_elems = 0;                   // 3*W*H the frame was sized for
+    // tiles into, and the 64-bit sum buffer sample shards add into; other ranks hold peer mappings of both.  The two are
+    // cudaMalloc'ed one each (not sub-allocated): CUDA IPC exports them.
+    DeviceArray<double> d_frame;      // owner: 3*W*H doubles' worth of room (float or double frame)
+    DeviceArray<uint64_t> d_sum;      // owner: 3*W*H fixed-point sums of a sample-sharded frame
     int frame_w = 0, frame_h = 0, frame_f64 = 0;
-    void *peer_frame = nullptr;               // non-owner: the owner's d_frame / d_sum (IPC mapping or same-process pointer)
-    unsigned long long *peer_sum = nullptr;
+    void *peer_frame = nullptr;       // non-owner: the owner's d_frame / d_sum (IPC mapping or same-process pointer)
+    uint64_t *peer_sum = nullptr;
     bool peer_is_ipc = false;
-    void *h_pinned = nullptr;                 // pinned staging for device->host copies into pageable user buffers
-    size_t h_pinned_bytes = 0;
-    int *h_state = nullptr;                   // pinned: CollapseState read back behind every build
-    // Device buffers are grow-only: rrtb_scene_set re-uses them when the next scene fits (a frame loop that re-sends
-    // its scene pays no cudaMalloc / cudaFree).  Capacity in bytes, keyed by the address of the pointer member.
-    std::unordered_map<const void *, size_t> capacity;
+    PinnedArray<unsigned char> h_pinned; // staging for device->host copies into pageable user buffers
+    PinnedArray<int> h_state;         // CollapseState read back behind every build
+
+    ~rrtb_ctx(); // closes the peer mappings, destroys the events and the stream; the arrays free themselves
 };
 
 namespace rrtb {
 
-// error helper: records the reference-style message (rrt.cu:31-40) and returns RRTB_ERR_CUDA
-int cuda_fail(rrtb_ctx *ctx, cudaError_t e, const char *expr, const char *file, int line);
-
-#define RRTB_CUDA(ctx, expr)                                                              \
-    do {                                                                                  \
-        cudaError_t _e = (expr);                                                          \
-        if (_e != cudaSuccess) return ::rrtb::cuda_fail((ctx), _e, #expr, __FILE__, __LINE__); \
-    } while (0)
+// rrtb_api.cu
+// device -> host copy on the context's stream, behind the kernels that wrote d_src; synchronises
+int read_back(rrtb_ctx *ctx, void *dst, const void *d_src, size_t bytes);
 
 // rrtb_bvh.cu
-void free_scene(rrtb_ctx *ctx);
+int prepare_and_build(rrtb_ctx *ctx); // from the raw scene in d_stage
 int refit_canonical(rrtb_ctx *ctx);
 
 // rrtb_render.cu

@@ -475,7 +475,7 @@ __global__ void __launch_bounds__(256) k_probe(float *out, int iters, float seed
 int launch_probe(rrtb_ctx *ctx, int mix, double *lane_instr_per_s)
 {
     const int iters = 4096, blocks = ctx->sm_count * 8;
-    float *d_out = (float *)ctx->d_counters;
+    float *d_out = (float *)ctx->d_counters.get();
     float ms = 0.f;
     for (int rep = 0; rep < 3; ++rep) { // last repetition is the measurement
         RRTB_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
@@ -563,19 +563,25 @@ static int grid_size(const rrtb_ctx *ctx, size_t n)
     return (int)(blocks > cap ? cap : (blocks < 1 ? 1 : blocks));
 }
 
+// Blocks of RENDER_TPB threads for a persistent kernel: one wave (the blocks that fit on every SM at once), but no more
+// than the `want` blocks the work can keep busy, and at least one.
+template <typename Kernel>
+static int persistent_blocks(rrtb_ctx *ctx, Kernel kernel, int smem, unsigned long long want, int *blocks)
+{
+    int per_sm = 0;
+    RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, smem));
+    const unsigned long long wave = (unsigned long long)ctx->sm_count * (per_sm < 1 ? 1 : per_sm);
+    *blocks = (int)(want < 1 ? 1 : (want < wave ? want : wave));
+    return RRTB_OK;
+}
+
 // the lane kernel: persistent, one wave, a multiple of the SM count
 template <class P, bool USE_BVH, bool LIGHTS = false>
 static int launch_lane(rrtb_ctx *ctx, const RenderArgs &args, bool cnt, int *blocks_out)
 {
     auto kernel = cnt ? k_render<P, USE_BVH, true, LIGHTS> : k_render<P, USE_BVH, false, LIGHTS>;
-    int per_sm = 0;
-    RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, 0));
-    if (per_sm < 1) per_sm = 1;
-    unsigned long long want = (args.n_items + RENDER_TPB - 1) / RENDER_TPB;
-    int blocks = ctx->sm_count * per_sm;
-    if ((unsigned long long)blocks > want) blocks = (int)(want ? want : 1);
-    kernel<<<blocks, RENDER_TPB, 0, ctx->stream>>>(args);
-    *blocks_out = blocks;
+    if (int rc = persistent_blocks(ctx, kernel, 0, (args.n_items + RENDER_TPB - 1) / RENDER_TPB, blocks_out)) return rc;
+    kernel<<<*blocks_out, RENDER_TPB, 0, ctx->stream>>>(args);
     return RRTB_OK;
 }
 
@@ -586,15 +592,10 @@ static int launch_pool(rrtb_ctx *ctx, const RenderArgs &args, bool cnt, int *blo
     constexpr int POOL = P::POOL;
     const int smem = (int)(sizeof(WarpPoolT<typename P::real, POOL>) * POOL_WARPS);
     RRTB_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    int per_sm = 0;
-    RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, smem));
-    if (per_sm < 1) per_sm = 1;
-    // persistent: one wave; every warp needs at least a pool's worth of paths to be worth launching
-    unsigned long long want = (args.n_items + (unsigned long long)POOL * POOL_WARPS - 1) / ((unsigned long long)POOL * POOL_WARPS);
-    int blocks = ctx->sm_count * per_sm;
-    if ((unsigned long long)blocks > want) blocks = (int)(want ? want : 1);
-    kernel<<<blocks, RENDER_TPB, smem, ctx->stream>>>(args);
-    *blocks_out = blocks;
+    // every warp needs at least a pool's worth of paths to be worth launching
+    const unsigned long long per_block = (unsigned long long)POOL * POOL_WARPS;
+    if (int rc = persistent_blocks(ctx, kernel, smem, (args.n_items + per_block - 1) / per_block, blocks_out)) return rc;
+    kernel<<<*blocks_out, RENDER_TPB, smem, ctx->stream>>>(args);
     return RRTB_OK;
 }
 
@@ -697,7 +698,7 @@ int finish_render(rrtb_ctx *ctx, rrtb_stats *stats)
         stats->rays = stats->box_tests = stats->sphere_tests = stats->msphere_tests = stats->triangle_tests = stats->hits = 0;
         if (p->count_rays) {
             unsigned long long c[8];
-            RRTB_CUDA(ctx, cudaMemcpy(c, ctx->d_counters, sizeof(c), cudaMemcpyDeviceToHost));
+            if (int rc = read_back(ctx, c, ctx->d_counters, sizeof(c))) return rc;
             stats->rays = c[1];
             stats->box_tests = c[2];
             stats->sphere_tests = c[3];
@@ -733,11 +734,8 @@ template <class P, bool USE_BVH>
 static int launch_aov_kernel(rrtb_ctx *ctx, const AovArgs &a, bool cnt)
 {
     auto kernel = cnt ? k_render_aov<P, USE_BVH, true> : k_render_aov<P, USE_BVH, false>;
-    int per_sm = 0;
-    RRTB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RENDER_TPB, 0));
-    if (per_sm < 1) per_sm = 1;
-    const int want = (a.n_local_tiles + RENDER_TPB / 32 - 1) / (RENDER_TPB / 32);
-    const int blocks = min(ctx->sm_count * per_sm, max(want, 1));
+    int blocks = 0;
+    if (int rc = persistent_blocks(ctx, kernel, 0, (a.n_local_tiles + RENDER_TPB / 32 - 1) / (RENDER_TPB / 32), &blocks)) return rc;
     kernel<<<blocks, RENDER_TPB, 0, ctx->stream>>>(a);
     return RRTB_OK;
 }
