@@ -751,7 +751,7 @@ static int scatter_one(const rrtb_material *m, f3 d_in, f3 n, int front, const u
         f3 ud = unit3(d_in);
         float dn = dot3(ud, n);
         f3 refl = F3(fmaf(-2.0f * dn, n.x, ud.x), fmaf(-2.0f * dn, n.y, ud.y), fmaf(-2.0f * dn, n.z, ud.z));
-        float fuzz = m->param < 1.0f ? m->param : 1.0f;
+        float fuzz = fabsf(m->param < 1.0f ? m->param : 1.0f); /* fuzz * random_in_unit_sphere(): radius |fuzz| */
         if (fuzz > 0.0f) {
             f3 u = sample_unit_sphere(orc_u01(rnd[0]), orc_u01(rnd[1]));
             float ra = orc_u01(rnd[2]);

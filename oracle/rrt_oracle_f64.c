@@ -363,7 +363,7 @@ static int scatter_d(const rrtb_material *m, d3 d_in, d3 n, int front, const uin
     if (m->type == RRTB_METAL) {
         double k = -2.0 * dn;
         d3 r = D3(fma(k, n.x, ud.x), fma(k, n.y, ud.y), fma(k, n.z, ud.z));
-        double fuzz = m->param < 1.0f ? (double)m->param : 1.0;
+        double fuzz = fabs(m->param < 1.0f ? (double)m->param : 1.0);
         if (fuzz > 0.0) {
             d3 u = unit_sphere_d(u01d(rnd[0]), u01d(rnd[1]));
             double ra = u01d(rnd[2]);

@@ -733,7 +733,7 @@ __device__ __forceinline__ bool scatter(int mtype, float4 m, const Ray &r, const
         dx = fmaf(k, nx, udx);
         dy = fmaf(k, ny, udy);
         dz = fmaf(k, nz, udz);
-        float fuzz = fminf(m.w, 1.0f);
+        float fuzz = fabsf(fminf(m.w, 1.0f)); // the ball is symmetric: a negative fuzz f blurs with radius |f|
         if (fuzz > 0.0f) {
             float ux, uy, uz;
             sample_unit_sphere(u01(rnd.x), u01(rnd.y), ux, uy, uz);

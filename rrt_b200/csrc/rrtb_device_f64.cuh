@@ -308,7 +308,7 @@ __device__ __forceinline__ bool scatter_d(int mtype, float4 m, const RayD &r, co
         dx = __fma_rn(k, nx, udx);
         dy = __fma_rn(k, ny, udy);
         dz = __fma_rn(k, nz, udz);
-        double fuzz = m.w < 1.0f ? (double)m.w : 1.0;
+        double fuzz = fabs(m.w < 1.0f ? (double)m.w : 1.0);
         if (fuzz > 0.0) {
             double ux, uy, uz;
             sample_unit_sphere_d(u01d(rnd.x), u01d(rnd.y), ux, uy, uz);

@@ -79,6 +79,16 @@ def test_f64_scatter_bit_exact(ctx, golden):
     got = ctx.scatter_f64(in16, rnd)
     want = Oracle(scene).scatter_f64(in16, rnd)
     assert got.tobytes() == want.tobytes(), name
+    if name == "final":  # the scatter step's parameter space and edges (tests/test_scatter_space.py), once
+        from test_scatter_space import cancel_inputs, space_inputs, space_scene
+
+        space = space_scene()
+        ctx.set_scene(space)
+        orc = Oracle(space)
+        in16, rnd, _ = space_inputs()
+        c16, crnd = cancel_inputs(orc, "f64")
+        for a, r in ((in16, rnd), (c16, crnd)):
+            assert ctx.scatter_f64(a, r).tobytes() == orc.scatter_f64(a, r).tobytes()
 
 
 def test_f64_render_bit_exact_vs_oracle(ctx, golden):

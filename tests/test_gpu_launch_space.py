@@ -15,11 +15,12 @@ with counting on AND off, so each row below is reached by both instantiations (C
     lane    [f32][LBVH]                               group 2, every case, RRTB_SCHED_SIMPLE
     lane    [f64][flat scan]                          group 1, every case, `scan`
     lane    [f64][LBVH]                               group 1, every case, RRTB_SCHED_SIMPLE
-    pool    [f32, no MTRI][plain nodes]               group 2, final / test2 / test3 (3 moving spheres: no motion nodes)
+    pool    [f32, no MTRI][plain nodes]               group 2, final / test2 / test3 (3 moving spheres: no motion nodes),
+                                                      varied (final.txt with negative and large fuzz, other indices)
     pool    [f32, no MTRI][motion nodes]              group 2, fast (64 moving spheres, open shutter)
     pool    [f32, MTRI][plain nodes]                  group 2, mtri_closed (8 moving triangles, shutter closed)
     pool    [f32, MTRI][motion nodes]                 group 2, mtri (8 moving triangles, open shutter)
-    pool    [f64][plain nodes]                        group 1, final / test2 / test3 / mtri_closed
+    pool    [f64][plain nodes]                        group 1, final / test2 / test3 / mtri_closed / varied
     pool    [f64][motion nodes]                       group 1, fast / mtri
 
 Groups: (1) double integrator == oracle, (2) float integrator: every scheduler the same bits, (3) tile and sample
@@ -39,6 +40,7 @@ from oracle_lib import Oracle
 from rrt_b200.types import SceneArrays
 from test_gpu_edge_cases import check_wide_tree, make_scene
 from test_moving_instances import fast_spheres_scene, load, scene_text
+from test_path_by_path import varied_scene
 from test_random_scenes import random_scene, special_rays
 
 pytestmark = pytest.mark.gpu
@@ -63,6 +65,7 @@ def scenes(tmp_path_factory):
     d = tmp_path_factory.mktemp("launch_space")
     out = {name: load_golden(name)[0] for name in ("final", "test2", "test3")}
     out["fast"] = fast_spheres_scene()
+    out["varied"] = varied_scene()
     out["mtri"] = load(d, scene_text("moving"), name="mtri.txt").arrays
     out["mtri_closed"] = load(d, scene_text("moving", 0.5, 0.5), name="mtri_closed.txt").arrays
     assert len(out["mtri"].mtriangles) == 8 and len(out["mtri_closed"].mtriangles) == 8
@@ -105,6 +108,8 @@ CASES = [
     ("mtri_closed", 8, 4, 33, 2, S0),
     ("mtri_closed", 33, 17, 100, 50, S2),
     ("mtri_closed", 31, 3, 16, 1, S1),
+    ("varied", 97, 61, 17, 50, S2),
+    ("varied", 33, 17, 100, 50, S3),
 ]
 SHAPES = {(2, 2), (8, 4), (9, 5), (31, 3), (33, 17), (97, 61)}
 SPPS = {1, 15, 16, 17, 33, 100}
@@ -119,7 +124,7 @@ def test_cases_cover_the_launch_space():
     assert {c[3] for c in CASES} == SPPS
     assert {c[4] for c in CASES} == {1, 2, 50}
     assert {c[5] for c in CASES} == {S0, S1, S2, S3}
-    assert {c[0] for c in CASES} == {"final", "test2", "test3", "fast", "mtri", "mtri_closed"}
+    assert {c[0] for c in CASES} == {"final", "test2", "test3", "fast", "mtri", "mtri_closed", "varied"}
     paths = [c[1] * c[2] * c[3] for c in CASES]
     assert min(paths) < 64 * 8 // 16 and max(paths) > 64 * 8 * 256
 
